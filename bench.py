@@ -2,6 +2,7 @@
 """Benchmark of the graph-convolution hot path (BASELINE.json metric: ChebyNet windows/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3a|3a1|3b|5] [--strong]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (BASELINE.json ``configs``; SURVEY.md 8d pins the shapes):
@@ -358,7 +359,13 @@ class TrainWorkload:
         return n
 
     def step(self, i):
-        self.last = self.trainer.step(self.ring_x[i % self.R], self.ring_y[i % self.R])[0]
+        self.out = self.trainer.step(self.ring_x[i % self.R], self.ring_y[i % self.R])
+        self.last = self.out[0]
+
+    def outputs(self):
+        """The last step's loss and logits, the gradient it computed and the parameters after its update."""
+        loss, logits = self.out
+        return {"loss": loss.reshape(1), "logits": logits, "grads": self.trainer.flat_g, "params": self.trainer.flat_p}
 
     def result_ok(self):
         v = float(self.last)
@@ -539,6 +546,9 @@ class PredictWorkload:
     def step(self, i):
         self._run(self.ring_x[i % self.R])
 
+    def outputs(self):
+        return {"logits": self.logits, "pred": self.pred.double()}
+
     def result_ok(self):
         assert bool(self.torch.isfinite(self.logits).all()), "non-finite logits"
         return {}
@@ -624,6 +634,8 @@ class VertexWorkload:
             dx, dW, db = self.torch.ops.gcn_b200.cheb_bwd(x, None, y, am, self.dy, *pl.tensors(), self.W, self.K, 1,
                                                           ops.BIAS_PER_FILTER, True, True, self.args.algo)
         self.last = dW
+        if self.args.dump_outputs:      # otherwise the step's 390 MB of outputs are freed as at any other step
+            self.out = (y, dx, dW, db)
         return y
 
     def count_launches(self):
@@ -634,6 +646,12 @@ class VertexWorkload:
 
     def step(self, i):
         self._fwd_bwd(self.ring_x[i % self.R])
+
+    def outputs(self):
+        """y and dx (266 MB and 125 MB at B=64) on a fixed sample of 2048 vertices, dW and db whole."""
+        y, dx, dW, db = self.out
+        idx = self.torch.as_tensor(np.sort(np.random.RandomState(0).choice(self.M, 2048, replace=False)), device=self.dev)
+        return {"y": y[:, idx], "dx": dx[:, idx], "dW": dW, "db": db}
 
     def result_ok(self):
         assert bool(self.torch.isfinite(self.last).all()), "non-finite gradient"
@@ -671,6 +689,23 @@ class VertexWorkload:
     cpu_what = "layer forward+backward"
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outputs, dirname):
+    """Write each device tensor as ``dirname/<name>.npy`` (float64 stays float64, everything else becomes float32)."""
+    arrays = {}
+    for name, t in outputs.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -686,6 +721,8 @@ def main():
     ap.add_argument("--nccl-allreduce", action="store_true", help="N>1: plain NCCL all-reduce instead of the peer-memory "
                     "reduction fused into the Adam kernel")
     ap.add_argument("--cublas-fc", action="store_true", help="(with --no-fused-head) FC GEMMs through cuBLAS fp32")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed "
+                    "(rank 0) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     if args.steps is None:
@@ -742,6 +779,8 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms)
     value = world * B * args.steps / (ms_total * 1e-3)
+    # copied on the device now, written once the clock-sampling window below has closed
+    dumped = {k: t.detach().clone() for k, t in wl.outputs().items()} if args.dump_outputs and rank == 0 else None
     if sampler:
         sampler.mark()
     # keep the GPU under the same load for >= 1.5 s so that nvidia-smi (100 ms period) sees the clocks.
@@ -755,6 +794,8 @@ def main():
         torch.cuda.synchronize()
         if sampler:
             sampler.marks[-1] = sampler._lines()
+    if dumped is not None:
+        dump_outputs(dumped, args.dump_outputs)
     extra_cfg = wl.result_ok()
 
     # ---- end to end: pinned host ring -> H2D -> step -> D2H result, all inside the timed region --------------------
@@ -762,9 +803,9 @@ def main():
     copy_stream = torch.cuda.Stream()
     ready = [torch.cuda.Event() for _ in range(2)]
     freed = [torch.cuda.Event() for _ in range(2)]
-    # the end-to-end leg runs at least 200 steps whatever --steps says: over 20 steps the one un-overlapped copy that
-    # fills the pipeline is 4 % of the region (round-1 verdict, weak #6); every rank derives the same count
-    n_e2e = args.steps if cfg["kind"] == "vertex" else max(args.steps, 200)
+    # --steps sets every timed region: over few steps the one un-overlapped copy that fills the pipeline is a visible
+    # share of the end-to-end time (4 % at 20 steps)
+    n_e2e = args.steps
     out_host = torch.zeros(max(n_e2e, 1), dtype=torch.float32).pin_memory()
 
     def e2e_loop(n, record):

@@ -1,6 +1,7 @@
 """Generate the committed fixtures under tests/golden/ (run in the build container).
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden           # everything (needs the reference)
+    python -m oracle.make_golden layers    # layer_cases.npz only, from the stored graph
 
 Two kinds of vectors:
 
@@ -83,47 +84,67 @@ def main():
                         x_perm=coarsening.perm_data_3d(x, perm4),
                         kat_parents0=np.array([4, 1, 1, 2, 2, 3, 0, 0, 3]), kat_parents1=np.array([2, 1, 0, 1, 0]))
 
-    # ---- E. layer cases from the oracle --------------------------------------------------------
+    layer_cases(L4)
+
+
+def layer_cases(L4):
+    """E. layer cases from the oracle.  Each case draws ``B`` windows and keeps the first ``nb`` of them (the draws, and so
+    the stored vectors, are those of the full-batch cases the file first held; fewer windows keep it under 1 MB).  Only
+    what the tests read is stored: the spectral cases' backward reference is recomputed from the stored basis, and the
+    pre-activation of the pooling checks comes from the oracle at test time."""
     rng = np.random.RandomState(7)
     cases = {}
 
-    def add(name, lvl, B, Fin, Fout, K, p, filt, brelu):
+    def add(name, lvl, B, nb, Fin, Fout, K, p, filt, brelu):
         L = L4[lvl]
         M = L.shape[0]
-        x = rng.randn(B, M, Fin).astype(np.float32)
+        x = rng.randn(B, M, Fin).astype(np.float32)[:nb]
         if filt == "fourier":
             W = (rng.randn(M, Fout, Fin) * 0.2).astype(np.float32)
         else:
             W = (rng.randn(Fin * K, Fout) * 0.2).astype(np.float32)
         b = (0.2 + 0.1 * rng.randn(*((M, Fout) if brelu == "b2relu" else (Fout,)))).astype(np.float32)
-        dy = rng.randn(B, -(-M // p), Fout).astype(np.float32)
+        dy = rng.randn(B, -(-M // p), Fout).astype(np.float32)[:nb]
         pr = [dict(W=W, b=b, K=K, p=p)]
-        c = dict(x=x, W=W, b=b, dy=dy, meta=np.array([lvl, B, Fin, Fout, K, p], np.int64),
+        c = dict(x=x, W=W, b=b, dy=dy, meta=np.array([lvl, nb, Fin, Fout, K, p], np.int64),
                  kind=np.array(filt + "/" + brelu))
         for tag, dt in (("64", np.float64), ("32", np.float32)):
             y, tr = O.conv_stack(x, [L], pr, filter=filt, brelu=brelu, dtype=dt, keep=True)
-            dx, g = O.conv_stack_bwd(tr, [L], pr, dy, filter=filt, brelu=brelu, dtype=dt, first_needs_dx=True)
-            if tag == "64":
-                c.update(z64=tr[0]["z"], y64=y, dx64=dx, dW64=g[0]["dW"], db64=g[0]["db"], argmax=tr[0]["argmax"])
-            else:  # the as-run fp32 oracle only documents the noise floor
-                c.update(y32=y, dW32=g[0]["dW"])
-        if filt == "fourier":
-            c["Ut"] = O.fourier_basis(L, np.float32)
+            if tag == "32":  # the as-run fp32 oracle only documents the noise floor
+                c.update(y32=y)
+            elif filt == "fourier":
+                c.update(y64=y, Ut=O.fourier_basis(L, np.float32))
+            else:
+                dx, g = O.conv_stack_bwd(tr, [L], pr, dy, filter=filt, brelu=brelu, dtype=dt, first_needs_dx=True)
+                c.update(y64=y, dx64=dx, dW64=g[0]["dW"], db64=g[0]["db"], argmax=tr[0]["argmax"])
         for k, v in c.items():
             cases[name + "." + k] = v
 
-    add("cheb_l2_k5_p4_b1", 2, 4, 32, 32, 5, 4, "chebyshev5", "b1relu")
-    add("cheb_l0_k5_p4_b1", 0, 2, 15, 32, 5, 4, "chebyshev5", "b1relu")
-    add("cheb_l0_k3_p1_b2", 0, 2, 15, 32, 3, 1, "chebyshev5", "b2relu")
-    add("cheb_l3_k1_p2_b1", 3, 3, 5, 8, 1, 2, "chebyshev5", "b1relu")
-    add("cheb_l2_k2_p2_b2", 2, 3, 6, 16, 2, 2, "chebyshev2", "b2relu")
-    add("cheb_l4_k20_p1_b1", 4, 2, 3, 7, 20, 1, "chebyshev5", "b1relu")
-    add("four_l2_p4_b1", 2, 3, 8, 16, 0, 4, "fourier", "b1relu")
-    add("four_l3_p1_b2", 3, 2, 5, 6, 0, 1, "fourier", "b2relu")
+    add("cheb_l2_k5_p4_b1", 2, 4, 2, 32, 32, 5, 4, "chebyshev5", "b1relu")
+    add("cheb_l0_k5_p4_b1", 0, 2, 1, 15, 32, 5, 4, "chebyshev5", "b1relu")
+    add("cheb_l0_k3_p1_b2", 0, 2, 1, 15, 32, 3, 1, "chebyshev5", "b2relu")
+    add("cheb_l3_k1_p2_b1", 3, 3, 3, 5, 8, 1, 2, "chebyshev5", "b1relu")
+    add("cheb_l2_k2_p2_b2", 2, 3, 3, 6, 16, 2, 2, "chebyshev2", "b2relu")
+    add("cheb_l4_k20_p1_b1", 4, 2, 2, 3, 7, 20, 1, "chebyshev5", "b1relu")
+    add("four_l2_p4_b1", 2, 3, 3, 8, 16, 0, 4, "fourier", "b1relu")
+    add("four_l3_p1_b2", 3, 2, 2, 5, 6, 0, 1, "fourier", "b2relu")
     np.savez_compressed(os.path.join(OUT, "layer_cases.npz"), **cases)
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 
 
+def stored_laplacians():
+    """The Laplacians of ``ref_graph_l4.npz`` (section A's output), so that the layer cases can be rebuilt without the
+    reference."""
+    z = np.load(os.path.join(OUT, "ref_graph_l4.npz"))
+    return [sp.csr_matrix((z["L%d_data" % i], z["L%d_indices" % i], z["L%d_indptr" % i]), shape=tuple(z["L%d_shape" % i]))
+            for i in range(len(z["sizes"]))]
+
+
 if __name__ == "__main__":
-    main()
+    import sys
+
+    if sys.argv[1:] == ["layers"]:
+        layer_cases(stored_laplacians())
+    else:
+        main()

@@ -92,7 +92,11 @@ def test_golden_layer_cases(dev, graph_l4, layer_cases):
             assert rel_inf(r["db"], c["db64"]) <= TOL, tag
             assert rel_inf(r["dx"], c["dx64"]) <= TOL, tag
             if p > 1:
-                a64 = O.b1relu(c["z64"], c["b"]) if brelu == "b1relu" else O.b2relu(c["z64"], c["b"])
+                # the fp64 pre-activation from the oracle (test_oracle.py pins it to the stored y64 and argmax)
+                _, tr = O.conv_stack(c["x"], [L], [dict(W=c["W"], b=c["b"], K=K, p=p)], filter=filt, brelu=brelu,
+                                     dtype=np.float64, keep=True)
+                z64 = tr[0]["z"]
+                a64 = O.b1relu(z64, c["b"]) if brelu == "b1relu" else O.b2relu(z64, c["b"])
                 check_argmax(r["argmax"], a64, p, tag)
 
 
