@@ -244,11 +244,15 @@ size_t gcnb_cheb_workspace_bytes(int B, int M, int nnz, int Fin, int Fout, int K
                                  int algo) {
   LayerShape s{B, M, nnz, Fin, Fout, K, p};
   const bool fused_ok = backward ? fused_bwd_supported(s, need_dx != 0) : fused_fwd_supported(s);
+  // given the fused kernels' saved basis, a backward without dx runs stack_dw even where the fused backward does not fit
+  // (gcnb_cheb_bwd_f32): its workspace must be there on the FUSED-unsupported and the general branch too (for every
+  // algo on the latter, so that AUTO keeps asking for exactly what one of the two families asks for)
+  const size_t stack_only = backward && !need_dx && stack_layout(s) == 1 ? stack_dw_workspace(s) + 512 : 0;
   if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && fused_ok))
     return fused_ok ? fused_cheb_workspace(s, backward != 0, need_dx != 0) + (backward ? stack_dw_workspace(s) + 512 : 0)
-                    : 0;
+                    : stack_only;
   return general_cheb_workspace(s, backward != 0, need_dx != 0) +
-         (backward ? align_up((size_t)B * ceil_div(M, p) * Fout * sizeof(float), 256) + 256 : 0);
+         (backward ? align_up((size_t)B * ceil_div(M, p) * Fout * sizeof(float), 256) + 256 : 0) + stack_only;
 }
 
 int gcnb_cheb_fwd_f32(const float* x, const int32_t* perm, int M_in, const gcnb_csr* L, const float* W,

@@ -310,8 +310,15 @@ def fourier_bwd(x, Ut, W, dz, dtype=np.float32):
 
 
 def conv_stack_bwd(trace, Ls, params, dy, filter="chebyshev5", brelu="b1relu", dtype=np.float32,
-                   first_needs_dx=False):
+                   first_needs_dx=False, decisions=None):
     """Back-propagate ``dy`` through the layers recorded by ``conv_stack(..., keep=True)``.
+
+    ``decisions`` (optional, one ``dict(argmax=uint8, relu=bool)`` per layer, both at pooled resolution
+    ``[N, ceil(M/p), F]``) routes the gradient the way another implementation decided: ``argmax`` replaces the
+    first-maximum bytes of the trace and ``relu`` (that implementation's ``y > 0``) replaces the ReLU mask.  Where a
+    window maximum or a pre-activation sits within rounding of a tie, an fp32 run may decide the other way and move a
+    whole gradient element; conditioning on its decisions keeps the comparison about the arithmetic.  Passing the
+    trace's own decisions gives bit for bit what passing none gives.
 
     Returns ``(dx_or_None, [dict(dW, db), ...])``.
     """
@@ -319,8 +326,13 @@ def conv_stack_bwd(trace, Ls, params, dy, filter="chebyshev5", brelu="b1relu", d
     for i in range(len(params) - 1, -1, -1):
         t, pr, L = trace[i], params[i], Ls[i]
         M = t["a"].shape[1]
-        da = mpool1_bwd(np.asarray(dy, dtype), t["argmax"], pr["p"], M)
-        dz, db = brelu_bwd(da, t["a"], per_vertex=(brelu == "b2relu"))
+        am, live = t["argmax"], t["a"]
+        if decisions is not None:
+            am = np.asarray(decisions[i]["argmax"], np.uint8).reshape(t["argmax"].shape)
+            # the routed element of a window is live iff the pooled value is: (a > 0) at the arg-max is (y > 0)
+            live = mpool1_bwd(np.asarray(decisions[i]["relu"], dtype).reshape(t["y"].shape), am, pr["p"], M)
+        da = mpool1_bwd(np.asarray(dy, dtype), am, pr["p"], M)
+        dz, db = brelu_bwd(da, live, per_vertex=(brelu == "b2relu"))
         need_dx = i > 0 or first_needs_dx
         if filter == "fourier":
             dx, dW = fourier_bwd(t["x"], fourier_basis(L, dtype), pr["W"], dz, dtype)
@@ -355,12 +367,13 @@ def counter_dropout_mask(rows, cols, keep, seed, step):
 
 
 def network_step(x, labels, Ls, params, fcs, regularization, filter="chebyshev5", brelu="b1relu", dtype=np.float32,
-                 dropout_masks=None, keep=1.0):
+                 dropout_masks=None, keep=1.0, conv_decisions=None):
     """Forward + loss + backward of the whole network (conv stack, mean over F, FC head, CE + L2).
 
     What one ``sess.run([op_train, ...])`` computes up to the optimiser update (models_gcn.py:146, :298-303).
     ``dropout_masks`` (one 0/1 array per hidden FC layer) with keep-probability ``keep`` reproduces ``tf.nn.dropout``
-    (models_gcn.py:677: kept activations scaled by 1/keep) for a GIVEN mask.
+    (models_gcn.py:677: kept activations scaled by 1/keep) for a GIVEN mask.  ``conv_decisions`` routes the conv
+    backward through given pooling / ReLU decisions (``conv_stack_bwd(decisions=...)``).
     Returns ``(loss, conv_grads, fc_grads)``.  Used as the CPU baseline and by the gradient parity test.
     """
     h, trace = conv_stack(x, Ls, params, filter=filter, brelu=brelu, dtype=dtype, keep=True)
@@ -391,7 +404,8 @@ def network_step(x, labels, Ls, params, fcs, regularization, filter="chebyshev5"
         fc_grads[i] = (acts[i].T @ d + regularization * np.asarray(W, dtype), d.sum(0) + regularization * np.asarray(b, dtype))
         d = d @ np.asarray(W, dtype).T
     dh = np.repeat(d[:, :, None], F_last, axis=2) / dtype(F_last)
-    _, conv_grads = conv_stack_bwd(trace, Ls, params, dh, filter=filter, brelu=brelu, dtype=dtype)
+    _, conv_grads = conv_stack_bwd(trace, Ls, params, dh, filter=filter, brelu=brelu, dtype=dtype,
+                                   decisions=conv_decisions)
     if filter != "chebyshev2":
         for g, p in zip(conv_grads, params):
             g["dW"] = g["dW"] + regularization * np.asarray(p["W"], dtype)

@@ -691,7 +691,8 @@ def _head_oracle(a0, labels, Ws, bs, masks, keep):
 
 @pytest.mark.parametrize("B,widths,keep", [(512, (25, 512, 256, 22), 1.0), (512, (25, 512, 256, 22), 0.5),
                                            (37, (25, 512, 256, 22), 0.5), (130, (7, 100, 50, 5), 0.75),
-                                           (64, (32, 129, 67, 32), 1.0)])
+                                           (64, (32, 129, 67, 32), 1.0), (2048, (25, 512, 256, 22), 0.5),
+                                           (4096, (25, 512, 256, 22), 0.5)])
 def test_head_step_kernel_matches_oracle(dev, B, widths, keep):
     """gcnb_head_step_f32 (one cooperative launch: FC x3, cross-entropy, full backward) against the fp64 oracle run with
     the SAME dropout masks (the counter-based mask is mirrored in oracle.counter_dropout_mask)."""
@@ -905,8 +906,10 @@ def _random_tcgen05_cases(n=14, seed=2026):
 @pytest.mark.parametrize("lvl,B,Fin,Fout,K,p,brelu", _random_tcgen05_cases())
 def test_layer_random_shapes(dev, graph_l4, lvl, B, Fin, Fout, K, p, brelu):
     """Seeded random layer shapes around the tcgen05 kernel's domain (9 <= Fin <= 32, Fout a multiple of 4, any K, p in
-    {1,2,4,8}, ragged batches): forward (y, arg-max) and backward (dx through the adjoint mode, dW/db from the saved
-    basis) against the fp64 oracle, with and without the host-built operator image where the shape has one."""
+    {1,2,4,8}, ragged batches): forward (y, arg-max) and the autograd backward against the fp64 oracle, with and without
+    the host-built operator image where the shape has one.  Autograd keeps no basis, so the backward recomputes it
+    (k_cheb_bwd_fused or the general path); the saved-basis backward of the training step is swept in
+    test_gpu_saved_basis.py."""
     from gcn_fmri_decoding_b200 import _lib, plan
 
     L = graph_l4["L"][lvl]
@@ -945,7 +948,7 @@ def test_layer_random_shapes(dev, graph_l4, lvl, B, Fin, Fout, K, p, brelu):
         assert rel_inf(r["dx"], dx64) <= TOL, tag
 
 
-@pytest.mark.parametrize("brelu,nlayers,B", [("b2relu", 5, 19), ("b1relu", 3, 150), ("b2relu", 8, 2)])
+@pytest.mark.parametrize("brelu,nlayers,B", [("b2relu", 5, 19), ("b1relu", 3, 150), ("b2relu", 8, 2), ("b1relu", 4, 445)])
 def test_layer_stack_is_bit_identical_to_layer_by_layer(dev, graph_l1, brelu, nlayers, B):
     """gcnb_cheb_stack_fwd_f32: a run of identical p = 1, 32 -> 32 layers in one launch (the production network's
     layers 2-6, model.py:271-274) gives bit for bit what the same layers give one launch at a time -- and hence the

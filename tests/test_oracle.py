@@ -327,3 +327,86 @@ def test_oracle_reproduces_the_vectors_of_the_reference_source(graph_l1, graph_l
                 assert str(filt) == "chebyshev2" and i < len(p) - 1
                 continue
             assert close(cg[i]["dW"], grad[key]) and close(cg[i]["db"], grad["conv%d/bias" % (i + 1)]), (name, i)
+
+
+# --------------------------------------------------------------------------------------------------------------------
+# Backward conditioned on given pooling / ReLU decisions (what the GPU tests use to compare with an fp32 run whose
+# near-tie decisions went the other way).
+def _own_decisions(trace):
+    return [dict(argmax=t["argmax"], relu=t["y"] > 0) for t in trace]
+
+
+@pytest.mark.parametrize("brelu,lvls,ps", [("b1relu", (0, 2), (4, 4)), ("b2relu", (3, 3), (1, 2)), ("b1relu", (2, 3), (2, 8))])
+def test_backward_with_its_own_decisions_is_bit_identical(graph_l4, brelu, lvls, ps):
+    """Passing the oracle's own arg-max bytes and ReLU mask changes nothing, bit for bit: conv_stack_bwd and
+    network_step.  (lvl 3 pooled by 8: 50 vertices, a ragged SAME window.)"""
+    rng = np.random.RandomState(17)
+    Ls = [graph_l4["L"][l] for l in lvls]
+    B, Fs, K = 6, (5, 8, 6), 3
+    params = []
+    for i, L in enumerate(Ls):
+        M = L.shape[0]
+        b = rng.randn(M, Fs[i + 1]) * 0.3 if brelu == "b2relu" else rng.randn(Fs[i + 1]) * 0.3
+        params.append(dict(W=rng.randn(Fs[i] * K, Fs[i + 1]) * 0.3, b=b, K=K, p=ps[i]))
+    x = rng.randn(B, Ls[0].shape[0], Fs[0])
+    y, tr = O.conv_stack(x, Ls, params, brelu=brelu, dtype=np.float64, keep=True)
+    assert 0.1 < np.mean([t["y"] > 0 for t in tr][-1]) < 0.9          # both branches of the ReLU are taken
+    dy = rng.randn(*y.shape)
+    dx0, g0 = O.conv_stack_bwd(tr, Ls, params, dy, brelu=brelu, dtype=np.float64, first_needs_dx=True)
+    dx1, g1 = O.conv_stack_bwd(tr, Ls, params, dy, brelu=brelu, dtype=np.float64, first_needs_dx=True,
+                               decisions=_own_decisions(tr))
+    assert np.array_equal(dx0, dx1)
+    for a, b in zip(g0, g1):
+        assert np.array_equal(a["dW"], b["dW"]) and np.array_equal(a["db"], b["db"])
+    labels = rng.randint(0, 4, B)
+    M_last = y.shape[1]
+    fcs = [(rng.randn(M_last, 7) * 0.2, rng.randn(7) * 0.1), (rng.randn(7, 4) * 0.2, rng.randn(4) * 0.1)]
+    masks = [(rng.rand(B, 7) < 0.5).astype(np.float64)]
+    r0 = O.network_step(x, labels, Ls, params, fcs, 5e-4, brelu=brelu, dtype=np.float64, dropout_masks=masks, keep=0.5)
+    r1 = O.network_step(x, labels, Ls, params, fcs, 5e-4, brelu=brelu, dtype=np.float64, dropout_masks=masks, keep=0.5,
+                        conv_decisions=_own_decisions(tr))
+    assert r0[0] == r1[0]
+    for a, b in zip(r0[1], r1[1]):
+        assert np.array_equal(a["dW"], b["dW"]) and np.array_equal(a["db"], b["db"])
+    for a, b in zip(r0[2], r1[2]):
+        assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
+
+
+def test_flipped_argmax_byte_moves_exactly_that_gradient(graph_l4):
+    """One arg-max byte sent to another vertex of its window moves that one dz element there: dW changes by
+    dy * (X[new row] - X[old row]) in that one column, the per-vertex bias gradient moves between the two vertices,
+    everything else stays put.  A dead ReLU decision removes the element instead."""
+    rng = np.random.RandomState(23)
+    L = graph_l4["L"][2]
+    M, B, Fin, Fout, K, p = L.shape[0], 3, 4, 5, 3, 4
+    pr = [dict(W=rng.randn(Fin * K, Fout) * 0.3, b=rng.randn(M, Fout) * 0.3, K=K, p=p)]
+    x = rng.randn(B, M, Fin)
+    y, tr = O.conv_stack(x, [L], pr, brelu="b2relu", dtype=np.float64, keep=True)
+    dy = rng.randn(*y.shape)
+    live = np.argwhere(tr[0]["y"] > 0)
+    n, j, f = live[len(live) // 2]
+    old = int(tr[0]["argmax"][n, j, f])
+    new = (old + 1) % p
+    dec = _own_decisions(tr)
+    dec[0]["argmax"] = dec[0]["argmax"].copy()
+    dec[0]["argmax"][n, j, f] = new
+    _, g0 = O.conv_stack_bwd(tr, [L], pr, dy, brelu="b2relu", dtype=np.float64)
+    _, g1 = O.conv_stack_bwd(tr, [L], pr, dy, brelu="b2relu", dtype=np.float64, decisions=dec)
+    X = O.chebyshev_stack(x, L, K, np.float64).reshape(B, M, Fin * K)
+    r_old, r_new = j * p + old, j * p + new
+    expect = g0[0]["dW"].copy()
+    expect[:, f] += dy[n, j, f] * (X[n, r_new] - X[n, r_old])
+    assert np.allclose(g1[0]["dW"], expect, rtol=0, atol=1e-12 * np.abs(expect).max())
+    assert not np.allclose(g1[0]["dW"][:, f], g0[0]["dW"][:, f], rtol=0, atol=1e-6 * np.abs(expect).max())
+    ddb = g1[0]["db"] - g0[0]["db"]
+    want = np.zeros_like(ddb)
+    want[r_old, f], want[r_new, f] = -dy[n, j, f], dy[n, j, f]
+    assert np.allclose(ddb, want, rtol=0, atol=1e-12)
+    # the same element declared dead: its gradient disappears from the bias gradient of its vertex
+    dec2 = _own_decisions(tr)
+    dec2[0]["relu"] = dec2[0]["relu"].copy()
+    dec2[0]["relu"][n, j, f] = False
+    _, g2 = O.conv_stack_bwd(tr, [L], pr, dy, brelu="b2relu", dtype=np.float64, decisions=dec2)
+    want = np.zeros_like(ddb)
+    want[r_old, f] = -dy[n, j, f]
+    assert np.allclose(g2[0]["db"] - g0[0]["db"], want, rtol=0, atol=1e-12)
