@@ -36,7 +36,7 @@ SIGNATURES = {
     "gcnb_launch_count": (C.c_ulonglong, []),
     "gcnb_cheb_fused_supported": (_i, [_i] * 9),
     "gcnb_cheb_workspace_bytes": (_z, [_i] * 10),
-    "gcnb_cheb_fwd_describe": (_i, [_i] * 7 + [C.c_char_p, _z]),
+    "gcnb_cheb_describe": (_i, [_i] * 11 + [C.c_char_p, _z, C.POINTER(_z)]),
     "gcnb_cheb_stack_width": (_i, [_i] * 7),
     "gcnb_cheb_image_bytes": (_z, [_p, _p] + [_i] * 8),
     "gcnb_cheb_image_build": (_i, [_p, _p, _p] + [_i] * 8 + [_p, _z]),
@@ -98,11 +98,17 @@ def lib():
     return _lib
 
 
+def describe(B, M, nnz, Fin, Fout, K, p, backward=False, need_dx=False, saved_basis=False, algo=ALGO_AUTO):
+    """The route a Chebyshev layer call takes, as ``("<route>: <its kernels>", workspace bytes of that route)``."""
+    buf, nbytes = C.create_string_buffer(512), _z()
+    check(lib().gcnb_cheb_describe(B, M, nnz, Fin, Fout, K, p, int(backward), int(need_dx), int(saved_basis), algo, buf,
+                                   512, C.byref(nbytes)), "gcnb_cheb_describe")
+    return buf.value.decode(), nbytes.value
+
+
 def describe_fwd(B, M, nnz, Fin, Fout, K, p):
     """Which forward kernel AUTO dispatch picks for this layer shape, and its tile geometry."""
-    buf = C.create_string_buffer(512)
-    check(lib().gcnb_cheb_fwd_describe(B, M, nnz, Fin, Fout, K, p, buf, 512), "gcnb_cheb_fwd_describe")
-    return buf.value.decode()
+    return describe(B, M, nnz, Fin, Fout, K, p)[0]
 
 
 def last_error():

@@ -61,8 +61,6 @@ __device__ __forceinline__ void adam_one(const AdamArParams& P, long long i, flo
 }
 
 __global__ void __launch_bounds__(256) k_adam_tf_allreduce(const AdamArParams P) {
-  pdl_trigger();
-  pdl_wait();  // the gradients come from the predecessors in the stream
   uint32_t* myflags = P.flags[P.rank];
   __shared__ uint32_t s_seq;
   if (threadIdx.x == 0) s_seq = *reinterpret_cast<volatile uint32_t*>(myflags + 63) + 1u;  // bumped by the LAST CTA only
@@ -150,7 +148,7 @@ int gcnb_adam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* deca
   if (rc) return rc;
   // at most one CTA per SM: every CTA spins on the flags, so all of them must be resident together with CTA 0
   const int grid = (int)std::max<long long>(1, std::min<long long>(ceil_div_ll(n, 256 * 4), di.sm_count));
-  GCNB_CUDA(launch_pdl(k_adam_tf_allreduce, dim3(grid), dim3(256), 0, static_cast<cudaStream_t>(stream), P));
+  k_adam_tf_allreduce<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(P);
   GCNB_LAUNCH_CHECK("k_adam_tf_allreduce");
   return GCNB_OK;
 }

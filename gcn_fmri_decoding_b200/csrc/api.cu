@@ -1,7 +1,6 @@
 // extern "C" entry points of libgcnb200.so: argument validation, kernel-family dispatch, and the
 // small stand-alone kernels (b1relu/b2relu, mpool1, perm gather, mean over filters).
 #include <algorithm>
-#include <cstdlib>
 #include <atomic>
 #include <mutex>
 
@@ -20,25 +19,6 @@ void set_error(const char* fmt, ...) {
 
 static std::atomic<unsigned long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    // Off by default: measured on the config-2 step (B200, CUDA graph) 0.343 ms with the attribute vs 0.338 ms
-    // without -- back-to-back launches of ONE kernel gain 3-5 %, the mixed chain of the step loses it again.
-    const char* v = getenv("GCNB_PDL");
-    return v && v[0] == '1';
-  }();
-  return on;
-}
-
-// GCNB_UMMA_ADJ=0 sends the input gradient back to k_cheb_bwd_fused (A/B runs); read once.
-static bool adjoint_umma_enabled() {
-  static const bool on = [] {
-    const char* v = getenv("GCNB_UMMA_ADJ");
-    return !(v && v[0] == '0');
-  }();
-  return on;
-}
 
 int device_info(DeviceInfo* out) {
   static std::mutex mu;
@@ -201,58 +181,159 @@ static int check_layer(const char* who, const gcnb_csr* L, int B, int Fin, int F
   return GCNB_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Chebyshev layer plan: the one place that decides which kernels a call runs and the workspace they take.  The
+// dispatch (gcnb_cheb_fwd_f32 / gcnb_cheb_bwd_f32) and every query (workspace, basis width, fused support, describe)
+// read it.
+// ------------------------------------------------------------------------------------------------
+enum ChebRoute {
+  ROUTE_UNSUPPORTED,
+  ROUTE_FWD_UMMA,        // k_cheb_fwd_umma (tcgen05 / TMEM)
+  ROUTE_FWD_FUSED,       // k_cheb_fwd_fused (mma.sync, shared-memory resident)
+  ROUTE_GENERAL,         // HBM-resident state, forward or backward
+  ROUTE_STACK_DW,        // dW / db streamed from the saved basis, no dx
+  ROUTE_STACK_ADJ,       // ... and dx through k_cheb_fwd_umma on L~^T
+  ROUTE_STACK_FUSED_DX,  // ... and dx through k_cheb_bwd_fused
+  ROUTE_FUSED_BWD,       // k_cheb_bwd_fused recomputes the basis
+};
+
+struct ChebPlan {
+  ChebRoute route;
+  // saved basis of the shape (only when the call passes one): 1 = the fused kernels' [K][B][M][FP], 2 = the general
+  // path's vertex-major [K][M][B][Fin] for graphs the fused kernels cannot hold, 0 = none exists
+  int layout;
+  size_t region[2];  // workspace regions of the route, in order; each a multiple of 256 bytes
+  const char* why;   // ROUTE_UNSUPPORTED: the reason, NULL when the fused kernels do not fit the shape
+  size_t total() const { return region[0] + region[1]; }
+};
+
+static ChebPlan plan_cheb(const LayerShape& s, bool backward, bool need_dx, bool saved, int algo) {
+  ChebPlan pl{ROUTE_UNSUPPORTED, 0, {0, 0}, nullptr};
+  auto route = [&pl](ChebRoute r, size_t a, size_t b = 0) {
+    pl.route = r;
+    pl.region[0] = a;
+    pl.region[1] = b;
+    return pl;
+  };
+  const bool fwd_ok = fused_fwd_supported(s);
+  if (saved) pl.layout = fwd_ok ? (stack_dw_supported(s) ? 1 : 0) : 2;
+  if (!backward) {
+    if (algo == GCNB_ALGO_FUSED && !fwd_ok) return pl;
+    // the tcgen05 kernel writes the same basis layout as the mma.sync one, where that layout exists
+    if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && fwd_ok))
+      return route(umma_fwd_supported(s) && (!saved || pl.layout == 1) ? ROUTE_FWD_UMMA : ROUTE_FWD_FUSED,
+                   fused_cheb_workspace(s, false, false));
+    if (saved && pl.layout != 2) {
+      pl.why = "the general path cannot produce the stack layout gcnb_cheb_stack_width() announced";
+      return pl;
+    }
+    return route(ROUTE_GENERAL, general_cheb_workspace(s, false, false));
+  }
+  if (saved && pl.layout == 0) {
+    pl.why = "no stack layout exists for this shape";
+    return pl;
+  }
+  // the fused kernels' saved basis: the weight gradient is one streamed GEMM (ALGO_GENERAL recomputes instead), also
+  // where the fused backward does not fit
+  const bool stack = pl.layout == 1 && algo != GCNB_ALGO_GENERAL;
+  const size_t sdw = stack ? stack_dw_workspace(s) + 512 : 0;
+  if (stack && !need_dx) return route(ROUTE_STACK_DW, sdw);
+  const bool bwd_ok = pl.layout != 2 && fused_bwd_supported(s, need_dx);
+  const size_t fw = bwd_ok ? fused_cheb_workspace(s, true, need_dx) : 0;
+  if (stack && bwd_ok) {  // only dx needs the adjoint recursion; ALGO_FUSED keeps it on k_cheb_bwd_fused
+    if (s.K > 1 && algo == GCNB_ALGO_AUTO && umma_adj_supported(s)) return route(ROUTE_STACK_ADJ, sdw);
+    return route(ROUTE_STACK_FUSED_DX, sdw, fw);
+  }
+  if (algo == GCNB_ALGO_FUSED && !bwd_ok) return pl;
+  if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && bwd_ok)) return route(ROUTE_FUSED_BWD, fw);
+  // the general path works on the full gradient: a dy given as the mean over the filters is expanded first
+  return route(ROUTE_GENERAL, general_cheb_workspace(s, true, need_dx),
+               align_up((size_t)s.B * ceil_div(s.M, s.p) * s.Fout * sizeof(float), 256) + 256);
+}
+
+// region i of the plan in the caller's workspace
+static Workspace plan_region(const ChebPlan& pl, int i, void* workspace, size_t bytes) {
+  const size_t off = i == 0 ? 0 : pl.region[0];
+  if (workspace == nullptr || off >= bytes) return Workspace(nullptr, 0);
+  return Workspace(static_cast<char*>(workspace) + off, std::min(pl.region[i], bytes - off));
+}
+
+static int plan_error(const char* who, const ChebPlan& pl, const LayerShape& s) {
+  if (pl.why)
+    set_error("%s: %s", who, pl.why);
+  else
+    set_error("%s: fused kernels do not support B=%d M=%d nnz=%d Fin=%d Fout=%d K=%d p=%d", who, s.B, s.M, s.nnz, s.Fin,
+              s.Fout, s.K, s.p);
+  return GCNB_ERR_INVALID;
+}
+
+static void plan_describe(const ChebPlan& pl, const LayerShape& s, bool backward, char* out, size_t n) {
+  switch (pl.route) {
+    case ROUTE_FWD_UMMA:
+      umma_fwd_describe(s, out, n);
+      return;
+    case ROUTE_FWD_FUSED:
+      snprintf(out, n, "k_cheb_fwd_fused: mma.sync, shared-memory resident");
+      return;
+    case ROUTE_GENERAL:
+      snprintf(out, n, "%s", backward ? "general path: HBM-resident state (k_spmm_tma + k_node_dw, k_dz_wt for dx)"
+                                      : "general path: HBM-resident state (k_spmm_tma + k_stack_contract)");
+      return;
+    case ROUTE_STACK_DW:
+      snprintf(out, n, "stack-dW: k_dw_from_stack + k_dw_from_partials");
+      return;
+    case ROUTE_STACK_ADJ:
+      snprintf(out, n, "stack-dW + tcgen05 adjoint: k_dw_from_stack + k_dw_from_partials, dx by k_cheb_fwd_umma on L~^T");
+      return;
+    case ROUTE_STACK_FUSED_DX:
+      snprintf(out, n, "stack-dW + fused dx: k_dw_from_stack + k_dw_from_partials, dx by k_cheb_bwd_fused");
+      return;
+    case ROUTE_FUSED_BWD:
+      snprintf(out, n, "fused recompute: k_cheb_bwd_fused + k_dw_from_partials");
+      return;
+    default:
+      snprintf(out, n, "unsupported: %s", pl.why ? pl.why : "the fused kernels do not fit this shape");
+  }
+}
+
 }  // namespace gcnb
 
 using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 100; }
+int gcnb_version(void) { return 101; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 
 unsigned long long gcnb_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-// Layout of the saved Chebyshev stack: 1 = fused kernels' [K][B][M][FP], 2 = general path's vertex-major
-// [K][M][B][Fin] (graphs the fused kernels cannot hold), 0 = this shape keeps no stack.
-static int stack_layout(const LayerShape& s) {
-  if (fused_fwd_supported(s)) return stack_dw_supported(s) ? 1 : 0;
-  return 2;
-}
-
 int gcnb_cheb_stack_width(int B, int M, int nnz, int Fin, int Fout, int K, int p) {
   LayerShape s{B, M, nnz, Fin, Fout, K, p};
-  const int layout = stack_layout(s);
+  const int layout = plan_cheb(s, false, false, true, GCNB_ALGO_AUTO).layout;
   return layout == 1 ? fused_feature_pad(Fin) : layout == 2 ? Fin : 0;
 }
 
-int gcnb_cheb_fwd_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, char* out, size_t n) {
+int gcnb_cheb_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx, int saved_basis,
+                       int algo, char* out, size_t n, size_t* route_workspace_bytes) {
   if (!out || n == 0) return GCNB_ERR_INVALID;
   LayerShape s{B, M, nnz, Fin, Fout, K, p};
-  if (umma_fwd_describe(s, out, n) > 0) return GCNB_OK;
-  snprintf(out, n, "%s", fused_fwd_supported(s) ? "k_cheb_fwd_fused: mma.sync, shared-memory resident"
-                                                  : "general path: HBM-resident state (k_spmm_tma + k_stack_contract)");
+  const ChebPlan pl = plan_cheb(s, backward != 0, need_dx != 0, saved_basis != 0, algo);
+  plan_describe(pl, s, backward != 0, out, n);
+  if (route_workspace_bytes) *route_workspace_bytes = pl.total();
   return GCNB_OK;
 }
 
 int gcnb_cheb_fused_supported(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx) {
   LayerShape s{B, M, nnz, Fin, Fout, K, p};
-  return backward ? (fused_bwd_supported(s, need_dx != 0) ? 1 : 0) : (fused_fwd_supported(s) ? 1 : 0);
+  return plan_cheb(s, backward != 0, need_dx != 0, false, GCNB_ALGO_FUSED).route != ROUTE_UNSUPPORTED;
 }
 
 size_t gcnb_cheb_workspace_bytes(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx,
                                  int algo) {
   LayerShape s{B, M, nnz, Fin, Fout, K, p};
-  const bool fused_ok = backward ? fused_bwd_supported(s, need_dx != 0) : fused_fwd_supported(s);
-  // given the fused kernels' saved basis, a backward without dx runs stack_dw even where the fused backward does not fit
-  // (gcnb_cheb_bwd_f32): its workspace must be there on the FUSED-unsupported and the general branch too (for every
-  // algo on the latter, so that AUTO keeps asking for exactly what one of the two families asks for)
-  const size_t stack_only = backward && !need_dx && stack_layout(s) == 1 ? stack_dw_workspace(s) + 512 : 0;
-  if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && fused_ok))
-    return fused_ok ? fused_cheb_workspace(s, backward != 0, need_dx != 0) + (backward ? stack_dw_workspace(s) + 512 : 0)
-                    : stack_only;
-  return general_cheb_workspace(s, backward != 0, need_dx != 0) +
-         (backward ? align_up((size_t)B * ceil_div(M, p) * Fout * sizeof(float), 256) + 256 : 0) + stack_only;
+  return std::max(plan_cheb(s, backward != 0, need_dx != 0, false, algo).total(),
+                  plan_cheb(s, backward != 0, need_dx != 0, true, algo).total());
 }
 
 int gcnb_cheb_fwd_f32(const float* x, const int32_t* perm, int M_in, const gcnb_csr* L, const float* W,
@@ -266,28 +347,24 @@ int gcnb_cheb_fwd_f32(const float* x, const int32_t* perm, int M_in, const gcnb_
                L->M);
   GCNB_REQUIRE(M_in >= 1, "gcnb_cheb_fwd_f32: M_in must be >= 1");
   LayerShape s{B, L->M, L->nnz, Fin, Fout, K, p};
-  Workspace ws(workspace, workspace_bytes);
+  const ChebPlan pl = plan_cheb(s, false, false, xstack != nullptr, algo);
+  Workspace ws = plan_region(pl, 0, workspace, workspace_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const bool fused_ok = fused_fwd_supported(s);
-  if (algo == GCNB_ALGO_FUSED && !fused_ok) {
-    set_error("gcnb_cheb_fwd_f32: fused kernels do not support B=%d M=%d nnz=%d Fin=%d Fout=%d K=%d p=%d", B, s.M,
-              s.nnz, Fin, Fout, K, p);
-    return GCNB_ERR_INVALID;
-  }
   const long long pooled_rows = (long long)B * ceil_div(s.M, p);
-  if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && fused_ok)) {
-    // tensor-core (tcgen05/TMEM) kernel when the shape fits it; it writes the same xstack layout as the mma.sync one
-    if (umma_fwd_supported(s) && (xstack == nullptr || stack_layout(s) == 1))
+  switch (pl.route) {
+    case ROUTE_FWD_UMMA:
       return umma_cheb_fwd(x, perm, M_in, *L, W, bias, y, argmax, y_mean, xstack, s, bias_mode, relu, st);
-    rc = fused_cheb_fwd(x, perm, M_in, *L, W, bias, y, argmax, y_mean, xstack, s, bias_mode, relu, ws, st);
-    if (rc == GCNB_OK && y_mean != nullptr && Fout > 32) rc = launch_mean_f(y, y_mean, pooled_rows, Fout, st);
-    return rc;
+    case ROUTE_FWD_FUSED:
+      rc = fused_cheb_fwd(x, perm, M_in, *L, W, bias, y, argmax, y_mean, xstack, s, bias_mode, relu, ws, st);
+      if (rc == GCNB_OK && y_mean != nullptr && Fout > 32) rc = launch_mean_f(y, y_mean, pooled_rows, Fout, st);
+      return rc;
+    case ROUTE_GENERAL:
+      rc = general_cheb_fwd(x, perm, M_in, *L, W, bias, y, argmax, xstack, s, bias_mode, relu, ws, st);
+      if (rc == GCNB_OK && y_mean != nullptr) rc = launch_mean_f(y, y_mean, pooled_rows, Fout, st);
+      return rc;
+    default:
+      return plan_error("gcnb_cheb_fwd_f32", pl, s);
   }
-  GCNB_REQUIRE(xstack == nullptr || stack_layout(s) == 2,
-               "gcnb_cheb_fwd_f32: the general path cannot produce the stack layout gcnb_cheb_stack_width() announced");
-  rc = general_cheb_fwd(x, perm, M_in, *L, W, bias, y, argmax, xstack, s, bias_mode, relu, ws, st);
-  if (rc == GCNB_OK && y_mean != nullptr) rc = launch_mean_f(y, y_mean, pooled_rows, Fout, st);
-  return rc;
 }
 
 int gcnb_cheb_stack_supported(const gcnb_csr* L, int B, int F, int K, int nlayers) {
@@ -349,43 +426,37 @@ int gcnb_cheb_bwd_f32(const float* x, const int32_t* perm, int M_in, const float
   GCNB_REQUIRE(dx == nullptr || K == 1 || (Lt && Lt->M == L->M && Lt->nnz == L->nnz),
                "gcnb_cheb_bwd_f32: dx needs the transposed operator Lt with the same M and nnz");
   LayerShape s{B, L->M, L->nnz, Fin, Fout, K, p};
-  Workspace ws(workspace, workspace_bytes);
+  const ChebPlan pl = plan_cheb(s, true, dx != nullptr, xstack != nullptr, algo);
+  Workspace ws = plan_region(pl, 0, workspace, workspace_bytes), ws1 = plan_region(pl, 1, workspace, workspace_bytes);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int layout = xstack ? stack_layout(s) : 0;
-  GCNB_REQUIRE(xstack == nullptr || layout != 0, "gcnb_cheb_bwd_f32: no stack layout exists for this shape");
-  if (layout == 1 && dx == nullptr && algo != GCNB_ALGO_GENERAL)
-    return stack_dw(xstack, y, argmax, dy, dy_is_mean, dW, db, s, bias_mode, relu, ws, st);
-  const bool fused_ok = layout != 2 && fused_bwd_supported(s, dx != nullptr);
-  if (layout == 1 && dx != nullptr && algo != GCNB_ALGO_GENERAL && fused_ok) {
-    // saved basis: the weight gradient is one streamed GEMM; the fused kernel only runs the adjoint recursion for dx
-    rc = stack_dw(xstack, y, argmax, dy, dy_is_mean, dW, db, s, bias_mode, relu, ws, st);
-    if (rc) return rc;
-    // dx = sum_k T_k(L~^T) dZ W_k^T: the tcgen05 forward kernel run on the transposed operator (cheb_fwd_umma.cu)
-    if (K > 1 && algo == GCNB_ALGO_AUTO && umma_adj_supported(s) && adjoint_umma_enabled())
-      return umma_cheb_adj(dy, dy_is_mean, y, argmax, *Lt, W, dx, s, relu, st);
-    Workspace ws2(static_cast<char*>(workspace) + align_up(ws.used, 256), workspace_bytes - align_up(ws.used, 256));
-    return fused_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, s, bias_mode, relu, dy_is_mean, true, ws2, st);
+  switch (pl.route) {
+    case ROUTE_STACK_DW:
+    case ROUTE_STACK_ADJ:
+    case ROUTE_STACK_FUSED_DX:
+      rc = stack_dw(xstack, y, argmax, dy, dy_is_mean, dW, db, s, bias_mode, relu, ws, st);
+      if (rc || pl.route == ROUTE_STACK_DW) return rc;
+      // dx = sum_k T_k(L~^T) dZ W_k^T: the tcgen05 forward kernel run on the transposed operator (cheb_fwd_umma.cu)
+      if (pl.route == ROUTE_STACK_ADJ) return umma_cheb_adj(dy, dy_is_mean, y, argmax, *Lt, W, dx, s, relu, st);
+      return fused_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, s, bias_mode, relu, dy_is_mean, true, ws1, st);
+    case ROUTE_FUSED_BWD:
+      return fused_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, s, bias_mode, relu, dy_is_mean, false, ws, st);
+    case ROUTE_GENERAL:
+      if (dy_is_mean) {
+        const long long pooled_rows = (long long)B * ceil_div(s.M, p);
+        float* full = ws1.take<float>((size_t)pooled_rows * Fout);
+        if (!full) {
+          set_error("gcnb_cheb_bwd_f32: workspace too small");
+          return GCNB_ERR_WORKSPACE;
+        }
+        rc = launch_mean_f_bwd(dy, full, pooled_rows, Fout, st);
+        if (rc) return rc;
+        dy = full;
+      }
+      return general_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, pl.layout == 2 ? xstack : nullptr, s,
+                              bias_mode, relu, ws, st);
+    default:
+      return plan_error("gcnb_cheb_bwd_f32", pl, s);
   }
-  if (algo == GCNB_ALGO_FUSED && !fused_ok) {
-    set_error("gcnb_cheb_bwd_f32: fused kernels do not support B=%d M=%d nnz=%d Fin=%d Fout=%d K=%d p=%d", B, s.M,
-              s.nnz, Fin, Fout, K, p);
-    return GCNB_ERR_INVALID;
-  }
-  if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && fused_ok))
-    return fused_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, s, bias_mode, relu, dy_is_mean, false, ws, st);
-  if (dy_is_mean) {  // the general path works on the full gradient: expand dy/Fout over the filters first
-    const long long pooled_rows = (long long)B * ceil_div(s.M, p);
-    float* full = ws.take<float>((size_t)pooled_rows * Fout);
-    if (!full) {
-      set_error("gcnb_cheb_bwd_f32: workspace too small");
-      return GCNB_ERR_WORKSPACE;
-    }
-    rc = launch_mean_f_bwd(dy, full, pooled_rows, Fout, st);
-    if (rc) return rc;
-    dy = full;
-  }
-  return general_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dx, dW, db, layout == 2 ? xstack : nullptr, s,
-                          bias_mode, relu, ws, st);
 }
 
 int gcnb_brelu_fwd_f32(const float* x, const float* bias, float* y, int B, int M, int F, int bias_mode,

@@ -179,7 +179,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdPara
 #define TRACEP() do { } while (0)
 #endif
   TRACEP();
-  pdl_trigger();  // the next kernel of the stream may start its own prologue as soon as SMs free up
   if ((sb & 1023u) != 0) __trap();  // the swizzled operand layouts need a 1 KB aligned base
   if (tid == 0) {
     mbar_init(bar_mma(0), 1); mbar_init(bar_mma(1), 1);
@@ -368,9 +367,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdPara
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
   TRACEP();
-  // Everything above read static data only (operator, taps, bias, permutation).  From here on the kernel reads the
-  // previous layer's output and writes its own: wait for the predecessor in the stream (programmatic dependent launch).
-  pdl_wait();
 
 #ifdef GCNB_TRACE
   int tr_n = 0;
@@ -1173,29 +1169,12 @@ struct UmmaFwdPlan {
       off_bias, off_bar, off_rp, off_img;
 };
 
-static bool umma_enabled() {
-  static const bool on = [] {
-    const char* v = std::getenv("GCNB_UMMA");
-    return !(v && v[0] == '0');
-  }();
-  return on;
-}
-
-static bool stage_enabled() {
-  static const bool on = [] {
-    const char* v = std::getenv("GCNB_STAGE");
-    return !(v && v[0] == '0');
-  }();
-  return on;
-}
-
 // ent_bytes < 0: the kernel builds its own (CSR-ordered) operator image in the prologue; otherwise the entry streams of
 // a host-built image take ent_bytes.
 static UmmaFwdPlan plan_umma_fwd(const LayerShape& s, int sm_count, int smem_optin, long long ent_bytes = -1) {
   UmmaFwdPlan pl{};
   pl.ok = false;
   pl.img = ent_bytes >= 0;
-  if (!umma_enabled()) return pl;
   if (s.Fin <= 8 || s.Fin > 32 || s.Fout < 4 || s.Fout > 32 || (s.Fout & 3)) return pl;
   if (s.p != 1 && s.p != 2 && s.p != 4 && s.p != 8) return pl;
   if (s.M % s.p != 0 || s.M < 1 || s.M > 2048 || s.K < 1 || s.B < 1) return pl;
@@ -1215,11 +1194,7 @@ static UmmaFwdPlan plan_umma_fwd(const LayerShape& s, int sm_count, int smem_opt
       pl.img ? 0 : 2 * (size_t)pl.NG * 16 + align_up((size_t)(s.M + 3) * 4, 16) + align_up((size_t)(s.M + 1) * 4, 16);
   const size_t budget = std::min<size_t>((size_t)smem_optin, 227 * 1024);
   double best = 1e30;
-  static const int ns_cap = [] {  // A/B knob: GCNB_UMMA_NS_MAX caps the window-slabs per tile
-    const char* v = std::getenv("GCNB_UMMA_NS_MAX");
-    return v ? std::max(1, std::atoi(v)) : 8;
-  }();
-  for (int ns = 1; ns <= std::min(8, ns_cap); ++ns) {
+  for (int ns = 1; ns <= 8; ++ns) {
     const int BQ = ns * pl.Q, T = ceil_div(BQ, 128);
     const int acc_cols = pl.G * s.p * T * 32;
     if (acc_cols > 512) continue;
@@ -1517,7 +1492,7 @@ static int umma_launch(const float* x, const int32_t* perm, int M_in, const gcnb
     // bulk copies need 16-byte aligned windows; the staged tile lies inside one state buffer, clear of its zero row
     const size_t wbytes = (size_t)M_in * s.Fin * 4;
     P.stage = !adj && (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (wbytes & 15) == 0 &&
-              (size_t)P.S * wbytes <= (size_t)s.p * pl.BQ * 128 && stage_enabled();
+              (size_t)P.S * wbytes <= (size_t)s.p * pl.BQ * 128;
   }
 #ifdef GCNB_TRACE
   P.debug = std::getenv("GCNB_UMMA_DEBUG") ? std::atoi(std::getenv("GCNB_UMMA_DEBUG")) : 0;
@@ -1526,7 +1501,7 @@ static int umma_launch(const float* x, const int32_t* perm, int M_in, const gcnb
 #define GCNB_UMMA_CASE(fp, mi, im, stk)                                                                                 \
   if (pl.FP == fp && pl.MAXI == mi && img == im && (P.nlayers > 1) == stk) {                                            \
     GCNB_CUDA(cudaFuncSetAttribute(k_cheb_fwd_umma<fp, mi, im, stk>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem)); \
-    GCNB_CUDA(launch_pdl(k_cheb_fwd_umma<fp, mi, im, stk>, dim3(grid), dim3(kThreads), pl.smem, st, P));                 \
+    k_cheb_fwd_umma<fp, mi, im, stk><<<grid, kThreads, pl.smem, st>>>(P);                                              \
   }
   GCNB_UMMA_CASE(16, 3, false, false) GCNB_UMMA_CASE(16, 5, false, false) GCNB_UMMA_CASE(32, 3, false, false)
   GCNB_UMMA_CASE(32, 5, false, false) GCNB_UMMA_CASE(16, 1, true, false) GCNB_UMMA_CASE(32, 1, true, false)

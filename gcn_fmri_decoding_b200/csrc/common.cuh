@@ -40,34 +40,6 @@ void count_launch();  // diagnostic counter behind gcnb_launch_count()
     }                                                                           \
   } while (0)
 
-// ---- programmatic dependent launch (PDL) ----------------------------------------------------------------------
-// The training step is a chain of dependent launches with ~3.5 us between them.  Kernels launched through
-// launch_pdl() may START while their predecessor in the stream is still running (as soon as every CTA of the
-// predecessor has executed pdl_trigger(), or exited) and must execute pdl_wait() before touching anything the
-// predecessor produces: the launch latency -- and, for the persistent forward kernels, the prologue that builds the
-// operator image from static data -- then overlaps the predecessor's tail.  pdl_wait() returns once the predecessor
-// grid has completed and its memory is visible; without the launch attribute both are no-ops.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-bool pdl_enabled();  // GCNB_PDL=1 turns the launch attribute on (off by default: see api.cu for the A/B numbers)
-
-template <class... KArgs, class... Args>
-static inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                     Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 __host__ __device__ static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline long long ceil_div_ll(long long a, long long b) { return (a + b - 1) / b; }

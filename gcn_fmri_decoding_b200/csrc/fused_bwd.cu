@@ -13,9 +13,7 @@
 // atomics: warps -> CTA through a shared-memory scratch (fixed order), CTAs -> a small second kernel.
 // The bias gradient is a separate two-stage column sum over the pooled tensors (also fixed order).
 #include <algorithm>
-#include <mutex>
 #include <cmath>
-#include <cstdlib>
 
 #include "fused_common.cuh"
 
@@ -45,7 +43,6 @@ struct BwdParams {
   int ntiles;
   int nchunks;     // MT*NT/2 accumulator chunks of 256 floats
   int off_opT, off_wfragT, off_dws, off_scratch, off_dz, off_slab;
-  int debug;  // profiling aid: bit0 skip sparse steps, bit1 skip dW contraction, bit2 skip reduction, bit3 skip dx phase
 };
 
 // MT = FP/16 (1 or 2) m-tiles over the input features, NT = FoP/8 n-tiles over the filters.
@@ -72,8 +69,7 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
   constexpr int NTF = MT * 2;  // n-tiles over the input features in the G contraction
   constexpr int NCH = MT * NT / 2;
 
-  // ---- once per CTA (static data only: runs ahead of the predecessor's completion under PDL) ------------------
-  pdl_trigger();
+  // ---- once per CTA ---------------------------------------------------------------------------------------------
   if (!P.skip_dw) build_operator(P.rowptr, P.col, P.val, G.M, G.Mpad, P.nnz, RS, opL);
   if (need_dx && P.K > 1) build_operator(P.rowptr_t, P.col_t, P.val_t, G.M, G.Mpad, P.nnz, RS, opT);
   if (need_dx) {
@@ -104,7 +100,6 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
 
   float dbacc = 0.f;  // this thread's filter (o = tid % FoP is the same in every iteration: FoP | blockDim)
 
-  pdl_wait();  // dy / y / arg-max (and everything this kernel writes) belong to the dependent part of the stream
   for (int tile = blockIdx.x; tile < P.ntiles; tile += gridDim.x) {
     const int b0 = tile * G.S;
     __syncthreads();
@@ -149,7 +144,7 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
       unsigned char* cur = (k & 1) ? slabB : slabA;
       if (k > 0) {
         const unsigned char* src = (k & 1) ? slabA : slabB;
-        if (!(P.debug & 1)) spmm_dispatch(G.LPR, opL, src, cur, G.Mpad, col_byte, rw, G.RW, k == 1 ? 1.f : 2.f, k > 1);
+        spmm_dispatch(G.LPR, opL, src, cur, G.Mpad, col_byte, rw, G.RW, k == 1 ? 1.f : 2.f, k > 1);
         __syncthreads();
       }
       float acc[MT][NT][4];
@@ -164,7 +159,7 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
       for (int a = 0; a < SLOTS; ++a) {
         const int tt = a / G.WS, s = a - tt * G.WS;
         const int rt = rw + tt * G.RW;
-        if (!(a < G.TPW * G.WS && rt < G.RT) || (P.debug & 2)) continue;
+        if (!(a < G.TPW * G.WS && rt < G.RT)) continue;
         const int scol = (sg * G.WS + s);
 #pragma unroll
         for (int h2 = 0; h2 < 2; ++h2) {
@@ -192,7 +187,7 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
       }
       // ---- warps -> CTA: fixed-order reduction through the scratch, two n-tiles (256 floats) per round --------
 #pragma unroll
-      for (int m = 0; m < ((P.debug & 4) ? 0 : MT); ++m) {
+      for (int m = 0; m < MT; ++m) {
 #pragma unroll
         for (int np = 0; np < NT / 2; ++np) {
           float* mine = scratch + (size_t)warp * 256 + lane;
@@ -221,7 +216,7 @@ __global__ void __launch_bounds__(896, 1) k_cheb_bwd_fused(const BwdParams P) {
     }
 
     // ---- phase B: dx by the Clenshaw form of the adjoint recursion ---------------------------------------------
-    if (need_dx && !(P.debug & 8)) {
+    if (need_dx) {
       const int KSo = FoP / 8;
       for (int k = P.K - 1; k >= 0; --k) {
         const int step = P.K - 1 - k;                       // 0, 1, 2, ...
@@ -327,8 +322,6 @@ __global__ void __launch_bounds__(256) k_dw_from_partials(const float* __restric
                                                            const float* __restrict__ db_part, float* __restrict__ db,
                                                            int FoP) {
   __shared__ float red[8][32];
-  pdl_trigger();
-  pdl_wait();
   const int NCH = MT * NT / 2;
   const int total = K * NCH * 256;
   const int ntot = total + (db_part != nullptr ? Fout : 0);
@@ -430,21 +423,6 @@ struct BwdPlan {
   int off_opT, off_wfragT, off_dws, off_scratch, off_dz, off_slab;
 };
 
-// Tuning / debugging knobs: each environment variable is read ONCE per process (first use) and cached.
-static int env_int_b(const char* name, int dflt) {
-  struct Slot { const char* name; int value; };
-  static Slot cache[16];
-  static int used = 0;
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lock(mu);
-  for (int i = 0; i < used; ++i)
-    if (cache[i].name == name) return cache[i].value;  // string literals: pointer identity is enough
-  const char* v = std::getenv(name);
-  const int val = v ? std::atoi(v) : dflt;
-  if (used < 16) cache[used++] = Slot{name, val};
-  return val;
-}
-
 static BwdPlan plan_bwd(const LayerShape& s, bool need_dx) {
   BwdPlan pl;
   pl.ok = false;
@@ -463,13 +441,10 @@ static BwdPlan plan_bwd(const LayerShape& s, bool need_dx) {
   const size_t op_bytes = operator_smem_bytes(g.Mpad, s.nnz);
   const size_t wfragT = need_dx ? (size_t)s.K * (pl.FoP / 8) * (pl.MT * 2) * 32 * 16 : 0;
   const size_t dws = (size_t)s.K * pl.nchunks * 256 * 4;
-  const int force_s = env_int_b("GCNB_BWD_S", 0), force_ws = env_int_b("GCNB_BWD_WS", 0);
   double best = -1;
   for (int S = 1; S <= 8; S *= 2) {
-    if (force_s && S != force_s) continue;
     if (S > s.B && S > 1) continue;
     for (int ws = 1; ws <= S; ws *= 2) {
-      if (force_ws && ws != force_ws) continue;
       const int cw = ws * g.FP;
       if (cw > 128) continue;
       const int sgn = S / ws;
@@ -529,8 +504,7 @@ int launch_dw_from_partials(const float* part, float* dW, int nblocks, int K, in
                             const float* db_part, float* db, int FoP, cudaStream_t st) {
   const int total = K * (MT * NT / 2) * 256;
   const int elems = total + (db_part != nullptr ? Fout : 0);
-  GCNB_CUDA(launch_pdl(k_dw_from_partials, dim3(ceil_div(elems, 32)), dim3(256), 0, st, part, dW, nblocks, K, MT, NT,
-                       Fin, Fout, db_part, db, FoP));
+  k_dw_from_partials<<<ceil_div(elems, 32), 256, 0, st>>>(part, dW, nblocks, K, MT, NT, Fin, Fout, db_part, db, FoP);
   GCNB_LAUNCH_CHECK("k_dw_from_partials");
   return GCNB_OK;
 }
@@ -570,7 +544,7 @@ template <int MT, int NT, int SLOTS>
 static int launch_bwd(const BwdParams& P, const BwdPlan& pl, int grid, cudaStream_t st) {
   auto kern = k_cheb_bwd_fused<MT, NT, SLOTS>;
   GCNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
-  GCNB_CUDA(launch_pdl(kern, dim3(grid), dim3(pl.g.nwarps * 32), pl.smem, st, P));
+  kern<<<grid, pl.g.nwarps * 32, pl.smem, st>>>(P);
   GCNB_LAUNCH_CHECK("k_cheb_bwd_fused");
   return GCNB_OK;
 }
@@ -609,7 +583,6 @@ int fused_cheb_bwd(const float* x, const int32_t* perm, int M_in, const float* y
   P.g = pl.g; P.FoP = pl.FoP; P.RSz = pl.RSz; P.ntiles = ntiles; P.nchunks = pl.nchunks;
   P.off_opT = pl.off_opT; P.off_wfragT = pl.off_wfragT; P.off_dws = pl.off_dws; P.off_scratch = pl.off_scratch;
   P.off_dz = pl.off_dz; P.off_slab = pl.off_slab;
-  P.debug = env_int_b("GCNB_BWD_DEBUG", 0);
   rc = GCNB_ERR_INVALID;
 #define GCNB_BWD_CASE(mt, nt, sl) \
   if (pl.MT == mt && pl.NT == nt && pl.SLOTS == sl) rc = launch_bwd<mt, nt, sl>(P, pl, grid, st);

@@ -4,9 +4,7 @@
 // layout transposes and the pre-pool activation of the reference (models_gcn.py:598-617, 619-639)
 // never exist in memory.  See fused_common.cuh for the CTA layout.
 #include <algorithm>
-#include <mutex>
 #include <cmath>
-#include <cstdlib>
 
 #include "fused_common.cuh"
 
@@ -33,7 +31,6 @@ struct FwdParams {
   int off_stage;            // raw staging buffer for the TMA bulk prefetch of the next tile (0 = none)
   int off_misc;             // int src_row[Mpad] (gather table, -1 = zero row) followed by float bias_f[64]
   int log2p;
-  int debug;  // profiling aid: bit0 skip sparse step, bit1 skip contraction, bit2 skip stores
 };
 
 // register-heavy instances (many accumulator fragments) run with at most 16 warps
@@ -140,7 +137,6 @@ __global__ void __launch_bounds__((SLOTS * NT > 8) ? 512 : 896, 1) k_cheb_fwd_fu
 
     // Contraction of the warp's own row tiles of X_k (in slab `cur`) with the taps of order k.
     auto contract = [&](int k, const unsigned char* cur) {
-      if (P.debug & 2) return;
       const float4* wk = wfrag + (size_t)k * KS * NT * 32 + lane;
       const float* curf = reinterpret_cast<const float*>(cur) + g * RS + sg * G.WS * FP + t;
       for (int ks = 0; ks < KS; ++ks) {
@@ -196,7 +192,7 @@ __global__ void __launch_bounds__((SLOTS * NT > 8) ? 512 : 896, 1) k_cheb_fwd_fu
       const unsigned char* prev = (k & 1) ? slabA : slabB;  // X_{k-1}
       spill(k - 1, prev);
       if (warp & 1) contract(k - 1, prev);
-      if (!(P.debug & 1)) spmm_dispatch(G.LPR, op, prev, cur, G.Mpad, col_byte, rw, G.RW, k == 1 ? 1.f : 2.f, k > 1);
+      spmm_dispatch(G.LPR, op, prev, cur, G.Mpad, col_byte, rw, G.RW, k == 1 ? 1.f : 2.f, k > 1);
       if (!(warp & 1)) contract(k - 1, prev);
       group_barrier(sg, G.RW * 32);  // X_k complete for this sample group's columns
     }
@@ -214,7 +210,7 @@ __global__ void __launch_bounds__((SLOTS * NT > 8) ? 512 : 896, 1) k_cheb_fwd_fu
         const int tt = a / G.WS, s = a - tt * G.WS;
         const int rt = rw + tt * G.RW;
         const int b = b0 + sg * G.WS + s;
-        const bool live = (a < G.TPW * G.WS) && rt < G.RT && b < P.B && !(P.debug & 4);  // warp-uniform
+        const bool live = (a < G.TPW * G.WS) && rt < G.RT && b < P.B;  // warp-uniform
         if (!live) continue;
         // own 16 rows, own column range (warps of other sample groups share the rows): CW = WS*FP >= 32 columns
         float* tile_s = fs + (size_t)rt * 16 * RS + sg * G.WS * FP;
@@ -276,21 +272,6 @@ struct FwdPlan {
   bool staged;
 };
 
-// Tuning / debugging knobs: each environment variable is read ONCE per process (first use) and cached.
-static int env_int(const char* name, int dflt) {
-  struct Slot { const char* name; int value; };
-  static Slot cache[16];
-  static int used = 0;
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lock(mu);
-  for (int i = 0; i < used; ++i)
-    if (cache[i].name == name) return cache[i].value;  // string literals: pointer identity is enough
-  const char* v = std::getenv(name);
-  const int val = v ? std::atoi(v) : dflt;
-  if (used < 16) cache[used++] = Slot{name, val};
-  return val;
-}
-
 // M_in: vertices of the raw input (differs from M when the permutation gather is fused in).
 static FwdPlan plan_fwd(const LayerShape& s, int M_in, bool x_aligned16) {
   FwdPlan pl;
@@ -310,12 +291,9 @@ static FwdPlan plan_fwd(const LayerShape& s, int M_in, bool x_aligned16) {
   // Candidates: WS samples per warp (CW = WS*FP columns in {32,64,128}) x SG sample groups.
   // Prefer the configuration with the fewest shared-memory wavefronts per nonzero (large CW), subject to
   // registers (SLOTS*NT accumulator fragments), warps (<= 28, or <= 16 for heavy instances) and smem.
-  const int force_ws = env_int("GCNB_FWD_WS", 0), force_sg = env_int("GCNB_FWD_SG", 0);
   double best_score = -1;
   for (int ws = 32 / g.FP; ws * g.FP <= 128; ws *= 2) {
-    if (force_ws && ws != force_ws) continue;
     for (int sgn = 1; sgn <= 8; ++sgn) {
-      if (force_sg && sgn != force_sg) continue;
       const int S = ws * sgn;
       if (S > s.B && !(ws == 32 / g.FP && sgn == 1)) continue;
       const int RS = S * g.FP + 4;
@@ -323,11 +301,10 @@ static FwdPlan plan_fwd(const LayerShape& s, int M_in, bool x_aligned16) {
       if (need > kSmemBudget) continue;
       // staging buffer for the bulk prefetch: only when a window is a multiple of 16 bytes and it fits
       const size_t stage_bytes = 16 + (size_t)S * M_in * s.Fin * 4;
-      const bool can_stage = x_aligned16 && ((long long)M_in * s.Fin) % 4 == 0 && need + stage_bytes <= kSmemBudget &&
-                             env_int("GCNB_FWD_NOSTAGE", 0) == 0;
+      const bool can_stage = x_aligned16 && ((long long)M_in * s.Fin) % 4 == 0 && need + stage_bytes <= kSmemBudget;
       if (can_stage) need += stage_bytes;
       for (int heavy = 0; heavy < 2; ++heavy) {
-        const int maxw = heavy ? 16 : env_int("GCNB_FWD_MAXW", 28);
+        const int maxw = heavy ? 16 : 28;
         int rwn = std::min(g.RT, maxw / sgn);
         if (rwn < 1) continue;
         const int tpw = ceil_div(g.RT, rwn);
@@ -402,7 +379,6 @@ int fused_cheb_fwd(const float* x, const int32_t* perm, int M_in, const gcnb_csr
   P.ntiles = ceil_div(s.B, pl.g.S);
   P.off_wfrag = pl.off_wfrag; P.off_slab = pl.off_slab; P.off_stage = pl.off_stage; P.off_misc = pl.off_misc;
   P.log2p = 0;
-  P.debug = env_int("GCNB_FWD_DEBUG", 0);
   while ((1 << P.log2p) < s.p) ++P.log2p;
 #define GCNB_FWD_CASE(nt, sl) \
   if (pl.NT == nt && pl.SLOTS == sl) return launch_fwd<nt, sl>(P, pl, st);

@@ -165,8 +165,6 @@ __global__ void __launch_bounds__(1024) k_colsum_multi(ColsumArgs a) {
 __global__ void k_adam_tf(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                           const uint8_t* __restrict__ decay, const float* __restrict__ state, long long n, float b1,
                           float b2, float eps, float reg, float gscale) {
-  pdl_trigger();
-  pdl_wait();
   const float lr_t = state[2];
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float pi = p[i];
@@ -251,8 +249,7 @@ int gcnb_adam_tf_f32(float* p, const float* g, float* m, float* v, const uint8_t
     GCNB_LAUNCH_CHECK("k_adam_tick");
   }
   const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(ceil_div_ll(n, 256), 148 * 8));
-  GCNB_CUDA(launch_pdl(k_adam_tf, dim3(grid), dim3(256), 0, st, p, (const float*)g, m, v, decay, (const float*)state, n,
-                       beta1, beta2, eps, reg, gscale));
+  k_adam_tf<<<grid, 256, 0, st>>>(p, g, m, v, decay, state, n, beta1, beta2, eps, reg, gscale);
   GCNB_LAUNCH_CHECK("k_adam_tf");
   return GCNB_OK;
 }

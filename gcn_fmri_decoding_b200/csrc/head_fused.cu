@@ -270,7 +270,6 @@ __device__ __noinline__ void colsum32(float* red /* [8][32] */, const float* X, 
 
 __global__ void __launch_bounds__(HT, 1) k_head_step(const HeadParams P) {
   cg::grid_group grid = cg::this_grid();
-  pdl_trigger();  // the first backward kernel may be scheduled as soon as SMs free up; it waits for this grid
   HTRACE(0);
   // one shared buffer, three views: the GEMM tiles, the staging of the narrow products, rows of h2 (+ W3)
   __shared__ __align__(16) float smem_f[16 * 16 * 33];

@@ -15,7 +15,6 @@
 //
 // Summation order = CSR order with fmaf, the same as k_spmm_step (general.cu), so both give identical bits.
 // Reference math: graph.chebyshev recursion, lib_new/graph.py:163-171 / models_gcn.py:600-609.
-#include <cstdlib>
 
 #include "fused_common.cuh"
 
@@ -257,14 +256,6 @@ bool plan_spmm(long long C, int* CW, int* nchunk, int* NS, uint32_t* stage_bytes
   return true;
 }
 
-bool tma_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("GCNB_SPMM_TMA");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 }  // namespace
 
 bool spmm_tma_supported(const gcnb_csr& L, long long C, const float* src, const float* add, const float* add2,
@@ -274,7 +265,7 @@ bool spmm_tma_supported(const gcnb_csr& L, long long C, const float* src, const 
   size_t smem;
   const uintptr_t bits = reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(add) |
                          reinterpret_cast<uintptr_t>(add2) | reinterpret_cast<uintptr_t>(out);
-  return tma_enabled() && L.M >= 1 && (bits & 15) == 0 && src != out && (add != nullptr || add2 == nullptr) && plan_spmm(C, &CW, &nchunk, &NS, &sb, &smem);
+  return L.M >= 1 && (bits & 15) == 0 && src != out && (add != nullptr || add2 == nullptr) && plan_spmm(C, &CW, &nchunk, &NS, &sb, &smem);
 }
 
 int spmm_tma(const gcnb_csr& L, const float* src, const float* add, const float* add2, float* out, long long C,

@@ -41,8 +41,6 @@ template <int K, int MT, int NT>
 // light instances (<= 20 accumulator fragments) run two CTAs per SM: one CTA's loads hide behind the other's MMAs
 __global__ void __launch_bounds__(256, (K * MT * NT > 20) ? 1 : 2) k_dw_from_stack(const StackDwParams P) {
   extern __shared__ __align__(16) unsigned char smem[];
-  pdl_trigger();
-  pdl_wait();  // dy (and the basis) come from the predecessor in the stream
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int CR = P.CR, SX = P.SX, SZ = P.SZ, FP = P.FP, NS = P.NS;
@@ -261,7 +259,7 @@ template <int K, int MT, int NT>
 static int launch_stack(const StackDwParams& P, const StackPlan& pl, int grid, cudaStream_t st) {
   auto kern = k_dw_from_stack<K, MT, NT>;
   GCNB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
-  GCNB_CUDA(launch_pdl(kern, dim3(grid), dim3(256), pl.smem, st, P));
+  kern<<<grid, 256, pl.smem, st>>>(P);
   GCNB_LAUNCH_CHECK("k_dw_from_stack");
   return GCNB_OK;
 }

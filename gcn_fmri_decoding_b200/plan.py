@@ -8,7 +8,6 @@
 from __future__ import annotations
 
 import ctypes as C
-import os
 import weakref
 
 import numpy as np
@@ -73,9 +72,9 @@ class GraphPlan:
         return self._images[key]
 
 
-# GCNB_IMAGE=0 (or plan.USE_IMAGES = False): never attach operator images -- the kernels then build their own CSR-ordered
-# work lists in every launch (A/B runs, and the tests that cover that path)
-USE_IMAGES = os.environ.get("GCNB_IMAGE", "1") != "0"
+# plan.USE_IMAGES = False: never attach operator images -- the kernels then build their own CSR-ordered work lists in
+# every launch (the tests that cover callers passing no image set it)
+USE_IMAGES = True
 
 # device address of a plan's value array -> (plan, is-transpose, tensor version at upload); lets csr_struct find the
 # plan (hence the cached operator images) behind the raw tensors the custom ops are called with

@@ -287,13 +287,10 @@ class FusedTrainer:
         # world > 1: the gradient average is fused into the optimiser kernel (gcnb_adam_tf_allreduce_f32): the flat
         # gradient buffers then live in peer-mapped symmetric memory, two of them used on alternate steps (a peer may
         # still be reading the previous one).  Falls back to one NCCL all-reduce when symmetric memory is unavailable.
-        import os
         self.allreduce_kind = "none"
         self._peer = None
-        # diagnostic only (timing the step without its collective; the replicas then drift apart)
-        self._skip_allreduce = os.environ.get("GCNB_DP_SKIP_ALLREDUCE") == "1"
         gbufs = None
-        if self.world > 1 and not self._skip_allreduce:
+        if self.world > 1:
             self.allreduce_kind = "nccl"
             if peer_allreduce and dev.type == "cuda":
                 try:
@@ -463,7 +460,7 @@ class FusedTrainer:
                                                 self._peer["flags"], self._peer["rank"], self.world, stream)
             self._lib.check(rc, "gcnb_adam_tf_allreduce_f32")
             return self._loss, logits
-        if self.world > 1 and not self._skip_allreduce:
+        if self.world > 1:
             dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM)
         rc = lib.gcnb_adam_tf_f32(vp(self.flat_p), vp(self.flat_g), vp(self.flat_m), vp(self.flat_v), vp(self.decay),
                                   vp(self.state), self.n, self.lr, self.b1, self.b2, self.eps,

@@ -79,8 +79,12 @@ GCNB_API unsigned long long gcnb_launch_count(void);
 /* 1 if the fused shared-memory kernels can take this layer shape, else 0 (no reference counterpart: dispatch query). */
 GCNB_API int gcnb_cheb_fused_supported(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx);
 
-/* Human-readable description of the forward kernel AUTO dispatch picks for this shape (diagnostics, bench records). */
-GCNB_API int gcnb_cheb_fwd_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, char* out, size_t n);
+/* Human-readable description of the route gcnb_cheb_fwd_f32 (backward = 0) or gcnb_cheb_bwd_f32 (backward = 1) takes
+ * for this shape: "<route>: <its kernels>" (diagnostics, bench records).  saved_basis: the call passes `xstack`.
+ * route_workspace_bytes (nullable) receives the workspace that route takes; gcnb_cheb_workspace_bytes is the largest
+ * of these over saved_basis = 0 and 1. */
+GCNB_API int gcnb_cheb_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx,
+                                int saved_basis, int algo, char* out, size_t n, size_t* route_workspace_bytes);
 
 /*
  * Operator image of a layer (see gcnb_csr.image) -- the counterpart of turning the rescaled Laplacian into a
@@ -122,7 +126,8 @@ GCNB_API int gcnb_cheb_tap_image_build(const float* W_host, int Fin, int Fout, i
  * graphs on the general path), or 0 when this shape keeps no basis. */
 GCNB_API int gcnb_cheb_stack_width(int B, int M, int nnz, int Fin, int Fout, int K, int p);
 
-/* Bytes of workspace gcnb_cheb_{fwd,bwd}_f32 need for this shape (256-byte aligned pointer). */
+/* Bytes of workspace gcnb_cheb_{fwd,bwd}_f32 need for this shape and algo, with or without a saved basis (256-byte
+ * aligned pointer). */
 GCNB_API size_t gcnb_cheb_workspace_bytes(int B, int M, int nnz, int Fin, int Fout, int K, int p, int backward, int need_dx,
                                  int algo);
 

@@ -429,12 +429,17 @@ def test_product_never_imports_the_oracle():
 def test_planner_queries_over_random_shapes():
     """The host-side planners (dispatch / workspace / basis-width / describe queries) over 400 seeded random layer shapes,
     including degenerate and oversized ones: they never fail, answer deterministically, and agree with each other --
-    the AUTO workspace is that of one of the two kernel families, sizes are multiples of 256 bytes,
-    the saved-basis width is 0, Fin, or Fin padded to a power of two, and the description names a kernel."""
+    every call (saved basis or not, with or without dx, each algo) takes one of the enumerated routes and the workspace
+    query covers that route, the AUTO workspace is no larger than the larger of the two kernel families', sizes are
+    multiples of 256 bytes, the saved-basis width is 0, Fin, or Fin padded to a power of two, and the forward
+    description names a kernel."""
     from gcn_fmri_decoding_b200 import _lib
 
     lib = _lib.lib()
     rng = np.random.RandomState(77)
+    routes = {0: ("k_cheb_fwd_umma<FP=16>", "k_cheb_fwd_umma<FP=32>", "k_cheb_fwd_fused", "general path", "unsupported"),
+              1: ("stack-dW", "stack-dW + tcgen05 adjoint", "stack-dW + fused dx", "fused recompute", "general path",
+                  "unsupported")}
     seen_fused = seen_general = 0
     for _ in range(400):
         B = int(rng.choice([1, 2, 7, 16, 64, 128, 512, 600]))
@@ -452,8 +457,13 @@ def test_planner_queries_over_random_shapes():
             general = lib.gcnb_cheb_workspace_bytes(*shape, bwd, dx, _lib.ALGO_GENERAL)
             fused_ws = lib.gcnb_cheb_workspace_bytes(*shape, bwd, dx, _lib.ALGO_FUSED)
             assert 0 <= auto < 2 ** 48 and 0 <= general < 2 ** 48 and 0 <= fused_ws < 2 ** 48
-            assert auto in (fused_ws, general), (shape, bwd, dx, auto, fused_ws, general)
+            assert auto <= max(fused_ws, general), (shape, bwd, dx, auto, fused_ws, general)
             assert auto % 256 == 0 and general % 256 == 0
+            for algo, query in ((_lib.ALGO_AUTO, auto), (_lib.ALGO_GENERAL, general), (_lib.ALGO_FUSED, fused_ws)):
+                for saved in (False, True):
+                    text, need = _lib.describe(*shape, bwd, dx, saved, algo)
+                    assert text.split(":")[0] in routes[bwd], (shape, bwd, dx, saved, algo, text)
+                    assert need <= query and need % 256 == 0, (shape, bwd, dx, saved, algo, text, need, query)
         width = lib.gcnb_cheb_stack_width(*shape)
         assert width == 0 or (width >= Fin and width in (Fin, 8, 16, 32, 64)), (shape, width)
         text = _lib.describe_fwd(*shape)

@@ -7,7 +7,6 @@ fp32 rounding, either decision is correct, and the one taken moves a whole gradi
 the device's decisions are admissible (``check_decisions``, built on ``check_argmax``) and then compares the gradients
 with the oracle routed through those same decisions (``conv_stack_bwd(decisions=...)``).
 """
-import os
 import re
 import time
 
@@ -28,7 +27,7 @@ RELU_GAP = 1e-5   # a ReLU decision may differ from fp64 only where |window-max 
 # at most 296 CTAs (stack_dw.cu), at most 3 stages
 RING_ROWS = 128 * 296
 
-STACK_DW, STACK_ADJ, STACK_FUSED, GENERAL = "stack-dW", "stack-dW + tcgen05 adjoint", "stack-dW + fused dx", "general"
+STACK_DW, STACK_ADJ, STACK_FUSED, GENERAL = "stack-dW", "stack-dW + tcgen05 adjoint", "stack-dW + fused dx", "general path"
 
 
 @pytest.fixture(scope="module")
@@ -43,29 +42,15 @@ def T(a, dev, dtype=torch.float32):
 
 
 def backward_route(B, M, nnz, Fin, Fout, K, p, need_dx, algo):
-    """Which backward ``gcnb_cheb_bwd_f32`` runs after ``cheb_fwd_mean(..., want_stack=True)``, from the library's own
-    dispatch queries (the conditions of its saved-basis branch, api.cu)."""
+    """Which backward ``gcnb_cheb_bwd_f32`` runs after ``cheb_fwd_mean(..., want_stack=True)``, as the library names it."""
     from gcn_fmri_decoding_b200 import _lib
 
-    lib = _lib.lib()
-    if algo == _lib.ALGO_GENERAL:
-        return GENERAL                          # cheb_fwd_mean keeps no basis for the general path
-    width = lib.gcnb_cheb_stack_width(B, M, nnz, Fin, Fout, K, p)
-    if width == 0:
-        return "fused recompute"                # no basis kept at all: not a saved-basis route
-    saved = lib.gcnb_cheb_fused_supported(B, M, nnz, Fin, Fout, K, p, 0, 0)   # else the general path's vertex-major basis
-    if saved and not need_dx:
-        return STACK_DW
-    if saved and lib.gcnb_cheb_fused_supported(B, M, nnz, Fin, Fout, K, p, 1, 1):
-        if (K > 1 and algo == _lib.ALGO_AUTO and Fin % 4 == 0 and Fout % 4 == 0 and os.environ.get("GCNB_UMMA_ADJ", "1")[:1] != "0"
-                and "tcgen05" in _lib.describe_fwd(B, M, nnz, Fout, Fin, K, 1)):
-            return STACK_ADJ
-        return STACK_FUSED
-    return GENERAL
+    saved = algo != _lib.ALGO_GENERAL and _lib.lib().gcnb_cheb_stack_width(B, M, nnz, Fin, Fout, K, p) > 0  # kept basis
+    return _lib.describe(B, M, nnz, Fin, Fout, K, p, True, need_dx, saved, algo)[0].split(":")[0]
 
 
 def tiles(B, M, nnz, Fin, Fout, K, p):
-    """Tiles of the k_cheb_fwd_umma launch for this shape (the last number of gcnb_cheb_fwd_describe)."""
+    """Tiles of the k_cheb_fwd_umma launch for this shape (the last number of the forward description)."""
     from gcn_fmri_decoding_b200 import _lib
 
     d = _lib.describe_fwd(B, M, nnz, Fin, Fout, K, p)
@@ -197,7 +182,9 @@ def _random_saved_basis_cases(n=28, seed=4257):
     return cases
 
 
-SWEEP = _random_saved_basis_cases()
+# a graph the fused forward cannot hold keeps the general path's basis; its backward is the general path, also where the
+# fused backward would fit the shape (the workspace query must cover it)
+SWEEP = _random_saved_basis_cases() + [(0, 2048, 7, 24, 3, 8, "b1relu", False, True)]
 
 
 @pytest.mark.parametrize("lvl,B,Fin,Fout,K,p,brelu,need_dx,dy_is_mean", SWEEP)
