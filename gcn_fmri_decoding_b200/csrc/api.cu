@@ -118,6 +118,20 @@ __global__ void k_mpool_bwd(const float* __restrict__ dy, const uint8_t* __restr
   }
 }
 
+// the adjoint of k_perm_gather for a permutation: dx[b][perm[m]] = dxp[b][m] where perm[m] < M_in (every raw row is
+// written exactly once, the rows of fake vertices are dropped)
+__global__ void k_perm_scatter(const float* __restrict__ dxp, const int32_t* __restrict__ perm, float* __restrict__ dx,
+                               int B, int M, int M_in, int F) {
+  const long long total = (long long)B * M * F;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int f = (int)(i % F);
+    const int m = (int)((i / F) % M);
+    const int b = (int)(i / ((long long)F * M));
+    const int dst = perm[m];
+    if (dst >= 0 && dst < M_in) dx[((long long)b * M_in + dst) * F + f] = dxp[i];
+  }
+}
+
 __global__ void k_perm_gather(const float* __restrict__ x, const int32_t* __restrict__ perm, float* __restrict__ y,
                               int B, int M_in, int M_out, int F) {
   const long long total = (long long)B * M_out * F;
@@ -195,6 +209,8 @@ enum ChebRoute {
   ROUTE_STACK_ADJ,       // ... and dx through k_cheb_fwd_umma on L~^T
   ROUTE_STACK_FUSED_DX,  // ... and dx through k_cheb_bwd_fused
   ROUTE_FUSED_BWD,       // k_cheb_bwd_fused recomputes the basis
+  ROUTE_ADJ_ONLY,        // input gradient only: k_cheb_fwd_umma (RAW) on L~^T, any input width, un-permuted in its store
+  ROUTE_FUSED_DX,        // input gradient only: k_cheb_bwd_fused without the weight gradient
 };
 
 struct ChebPlan {
@@ -202,19 +218,36 @@ struct ChebPlan {
   // saved basis of the shape (only when the call passes one): 1 = the fused kernels' [K][B][M][FP], 2 = the general
   // path's vertex-major [K][M][B][Fin] for graphs the fused kernels cannot hold, 0 = none exists
   int layout;
-  size_t region[2];  // workspace regions of the route, in order; each a multiple of 256 bytes
+  // workspace regions of the route, in order; each a multiple of 256 bytes.  The input-gradient-only routes that run a
+  // backward kernel (dx_only) put its unwanted weight gradient in region 2 and the permuted dx in region 3.
+  size_t region[4];
   const char* why;   // ROUTE_UNSUPPORTED: the reason, NULL when the fused kernels do not fit the shape
-  size_t total() const { return region[0] + region[1]; }
+  size_t total() const { return region[0] + region[1] + region[2] + region[3]; }
 };
 
-static ChebPlan plan_cheb(const LayerShape& s, bool backward, bool need_dx, bool saved, int algo) {
-  ChebPlan pl{ROUTE_UNSUPPORTED, 0, {0, 0}, nullptr};
-  auto route = [&pl](ChebRoute r, size_t a, size_t b = 0) {
+// dx_only (backward, need_dx, no saved basis): the input gradient alone, gcnb_cheb_dx_f32
+static ChebPlan plan_cheb(const LayerShape& s, bool backward, bool need_dx, bool saved, int algo, bool dx_only = false) {
+  ChebPlan pl{ROUTE_UNSUPPORTED, 0, {0, 0, 0, 0}, nullptr};
+  auto route = [&pl](ChebRoute r, size_t a, size_t b = 0, size_t c = 0, size_t d = 0) {
     pl.route = r;
     pl.region[0] = a;
     pl.region[1] = b;
+    pl.region[2] = c;
+    pl.region[3] = d;
     return pl;
   };
+  if (dx_only) {
+    // the tcgen05 adjoint takes any input width; ALGO_FUSED keeps dx on k_cheb_bwd_fused, as in the full backward
+    if (algo == GCNB_ALGO_AUTO && umma_adj_raw_supported(s)) return route(ROUTE_ADJ_ONLY, 0);
+    const size_t dxp = align_up((size_t)s.B * s.M * s.Fin * sizeof(float), 256) + 256;
+    const bool bwd_ok = fused_bwd_supported(s, true);
+    if (algo == GCNB_ALGO_FUSED && !bwd_ok) return pl;
+    if (algo == GCNB_ALGO_FUSED || (algo == GCNB_ALGO_AUTO && bwd_ok))
+      return route(ROUTE_FUSED_DX, fused_cheb_workspace(s, true, true), 0, 0, dxp);
+    return route(ROUTE_GENERAL, general_cheb_workspace(s, true, true),
+                 align_up((size_t)s.B * ceil_div(s.M, s.p) * s.Fout * sizeof(float), 256) + 256,
+                 align_up((size_t)s.Fin * s.K * s.Fout * sizeof(float), 256) + 256, dxp);
+  }
   const bool fwd_ok = fused_fwd_supported(s);
   if (saved) pl.layout = fwd_ok ? (stack_dw_supported(s) ? 1 : 0) : 2;
   if (!backward) {
@@ -253,7 +286,8 @@ static ChebPlan plan_cheb(const LayerShape& s, bool backward, bool need_dx, bool
 
 // region i of the plan in the caller's workspace
 static Workspace plan_region(const ChebPlan& pl, int i, void* workspace, size_t bytes) {
-  const size_t off = i == 0 ? 0 : pl.region[0];
+  size_t off = 0;
+  for (int r = 0; r < i; ++r) off += pl.region[r];
   if (workspace == nullptr || off >= bytes) return Workspace(nullptr, 0);
   return Workspace(static_cast<char*>(workspace) + off, std::min(pl.region[i], bytes - off));
 }
@@ -302,7 +336,7 @@ using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 101; }
+int gcnb_version(void) { return 102; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 
@@ -457,6 +491,86 @@ int gcnb_cheb_bwd_f32(const float* x, const int32_t* perm, int M_in, const float
     default:
       return plan_error("gcnb_cheb_bwd_f32", pl, s);
   }
+}
+
+int gcnb_cheb_dx_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, int algo, char* out, size_t n,
+                          size_t* workspace_bytes) {
+  if (!out || n == 0) return GCNB_ERR_INVALID;
+  LayerShape s{B, M, nnz, Fin, Fout, K, p};
+  const ChebPlan pl = plan_cheb(s, true, true, false, algo, true);
+  switch (pl.route) {
+    case ROUTE_ADJ_ONLY: {
+      const int w = snprintf(out, n, "tcgen05 adjoint only: ");
+      if (w >= 0 && (size_t)w < n) umma_adj_describe(s, out + w, n - w);
+      break;
+    }
+    case ROUTE_FUSED_DX:
+      snprintf(out, n, "fused dx: k_cheb_bwd_fused without the weight gradient, k_perm_scatter with perm");
+      break;
+    case ROUTE_GENERAL:
+      snprintf(out, n, "general path: HBM-resident state (k_spmm_tma, k_dz_wt for dx; dW to scratch), k_perm_scatter "
+                       "with perm");
+      break;
+    default:
+      plan_describe(pl, s, true, out, n);
+  }
+  if (workspace_bytes) *workspace_bytes = pl.total();
+  return GCNB_OK;
+}
+
+int gcnb_cheb_dx_f32(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax,
+                     const float* dy, int dy_is_mean, const gcnb_csr* L, const gcnb_csr* Lt, const float* W, float* dx,
+                     int B, int Fin, int Fout, int K, int p, int relu, int algo, void* workspace, size_t workspace_bytes,
+                     gcnb_stream_t stream) {
+  int rc = check_layer("gcnb_cheb_dx_f32", L, B, Fin, Fout, K, p, GCNB_BIAS_NONE, nullptr);
+  if (rc) return rc;
+  GCNB_REQUIRE(y && dy && W && dx, "gcnb_cheb_dx_f32: y, dy, W and dx must not be NULL");
+  GCNB_REQUIRE(p == 1 || argmax != nullptr, "gcnb_cheb_dx_f32: argmax is required when p > 1");
+  GCNB_REQUIRE(M_in >= 1 && (perm != nullptr || M_in == L->M),
+               "gcnb_cheb_dx_f32: without perm, M_in (%d) must equal M (%d)", M_in, L->M);
+  GCNB_REQUIRE(K == 1 || (Lt && Lt->M == L->M && Lt->nnz == L->nnz),
+               "gcnb_cheb_dx_f32: needs the transposed operator Lt with the same M and nnz");
+  LayerShape s{B, L->M, L->nnz, Fin, Fout, K, p};
+  const ChebPlan pl = plan_cheb(s, true, true, false, algo, true);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (pl.route == ROUTE_ADJ_ONLY) {
+    // K = 1 applies no operator: L only provides the kernel's row tables (its image belongs to the forward shape)
+    gcnb_csr op = Lt ? *Lt : *L;
+    if (!Lt) op.image = nullptr, op.image_bytes = 0;
+    return umma_cheb_adj_raw(dy, dy_is_mean, y, argmax, op, W, dx, perm, M_in, s, relu, st);
+  }
+  if (pl.route != ROUTE_FUSED_DX && pl.route != ROUTE_GENERAL) return plan_error("gcnb_cheb_dx_f32", pl, s);
+  GCNB_REQUIRE(pl.route != ROUTE_GENERAL || x != nullptr,
+               "gcnb_cheb_dx_f32: the general path recomputes the Chebyshev basis and needs x");
+  Workspace ws = plan_region(pl, 0, workspace, workspace_bytes), ws1 = plan_region(pl, 1, workspace, workspace_bytes);
+  Workspace ws2 = plan_region(pl, 2, workspace, workspace_bytes), ws3 = plan_region(pl, 3, workspace, workspace_bytes);
+  float* dxp = perm ? ws3.take<float>((size_t)B * s.M * Fin) : dx;  // gradient w.r.t. the permuted input
+  if (!dxp) {
+    set_error("gcnb_cheb_dx_f32: workspace too small");
+    return GCNB_ERR_WORKSPACE;
+  }
+  if (pl.route == ROUTE_FUSED_DX) {
+    rc = fused_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dxp, nullptr, nullptr, s, GCNB_BIAS_NONE, relu, dy_is_mean,
+                        true, ws, st);
+  } else {
+    float* dW = ws2.take<float>((size_t)Fin * K * Fout);
+    float* full = dy_is_mean ? ws1.take<float>((size_t)B * ceil_div(s.M, p) * Fout) : nullptr;
+    if (!dW || (dy_is_mean && !full)) {
+      set_error("gcnb_cheb_dx_f32: workspace too small");
+      return GCNB_ERR_WORKSPACE;
+    }
+    if (dy_is_mean) {
+      rc = launch_mean_f_bwd(dy, full, (long long)B * ceil_div(s.M, p), Fout, st);
+      if (rc) return rc;
+      dy = full;
+    }
+    rc = general_cheb_bwd(x, perm, M_in, y, argmax, dy, *L, Lt, W, dxp, dW, nullptr, nullptr, s, GCNB_BIAS_NONE, relu, ws,
+                          st);
+  }
+  if (rc || !perm) return rc;
+  k_perm_scatter<<<grid_for((long long)B * s.M * Fin), 256, 0, st>>>(dxp, perm, dx, B, s.M, M_in, Fin);
+  GCNB_LAUNCH_CHECK("k_perm_scatter");
+  return GCNB_OK;
 }
 
 int gcnb_brelu_fwd_f32(const float* x, const float* bias, float* y, int B, int M, int F, int bias_mode,

@@ -141,8 +141,11 @@ struct UmmaFwdParams {
 };
 
 // ---------------------------------------------------------------------------------------------------------------
-// STACK: the layer-stack variant (UmmaFwdParams::nlayers > 1); the single-layer instances carry none of its code
-template <int FP, int MAXI, bool IMG, bool STACK>
+// STACK: the layer-stack variant (UmmaFwdParams::nlayers > 1); the single-layer instances carry none of its code.
+// RAW: adjoint mode writing the input gradient of a first layer -- output rows of any width (Fout need not be a multiple
+// of 4: element stores), row m sent to raw row perm[m] when perm is given (fake vertices dropped), MMA N = 16 for
+// outputs of at most 16 columns.  The other instances carry none of its code.
+template <int FP, int MAXI, bool IMG, bool STACK, bool RAW>
 __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdParams P) {
   extern __shared__ __align__(1024) unsigned char smem[];
   constexpr int G = 32 / FP;    // windows per 128-byte row
@@ -389,6 +392,23 @@ __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdPara
           const bool valid = rb < BQ && j < Mo && b < P.B;
           const long long orow = (long long)b * Mo + j;
           const uint32_t tbase = tmem + ((uint32_t)(e * 32) << 16) + (uint32_t)(buf * P.acc_cols + (g * p * P.T + t) * 32);
+          if constexpr (RAW) {
+            // p = 1, no bias / ReLU: row j of the layer's vertex order is the gradient of raw row src_row[j] (perm[j], or
+            // -1 for a fake vertex, whose gradient is dropped).  Every raw row has exactly one such j: plain stores, no
+            // zero fill.  A row of Fout floats need not be 16-byte aligned: element stores.
+            const int dst = valid ? src_row[j] : -1;
+            float* dxp = dst >= 0 ? P.y + ((long long)b * P.M_in + dst) * P.Fout : nullptr;
+            for (int h = h0; h < h1 && h * 16 < P.Fout; ++h) {
+              float m[16];
+              tmem_ld16(tbase + h * 16, m);
+              if (dxp) {
+#pragma unroll
+                for (int o = 0; o < 16; ++o)
+                  if (h * 16 + o < P.Fout) dxp[h * 16 + o] = m[o];
+              }
+            }
+            return;
+          }
           float msum = 0.f;
           for (int h = h0; h < h1; ++h) {
             float m[16];
@@ -1033,6 +1053,11 @@ __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdPara
             bb[j] = smem_desc(kDescTaps, sb + P.off_wb + (uint32_t)(k * (FP / 8) * 4) * 128u + j * 1024);
           const uint32_t first_acc = k != 0;
           const uint32_t d0 = tmem + (uint32_t)(buf * P.acc_cols);
+          uint32_t idesc_tf32 = kIdescTf32, idesc_bf16 = kIdescBf16;
+          if constexpr (RAW) {
+            // at most 16 output columns: the zero tap columns 16..31 are not multiplied (the epilogue never reads them)
+            if (P.Fout <= 16) idesc_tf32 = kIdescTf32N16, idesc_bf16 = kIdescBf16N16;
+          }
 #ifdef GCNB_TRACE
           const bool t_tf32 = !(P.debug & 16), t_lo = !(P.debug & 64), t_bf16 = !(P.debug & 32);
           if (!(P.debug & 2))
@@ -1051,13 +1076,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_cheb_fwd_umma(const UmmaFwdPara
                 if (leader) {
 #pragma unroll
                   for (int j = 0; j < FP / 8; ++j)
-                    if (t_tf32) mma_tf32(d, da + 2 * j, bh[j], kIdescTf32, j ? 1u : first_acc);
+                    if (t_tf32) mma_tf32(d, da + 2 * j, bh[j], idesc_tf32, j ? 1u : first_acc);
 #pragma unroll
                   for (int j = 0; j < FP / 8; ++j)
-                    if (t_tf32 && t_lo) mma_tf32(d, da + 2 * j, bl[j], kIdescTf32, 1);
+                    if (t_tf32 && t_lo) mma_tf32(d, da + 2 * j, bl[j], idesc_tf32, 1);
 #pragma unroll
                   for (int j = 0; j < FP / 16; ++j)
-                    if (t_bf16) mma_bf16(d, dl + 2 * j, bb[j], kIdescBf16, 1);
+                    if (t_bf16) mma_bf16(d, dl + 2 * j, bb[j], idesc_bf16, 1);
                 }
                 d += 32;
                 at += 128 * 128 / 16;  // the next 128 rows of the block
@@ -1170,12 +1195,13 @@ struct UmmaFwdPlan {
 };
 
 // ent_bytes < 0: the kernel builds its own (CSR-ordered) operator image in the prologue; otherwise the entry streams of
-// a host-built image take ent_bytes.
-static UmmaFwdPlan plan_umma_fwd(const LayerShape& s, int sm_count, int smem_optin, long long ent_bytes = -1) {
+// a host-built image take ent_bytes.  raw: the adjoint instances that store rows of any width (RAW), Fout % 4 != 0 too.
+static UmmaFwdPlan plan_umma_fwd(const LayerShape& s, int sm_count, int smem_optin, long long ent_bytes = -1,
+                                 bool raw = false) {
   UmmaFwdPlan pl{};
   pl.ok = false;
   pl.img = ent_bytes >= 0;
-  if (s.Fin <= 8 || s.Fin > 32 || s.Fout < 4 || s.Fout > 32 || (s.Fout & 3)) return pl;
+  if (s.Fin <= 8 || s.Fin > 32 || s.Fout < 4 || s.Fout > 32 || (!raw && (s.Fout & 3))) return pl;
   if (s.p != 1 && s.p != 2 && s.p != 4 && s.p != 8) return pl;
   if (s.M % s.p != 0 || s.M < 1 || s.M > 2048 || s.K < 1 || s.B < 1) return pl;
   if (pl.img && (s.M & 3)) return pl;
@@ -1346,7 +1372,7 @@ size_t cheb_image_bytes(const int32_t* rowptr, const int32_t* col, const LayerSh
   for (int st : steps) ent += (long long)(st / 2) * kImgPair;
   DeviceInfo di;
   plan_device(&di);
-  const UmmaFwdPlan pl = plan_umma_fwd(s, di.sm_count, di.smem_optin, ent);
+  const UmmaFwdPlan pl = plan_umma_fwd(s, di.sm_count, di.smem_optin, ent, adjoint != 0);
   return pl.ok ? pl.img_bytes : 0;
 }
 
@@ -1363,7 +1389,7 @@ int cheb_image_build(const int32_t* rowptr, const int32_t* col, const float* val
   for (int st : steps) ent += (long long)(st / 2) * kImgPair;
   DeviceInfo di;
   plan_device(&di);
-  const UmmaFwdPlan pl = plan_umma_fwd(s, di.sm_count, di.smem_optin, ent);
+  const UmmaFwdPlan pl = plan_umma_fwd(s, di.sm_count, di.smem_optin, ent, adjoint != 0);
   GCNB_REQUIRE(pl.ok, "gcnb_cheb_image_build: no image-based kernel for this shape");
   GCNB_REQUIRE(bytes == pl.img_bytes, "gcnb_cheb_image_build: buffer has %zu bytes, the image needs %zu", bytes, pl.img_bytes);
   const ImgGeom ge = img_geom(s.M);
@@ -1412,6 +1438,9 @@ struct UmmaAdjoint {
   const float* y;
   const uint8_t* argmax;
   int p, relu, dy_is_mean;
+  bool raw;             // the RAW instances: output rows of any width, sent to raw row perm[m] (perm nullable)
+  const int32_t* perm;
+  int M_in;
 };
 
 struct UmmaStack {  // a stack of identical layers run back to back on a tile (UmmaFwdParams::nlayers)
@@ -1434,8 +1463,9 @@ static int umma_launch(const float* x, const int32_t* perm, int M_in, const gcnb
                      (reinterpret_cast<uintptr_t>(L.image) & 15) == 0,
                  "operator image: bad size or alignment");
   }
-  const UmmaFwdPlan pl = img ? plan_umma_fwd(s, di.sm_count, di.smem_optin, (long long)(L.image_bytes - img_geom(s.M).ent_off))
-                             : plan_umma_fwd(s, di.sm_count, di.smem_optin);
+  const bool raw = adj != nullptr && adj->raw;
+  const UmmaFwdPlan pl = img ? plan_umma_fwd(s, di.sm_count, di.smem_optin, (long long)(L.image_bytes - img_geom(s.M).ent_off), raw)
+                             : plan_umma_fwd(s, di.sm_count, di.smem_optin, -1, raw);
   if (!pl.ok) {
     set_error(img ? "the operator image does not belong to this layer shape" : "tcgen05 forward does not support this shape");
     return GCNB_ERR_INVALID;
@@ -1474,6 +1504,10 @@ static int umma_launch(const float* x, const int32_t* perm, int M_in, const gcnb
     P.adj_log2p = 0;
     while ((1 << P.adj_log2p) < adj->p) ++P.adj_log2p;
     P.adj_Mo = s.M >> P.adj_log2p;
+    if (raw) {  // the prologue's source-row table becomes the destination-row table of the epilogue
+      P.perm = adj->perm;
+      P.M_in = adj->M_in;
+    }
   }
   P.NS = pl.NS; P.S = pl.NS * pl.G; P.Q = pl.Q; P.BQ = pl.BQ; P.T = pl.T; P.NG = pl.NG; P.nlo = pl.nlo; P.nacc = pl.nacc;
   P.acc_cols = pl.acc_cols; P.tmem_cols = pl.tmem_cols; P.slab_rows = pl.slab_rows;
@@ -1498,14 +1532,18 @@ static int umma_launch(const float* x, const int32_t* perm, int M_in, const gcnb
   P.debug = std::getenv("GCNB_UMMA_DEBUG") ? std::atoi(std::getenv("GCNB_UMMA_DEBUG")) : 0;
 #endif
   const int grid = std::min(P.ntiles, di.sm_count);
-#define GCNB_UMMA_CASE(fp, mi, im, stk)                                                                                 \
-  if (pl.FP == fp && pl.MAXI == mi && img == im && (P.nlayers > 1) == stk) {                                            \
-    GCNB_CUDA(cudaFuncSetAttribute(k_cheb_fwd_umma<fp, mi, im, stk>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem)); \
-    k_cheb_fwd_umma<fp, mi, im, stk><<<grid, kThreads, pl.smem, st>>>(P);                                              \
+#define GCNB_UMMA_CASE(fp, mi, im, stk, rw)                                                                             \
+  if (pl.FP == fp && pl.MAXI == mi && img == im && (P.nlayers > 1) == stk && raw == rw) {                               \
+    GCNB_CUDA(cudaFuncSetAttribute(k_cheb_fwd_umma<fp, mi, im, stk, rw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem)); \
+    k_cheb_fwd_umma<fp, mi, im, stk, rw><<<grid, kThreads, pl.smem, st>>>(P);                                          \
   }
-  GCNB_UMMA_CASE(16, 3, false, false) GCNB_UMMA_CASE(16, 5, false, false) GCNB_UMMA_CASE(32, 3, false, false)
-  GCNB_UMMA_CASE(32, 5, false, false) GCNB_UMMA_CASE(16, 1, true, false) GCNB_UMMA_CASE(32, 1, true, false)
-  GCNB_UMMA_CASE(32, 1, true, true)
+  GCNB_UMMA_CASE(16, 3, false, false, false) GCNB_UMMA_CASE(16, 5, false, false, false)
+  GCNB_UMMA_CASE(32, 3, false, false, false) GCNB_UMMA_CASE(32, 5, false, false, false)
+  GCNB_UMMA_CASE(16, 1, true, false, false) GCNB_UMMA_CASE(32, 1, true, false, false)
+  GCNB_UMMA_CASE(32, 1, true, true, false)
+  GCNB_UMMA_CASE(16, 3, false, false, true) GCNB_UMMA_CASE(16, 5, false, false, true)
+  GCNB_UMMA_CASE(32, 3, false, false, true) GCNB_UMMA_CASE(32, 5, false, false, true)
+  GCNB_UMMA_CASE(16, 1, true, false, true) GCNB_UMMA_CASE(32, 1, true, false, true)
 #undef GCNB_UMMA_CASE
   GCNB_LAUNCH_CHECK("k_cheb_fwd_umma");
   return GCNB_OK;
@@ -1582,7 +1620,32 @@ bool umma_adj_supported(const LayerShape& s) {
 
 int umma_cheb_adj(const float* dy, int dy_is_mean, const float* y, const uint8_t* argmax, const gcnb_csr& Lt, const float* W,
                   float* dx, const LayerShape& s, int relu, cudaStream_t st) {
-  UmmaAdjoint a{dy, y, argmax, s.p, relu, dy_is_mean};
+  UmmaAdjoint a{dy, y, argmax, s.p, relu, dy_is_mean, false, nullptr, s.M};
+  return umma_launch(nullptr, nullptr, s.M, Lt, W, nullptr, dx, nullptr, nullptr, nullptr, adjoint_shape(s), GCNB_BIAS_NONE, 0,
+                     &a, st);
+}
+
+// The same for any input width Fin in [4, 32] (the RAW instances); the layer's Fout must still be a multiple of 4 (dZ is
+// rebuilt from dy / y / arg-max with 16-byte loads).
+bool umma_adj_raw_supported(const LayerShape& s) {
+  if ((s.Fout & 3) || s.M % s.p != 0 || s.p > 255) return false;
+  DeviceInfo di;
+  plan_device(&di);
+  return plan_umma_fwd(adjoint_shape(s), di.sm_count, di.smem_optin, -1, true).ok;
+}
+
+int umma_adj_describe(const LayerShape& s, char* out, size_t n) {
+  DeviceInfo di;
+  plan_device(&di);
+  const UmmaFwdPlan pl = plan_umma_fwd(adjoint_shape(s), di.sm_count, di.smem_optin, -1, true);
+  if (!pl.ok) return 0;
+  return snprintf(out, n, "k_cheb_fwd_umma<FP=%d, RAW> on L~^T, MMA N=%d, %d windows/tile, %zu B smem, %d tiles", pl.FP,
+                  s.Fin <= 16 ? 16 : 32, pl.NS * pl.G, pl.smem, ceil_div(s.B, pl.NS * pl.G));
+}
+
+int umma_cheb_adj_raw(const float* dy, int dy_is_mean, const float* y, const uint8_t* argmax, const gcnb_csr& Lt,
+                      const float* W, float* dx, const int32_t* perm, int M_in, const LayerShape& s, int relu, cudaStream_t st) {
+  UmmaAdjoint a{dy, y, argmax, s.p, relu, dy_is_mean, true, perm, M_in};
   return umma_launch(nullptr, nullptr, s.M, Lt, W, nullptr, dx, nullptr, nullptr, nullptr, adjoint_shape(s), GCNB_BIAS_NONE, 0,
                      &a, st);
 }

@@ -131,6 +131,12 @@ int cheb_tap_image_build(const float* W, int Fin, int Fout, int K, void* out, si
 bool umma_adj_supported(const LayerShape& s);
 int umma_cheb_adj(const float* dy, int dy_is_mean, const float* y, const uint8_t* argmax, const gcnb_csr& Lt, const float* W,
                   float* dx, const LayerShape& s, int relu, cudaStream_t st);
+// ... for any input width Fin in [4, 32], dx stored row by row, row m to raw row perm[m] (perm nullable; rows with
+// perm[m] >= M_in dropped): the input gradient of a first layer
+bool umma_adj_raw_supported(const LayerShape& s);
+int umma_adj_describe(const LayerShape& s, char* out, size_t n);  // 0 when the shape is not supported
+int umma_cheb_adj_raw(const float* dy, int dy_is_mean, const float* y, const uint8_t* argmax, const gcnb_csr& Lt,
+                      const float* W, float* dx, const int32_t* perm, int M_in, const LayerShape& s, int relu, cudaStream_t st);
 
 // ---- fused (shared-memory resident) path, fused_fwd.cu / fused_bwd.cu ------------------------
 bool fused_fwd_supported(const LayerShape& s);

@@ -119,6 +119,9 @@ __host__ __device__ constexpr uint32_t instr_desc(uint32_t ab_format, uint32_t M
 }
 constexpr uint32_t kIdescTf32 = instr_desc(2, 128, 32);
 constexpr uint32_t kIdescBf16 = instr_desc(1, 128, 32);
+// N = 16: the same tap layout, only its first two 8-filter groups are read (outputs of at most 16 columns)
+constexpr uint32_t kIdescTf32N16 = instr_desc(2, 128, 16);
+constexpr uint32_t kIdescBf16N16 = instr_desc(1, 128, 16);
 
 // D[tmem] (+)= A[smem] * B[smem]; issued by ONE thread on behalf of the CTA.
 __device__ __forceinline__ void mma_tf32(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {

@@ -343,6 +343,49 @@ class cgcnn(nn.Module):
             out += (all_logits,)
         return out if len(out) > 1 else out[0]
 
+    def saliency(self, data, target=None, gather=None):
+        """Gradient saliency maps: ``(grad [n, n_input_vertices, channel] float32, target [n] int64)``, the gradient of
+        the logit of class ``target[i]`` w.r.t. window ``i`` of ``data`` -- which ROIs and which TRs drive the decision.
+        ``target=None`` takes the predicted class (the arg-max of the logits, as ``prediction()``).  Batched like
+        ``predict``: batches of ``batch_size``, the last one zero-padded.  ``gather`` follows ``forward``: raw windows
+        are permuted in the first layer's load and their gradient un-permuted in its store (with ``gather=False`` the
+        data and the gradient are in the first layer's vertex order, ``[n, M_0, channel]``).  Runs on the GPU through
+        ``saliency.InputGradient`` (one CUDA graph per batch shape)."""
+        from .saliency import InputGradient
+
+        M0 = self.L[0].shape[0]
+        if gather is None:
+            if self.perm is not None and self.n_input_vertices == M0:
+                raise ValueError("cgcnn.saliency: with perm set and n_input_vertices == M_0 say gather=True (raw windows) "
+                                 "or gather=False (already permuted) -- the shapes are identical")
+            gather = self.perm is not None and data.shape[1] == self.n_input_vertices != M0
+        gather = bool(gather) and self.perm is not None
+        if gather:
+            # the first layer writes each raw row's gradient exactly once: that needs a permutation of [0, M_0)
+            perm = self.perm.cpu().numpy()
+            if not np.array_equal(np.sort(perm), np.arange(M0)):
+                raise ValueError("cgcnn.saliency: perm is not a permutation of [0, M_0 = %d)" % M0)
+        params = tuple(p.data_ptr() for p in self.parameters())
+        cached = self.__dict__.get("_saliency")
+        if cached is None or cached[0] != params:
+            cached = self.__dict__["_saliency"] = (params, InputGradient(self))
+        ig = cached[1]
+        size, bs = data.shape[0], self.batch_size
+        grads = np.empty((size,) + tuple(data.shape[1:]), np.float32)
+        targets = np.empty(size, np.int64)
+        for begin in range(0, size, bs):
+            end = min(begin + bs, size)
+            batch = torch.zeros((bs,) + tuple(data.shape[1:]), dtype=torch.float32, device=self.dev)
+            batch[: end - begin] = torch.as_tensor(np.asarray(data[begin:end]), dtype=torch.float32, device=self.dev)
+            t = None
+            if target is not None:
+                t = torch.zeros(bs, dtype=torch.long, device=self.dev)
+                t[: end - begin] = torch.as_tensor(np.asarray(target[begin:end]), dtype=torch.long, device=self.dev)
+            g, _, tg = ig(batch, t, gather=gather)
+            grads[begin:end] = g[: end - begin].cpu().numpy()
+            targets[begin:end] = tg[: end - begin].cpu().numpy()
+        return grads, targets
+
     # ------------------------------------------------------------------ base_model's small public methods
     def inference(self, data, dropout=1.0):
         """Logits of a batch (models_gcn.py:224-239); raw windows are permuted on the way in, as in ``forward``."""

@@ -13,6 +13,8 @@ Op                       replaces (``/root/reference/lib_new/models_gcn.py``)
 ``mpool_fwd / _bwd``      mpool1 stand-alone (tf.nn.max_pool SAME)
 ``perm_gather``           coarsening.perm_data_3d (``lib_new/coarsening.py:244-265``)
 ``mean_f_fwd / _bwd``     tf.reduce_mean(x, -1) of ``_inference`` ``:673``
+``cheb_dx``               input gradient of a ChebyNet layer alone (saliency maps, ``saliency.py``; no reference
+                          counterpart)
 """
 from __future__ import annotations
 
@@ -254,6 +256,54 @@ def _(x, perm, y, argmax, dy, dy_is_mean, rowptr, col, val, rowptr_t, col_t, val
     return x.new_empty((x.shape[0], rowptr.numel() - 1, x.shape[2]) if need_dx else (0,))
 
 
+@torch.library.custom_op("gcn_b200::cheb_dx", mutates_args=(), device_types="cuda")
+def cheb_dx(x: Optional[Tensor], perm: Optional[Tensor], M_in: int, y: Tensor, argmax: Tensor, dy: Tensor,
+            dy_is_mean: bool, rowptr: Tensor, col: Tensor, val: Tensor, rowptr_t: Tensor, col_t: Tensor, val_t: Tensor,
+            W: Tensor, K: int, p: int, relu: bool, algo: int) -> Tensor:
+    """Input gradient of a ChebyNet layer alone (``gcnb_cheb_dx_f32``: no dW, no db).  With ``perm`` (a Graclus
+    permutation of the layer's vertices) it is the gradient w.r.t. the raw windows ``[B, M_in, Fin]``, un-permuted in the
+    kernel's store; without, w.r.t. the layer input ``[B, M, Fin]``.  ``x`` (the layer input) may be None on the tcgen05
+    route, which never reads it (``_lib.describe_dx`` names the route)."""
+    dy = dy.contiguous()
+    B = y.shape[0]
+    M = rowptr.numel() - 1
+    Fout = W.shape[1]
+    Fin = W.shape[0] // K
+    if perm is None and M_in != M:
+        raise ValueError("without perm the layer input has M = %d vertices (got M_in = %d)" % (M, M_in))
+    if perm is not None and (perm.dtype != torch.int32 or perm.numel() != M):
+        raise ValueError("perm must be int32 with one entry per (padded) vertex")
+    if x is not None:
+        x = x.contiguous()
+        if tuple(x.shape) != (B, M_in, Fin):
+            raise ValueError("x must be [B, M_in, Fin] = %s, got %s" % ((B, M_in, Fin), tuple(x.shape)))
+    dx = torch.empty((B, M_in, Fin), dtype=torch.float32, device=y.device)
+    L = _lib.lib()
+    _, nbytes = _lib.describe_dx(B, M, val.numel(), Fin, Fout, K, p, algo)
+    ws = _workspace(nbytes, y.device)
+    csr = csr_struct(rowptr, col, val)
+    csr_t = csr_struct(rowptr_t, col_t, val_t, (B, Fin, Fout, K, p))
+    rc = L.gcnb_cheb_dx_f32(_ptr(x), _ptr(perm), M_in, _ptr(y), _ptr(argmax), _ptr(dy), int(dy_is_mean), C.byref(csr),
+                            C.byref(csr_t), _ptr(W.contiguous()), _ptr(dx), B, Fin, Fout, K, p, int(relu), algo, _ptr(ws),
+                            ws.numel(), _stream(y))
+    _lib.check(rc, "gcnb_cheb_dx_f32")
+    return dx
+
+
+@cheb_dx.register_fake
+def _(x, perm, M_in, y, argmax, dy, dy_is_mean, rowptr, col, val, rowptr_t, col_t, val_t, W, K, p, relu, algo):
+    return y.new_empty((y.shape[0], M_in, W.shape[0] // K))
+
+
+def unpermute(dx: Tensor, perm: Tensor, M_in: int) -> Tensor:
+    """Gradient w.r.t. the raw windows ``[B, M_in, F]`` from the gradient ``dx [B, M, F]`` w.r.t. the input permuted by
+    ``perm`` (the adjoint of ``perm_gather``): row m goes back to raw row ``perm[m]``; fake vertices (``perm[m] >= M_in``)
+    are dropped.  No host synchronisation (CUDA-graph capturable): fake vertices land in one extra row, cut off."""
+    gx = dx.new_zeros((dx.shape[0], M_in + 1, dx.shape[2]))
+    gx.index_copy_(1, torch.where(perm < M_in, perm, M_in).long(), dx)
+    return gx[:, :M_in]
+
+
 def _cheb_setup(ctx, inputs, output):
     (x, perm, rowptr, col, val, rowptr_t, col_t, val_t, W, bias, K, p, bias_mode, relu, want_argmax, algo) = inputs
     y, argmax = output
@@ -271,12 +321,7 @@ def _cheb_backward(ctx, dy, _dargmax):
                                              bias_mode, relu, need_dx, algo)
     gx = None
     if need_dx:
-        if perm is None:
-            gx = dx
-        else:  # gradient w.r.t. the un-permuted data: scatter the real vertices back (rarely needed)
-            real = perm < x.shape[1]
-            gx = torch.zeros_like(x)
-            gx[:, perm[real].long(), :] = dx[:, real, :]
+        gx = dx if perm is None else unpermute(dx, perm, x.shape[1])
     gb = db.reshape(bshape) if (bshape is not None and ctx.needs_input_grad[9]) else None
     return (gx, None, None, None, None, None, None, None, dW if ctx.needs_input_grad[8] else None, gb,
             None, None, None, None, None, None)

@@ -177,6 +177,26 @@ GCNB_API int gcnb_cheb_bwd_f32(const float* x, const int32_t* perm, int M_in, co
                       size_t workspace_bytes, gcnb_stream_t stream);
 
 /*
+ * Input gradient of the fused layer only (no dW, no db): dx = sum_k T_k(L~^T) (dz W_k^T) with dz rebuilt from dy / y /
+ * argmax as in gcnb_cheb_bwd_f32 -- what a gradient saliency map of a trained network needs of each conv layer.
+ * perm (nullable): the first layer's Graclus ordering, which must be a permutation of [0, M) (every raw vertex appears
+ *   exactly once; entries >= M_in are fake vertices).  dx is then the gradient w.r.t. the UN-permuted input
+ *   x_raw[B][M_in][Fin]: row m goes to raw row perm[m], fake vertices are dropped.  Without perm dx is [B][M][Fin].
+ * x [B][M_in][Fin] (the layer input, as in the forward) may be NULL where the route never reads it: the general path
+ *   recomputes the Chebyshev basis and refuses a NULL x.  Lt is required when K > 1; an operator image in Lt->image
+ *   (gcnb_cheb_image_build with adjoint != 0) serves the tcgen05 route.  No bias argument: the bias does not enter dx.
+ * gcnb_cheb_dx_describe names the route ("<route>: <its kernels>") and returns the workspace it takes (256-byte aligned
+ * pointer).  Routes: the tcgen05 adjoint (k_cheb_fwd_umma on L~^T, any Fin in [4, 32], ALGO_AUTO), k_cheb_bwd_fused
+ * without the weight gradient, or the general path (dW to workspace scratch); the last two un-permute in a second launch.
+ */
+GCNB_API int gcnb_cheb_dx_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, int algo, char* out, size_t n,
+                                   size_t* workspace_bytes);
+GCNB_API int gcnb_cheb_dx_f32(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax,
+                              const float* dy, int dy_is_mean, const gcnb_csr* L, const gcnb_csr* Lt, const float* W,
+                              float* dx, int B, int Fin, int Fout, int K, int p, int relu, int algo, void* workspace,
+                              size_t workspace_bytes, gcnb_stream_t stream);
+
+/*
  * Spectral layer (cgcnn.fourier + filter_in_fourier, models_gcn.py:512-539) with the same fused
  * bias/ReLU/pool epilogue.  Ut[M][M] is the transposed eigenvector matrix (row i = i-th
  * eigenvector), exactly the constant the reference builds at :536.  W[M][Fout][Fin].
