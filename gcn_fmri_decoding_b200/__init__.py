@@ -7,11 +7,11 @@ compute path: calling a layer without the library or without a GPU raises.
 """
 from . import graclus, graphs, synth  # noqa: F401
 
-__all__ = ["graclus", "graphs", "synth", "ops", "models", "train", "plan"]
+__all__ = ["graclus", "graphs", "synth", "ops", "models", "finetune", "train", "plan"]
 
 
 def __getattr__(name):  # lazy: importing the package must not require torch
-    if name in ("ops", "models", "train", "plan", "_lib"):
+    if name in ("ops", "models", "finetune", "train", "plan", "_lib"):
         import importlib
 
         return importlib.import_module("." + name, __name__)

@@ -73,6 +73,8 @@ SIGNATURES = {
                                         _p, _p, _i, _i, _p]),
     "gcnb_adam_tf_f32": (_i, [_p, _p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,
                               C.c_float, C.c_float, _i, _p]),
+    "gcnb_nadam_tf_f32": (_i, [_p, _p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,
+                               C.c_float, _i, _p]),
 }
 
 _lib = None

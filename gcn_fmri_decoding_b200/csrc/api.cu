@@ -336,7 +336,7 @@ using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 102; }
+int gcnb_version(void) { return 103; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 

@@ -1,6 +1,7 @@
 // Training-step pieces around the conv stack ("next" rows of the scope table, SURVEY.md 8f):
 //   * sparse softmax cross-entropy, forward and backward in one pass (models_gcn.py:253-259),
-//   * TensorFlow-1.x Adam over one flat parameter buffer, L2 term folded in (models_gcn.py:260-262, :294).
+//   * TensorFlow-1.x Adam over one flat parameter buffer, L2 term folded in (models_gcn.py:260-262, :294), and its
+//     Nesterov variant (tf.contrib.opt.NadamOptimizer) for fine-tuning a new classifier head.
 // They exist so that a whole training step is a handful of launches inside one CUDA graph.
 #include <algorithm>
 
@@ -161,7 +162,9 @@ __global__ void __launch_bounds__(1024) k_colsum_multi(ColsumArgs a) {
   }
 }
 
-// g_total = g * gscale + reg * p (where decay[i] != 0);  m, v, p updated in place (TF "epsilon hat" form)
+// g_total = g * gscale + reg * p (where decay[i] != 0);  m, v, p updated in place (TF "epsilon hat" form).
+// kNesterov: TF's NadamOptimizer (ApplyAdam with use_nesterov), the step takes b1 m + (1-b1) g_total in place of m.
+template <bool kNesterov>
 __global__ void k_adam_tf(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                           const uint8_t* __restrict__ decay, const float* __restrict__ state, long long n, float b1,
                           float b2, float eps, float reg, float gscale) {
@@ -174,7 +177,7 @@ __global__ void k_adam_tf(float* __restrict__ p, const float* __restrict__ g, fl
     const float vi = fmaf(1.f - b2, gi * gi - v[i], v[i]);
     m[i] = mi;
     v[i] = vi;
-    p[i] = pi - lr_t * mi / (sqrtf(vi) + eps);
+    p[i] = pi - lr_t * (kNesterov ? fmaf(b1, mi, (1.f - b1) * gi) : mi) / (sqrtf(vi) + eps);
   }
 }
 
@@ -249,8 +252,22 @@ int gcnb_adam_tf_f32(float* p, const float* g, float* m, float* v, const uint8_t
     GCNB_LAUNCH_CHECK("k_adam_tick");
   }
   const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(ceil_div_ll(n, 256), 148 * 8));
-  k_adam_tf<<<grid, 256, 0, st>>>(p, g, m, v, decay, state, n, beta1, beta2, eps, reg, gscale);
+  k_adam_tf<false><<<grid, 256, 0, st>>>(p, g, m, v, decay, state, n, beta1, beta2, eps, reg, gscale);
   GCNB_LAUNCH_CHECK("k_adam_tf");
+  return GCNB_OK;
+}
+
+int gcnb_nadam_tf_f32(float* p, const float* g, float* m, float* v, const uint8_t* decay, float* state, long long n,
+                      float lr, float beta1, float beta2, float eps, float reg, int tick, gcnb_stream_t stream) {
+  GCNB_REQUIRE(p && g && m && v && state && n >= 1, "gcnb_nadam_tf_f32: bad arguments");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (tick) {
+    k_adam_tick<<<1, 1, 0, st>>>(state, lr, beta1, beta2);
+    GCNB_LAUNCH_CHECK("k_adam_tick");
+  }
+  const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(ceil_div_ll(n, 256), 148 * 8));
+  k_adam_tf<true><<<grid, 256, 0, st>>>(p, g, m, v, decay, state, n, beta1, beta2, eps, reg, 1.f);
+  GCNB_LAUNCH_CHECK("k_adam_tf<true>");
   return GCNB_OK;
 }
 

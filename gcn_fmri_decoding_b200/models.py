@@ -289,6 +289,10 @@ class cgcnn(nn.Module):
         """logits = head(conv_stack(x)); ``dropout`` is the keep probability, as in the reference."""
         x = self.conv_stack(x, gather=gather)
         x = ops.mean_f_fwd(x)  # tf.reduce_mean(x, -1), models_gcn.py:673
+        return self._head(x, dropout)
+
+    def _head(self, x, dropout=1.0):
+        """The FC layers of ``_inference`` (models_gcn.py:674-682) on the mean over the last conv layer's filters."""
         for i in range(len(self.M) - 1):
             x = self.fc(x, i)
             if dropout < 1.0:
@@ -318,16 +322,27 @@ class cgcnn(nn.Module):
         """Batched prediction with the reference's zero-padded last batch (models_gcn.py:31-71); with ``return_logits``
         the logits ``[size, n_classes]`` are returned as a third (second, without labels) value -- what
         ``model_perf.predict`` collects (:1012-1016)."""
-        size = data.shape[0]
+        return self._predict(data.shape[0], lambda begin: self.forward(self._padded_batch(data, begin)), labels,
+                             return_logits)
+
+    def _padded_batch(self, data, begin):
+        """Rows ``begin : begin + batch_size`` of ``data`` on the device, zero-padded past its end as ``predict`` pads."""
+        bs = self.batch_size
+        end = min(begin + bs, data.shape[0])
+        batch = torch.zeros((bs,) + tuple(data.shape[1:]), dtype=torch.float32, device=self.dev)
+        batch[: end - begin] = torch.as_tensor(np.asarray(data[begin:end]), dtype=torch.float32, device=self.dev)
+        return batch
+
+    def _predict(self, size, logits_at, labels, return_logits):
+        """``predict`` over ``size`` windows with ``logits_at(begin)`` giving the logits of the batch that starts at window
+        ``begin``: the batching, the cropping and the loss of the zero-padded last batch."""
         preds = np.empty(size)
         all_logits = np.empty((size, self.M[-1]), np.float32) if return_logits else None
         total = 0.0
         bs = self.batch_size
         for begin in range(0, size, bs):
             end = min(begin + bs, size)
-            batch = torch.zeros((bs,) + tuple(data.shape[1:]), dtype=torch.float32, device=self.dev)
-            batch[: end - begin] = torch.as_tensor(np.asarray(data[begin:end]), dtype=torch.float32, device=self.dev)
-            logits = self.forward(batch)
+            logits = logits_at(begin)
             if labels is not None:
                 lab = torch.zeros(bs, dtype=torch.long, device=self.dev)
                 lab[: end - begin] = torch.as_tensor(np.asarray(labels[begin:end]), dtype=torch.long, device=self.dev)
@@ -413,14 +428,21 @@ class cgcnn(nn.Module):
         checkpoints by validation accuracy are kept (checkmat.py, directory ``best_checkpoint_dir`` or
         ``checkpoints/<dir_name>/model``).  Returns ``(accuracies, losses, t_step)`` like the reference.  On a CUDA
         device the steps run through ``train.FusedTrainer`` fed by ``train.InputPipeline``."""
+        from . import train
+
+        if trainer is None:
+            fused = self.dev.type == "cuda" and self.momentum != 0
+            trainer = train.FusedTrainer(self) if fused else train.Trainer(self)
+        return self._fit(train_data, train_labels, lambda: self.evaluate(val_data, val_labels), best_checkpoint_dir,
+                         trainer)
+
+    def _fit(self, train_data, train_labels, evaluate, best_checkpoint_dir, trainer):
+        """The loop of ``fit`` on ``train_data`` with ``evaluate()`` giving ``evaluate``'s result at every evaluation."""
         import os
         import time
 
         from . import checkpoints, train
 
-        if trainer is None:
-            fused = self.dev.type == "cuda" and self.momentum != 0
-            trainer = train.FusedTrainer(self) if fused else train.Trainer(self)
         path = best_checkpoint_dir or os.path.join("checkpoints", self.dir_name, "model")
         keeper = checkpoints.BestCheckpoints(path, num_to_keep=3, maximize=True)
         n = train_data.shape[0]
@@ -432,7 +454,7 @@ class cgcnn(nn.Module):
         def on_eval(step, num_steps, loss_average):
             print("step {} / {} (epoch {:.2f} / {}):".format(step, num_steps, step * self.batch_size / n, self.num_epochs))
             print("  loss_average = {:.2e}".format(loss_average))
-            string, accuracy, f1, loss = self.evaluate(val_data, val_labels)
+            string, accuracy, f1, loss = evaluate()
             accuracies.append(accuracy)
             losses.append(loss)
             print("  validation {}".format(string))
@@ -490,3 +512,13 @@ class cgcnn(nn.Module):
             if tuple(a.shape) != tuple(v.shape):
                 raise ValueError("%s: shape %s does not match %s" % (k, a.shape, tuple(v.shape)))
             v.copy_(torch.from_numpy(a).to(v.device))
+
+
+def __getattr__(name):
+    # the fine-tuning model lives in finetune.py (it subclasses cgcnn) and is importable from here, next to cgcnn, as the
+    # reference keeps both classes in models_gcn.py
+    if name == "finetuning_cgcnn":
+        from .finetune import finetuning_cgcnn
+
+        return finetuning_cgcnn
+    raise AttributeError("module %r has no attribute %r" % (__name__, name))

@@ -9,6 +9,8 @@
   the gradients (SURVEY 8e).  The reference has no distributed code; this is the only
   collective the path needs.
 * ``fit`` -- the reference's step loop (``:112-184``) without sessions/checkpoints/summaries.
+* ``FusedTrainer`` -- the same step with an explicit schedule, one CUDA graph; ``HeadTrainer`` -- its head alone on cached
+  conv features with TF's Nadam, the step of the fine-tuning model (``:685-933``).
 """
 from __future__ import annotations
 
@@ -248,10 +250,7 @@ class FusedTrainer:
 
         from . import _lib, ops
 
-        if getattr(model, "momentum", 0.9) == 0:
-            raise NotImplementedError("FusedTrainer implements the Adam branch of the reference's optimiser choice "
-                                      "(models_gcn.py:294, what every reference script selects); momentum == 0 (decayed "
-                                      "SGD, :291-292) trains through train.Trainer")
+        self.params = self._trained_parameters(model)
         self.model, self.lr, self.b1, self.b2, self.eps = model, lr, beta1, beta2, eps
         self.C, self._lib, self.ops = C, _lib, ops
         # keep-probability of the FC dropout: the model's own (what Trainer and the reference use, models_gcn.py:145,677)
@@ -275,7 +274,6 @@ class FusedTrainer:
         self.gather = gather
         self.distributed = dist.is_available() and dist.is_initialized() if distributed is None else distributed
         self.world = dist.get_world_size() if self.distributed else 1
-        self.params = [p for p in model.parameters()]
         dev = self.params[0].device
         sizes = [p.numel() for p in self.params]
         self.n = sum(sizes)
@@ -323,6 +321,14 @@ class FusedTrainer:
         self._sx = self._sl = None
         self._loss = torch.zeros((), dtype=torch.float32, device=dev)
 
+    def _trained_parameters(self, model):
+        """The parameters the step updates: all of them, with TF Adam."""
+        if getattr(model, "momentum", 0.9) == 0:
+            raise NotImplementedError("FusedTrainer implements the Adam branch of the reference's optimiser choice "
+                                      "(models_gcn.py:294, what every reference script selects); momentum == 0 (decayed "
+                                      "SGD, :291-292) trains through train.Trainer")
+        return [p for p in model.parameters()]
+
     def _setup_peer_buffers(self, dev):
         """Symmetric (peer-mapped) memory of every rank: two flat gradient buffers + the flag array, zeroed; returns the
         per-parity pointer tables for the kernel and the two local gradient tensors."""
@@ -352,7 +358,7 @@ class FusedTrainer:
         lib = self._lib.lib()
         stream = C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
         vp = lambda t: C.c_void_p(t.data_ptr())
-        nconv, nfc = len(m.p), len(m.M)
+        nconv = len(m.p)
         mode = m._bias_mode()
         cheb = m.filter_name != "fourier"
         gather = self.gather
@@ -382,59 +388,7 @@ class FusedTrainer:
             h = y
         if h0 is None:
             h0 = ops.mean_f_fwd(h)
-        # ---- forward: head ----
-        def gemm(A, Bm, out, bias, M_, N_, K_, ta, tb):
-            rc = lib.gcnb_gemm_f32(vp(A), vp(Bm), vp(out), None if bias is None else vp(bias), M_, N_, K_, A.shape[1],
-                                   Bm.shape[1], out.shape[1], ta, tb, stream)
-            self._lib.check(rc, "gcnb_gemm_f32")
-            return out
-
-        # The FC GEMMs are plain library GEMMs (cuBLAS fp32): at B=512 they are a few microseconds each and launch
-        # bound; the in-house 3xTF32 kernel (`gemm`, used by the spectral layer) pays off only for large operands.
-        use_own_gemm = self.own_gemm
-
-        def gemm_epi(A, Bm, out, bias, M_, N_, K_, ta, tb, epi, aux, seed):
-            rc = lib.gcnb_gemm_epilogue_f32(vp(A), vp(Bm), vp(out), None if bias is None else vp(bias), M_, N_, K_,
-                                            A.shape[1], Bm.shape[1], out.shape[1], ta, tb, epi,
-                                            None if aux is None else vp(aux), 0 if aux is None else aux.shape[1],
-                                            self.keep, seed, vp(self.state), stream)
-            self._lib.check(rc, "gcnb_gemm_epilogue_f32")
-            return out
-
-        def fc_fwd(i, a_in, hidden):
-            """FC layer i; hidden layers apply ReLU + dropout (fused into the GEMM store on the in-house path)."""
-            W = m.fc_weights[i]
-            if not use_own_gemm:
-                a = torch.addmm(m.fc_bias[i], a_in, W)
-                if hidden:
-                    rc = lib.gcnb_relu_dropout_fwd_f32(vp(a), a.shape[0], a.shape[1], a.shape[1], self.keep, self.dropout_seed + i,
-                                                       vp(self.state), stream)
-                    self._lib.check(rc, "gcnb_relu_dropout_fwd_f32")
-                return a
-            out = torch.empty((a_in.shape[0], W.shape[1]), dtype=torch.float32, device=x.device)
-            if hidden:
-                return gemm_epi(a_in, W, out, m.fc_bias[i], a_in.shape[0], W.shape[1], W.shape[0], 0, 0,
-                                self._lib.EPI_RELU_DROPOUT, None, self.dropout_seed + i)
-            return gemm(a_in, W, out, m.fc_bias[i], a_in.shape[0], W.shape[1], W.shape[0], 0, 0)
-
-        B = h0.shape[0]
-        widths = [h0.shape[1]] + [w.shape[1] for w in m.fc_weights]
-        head_ws = lib.gcnb_head_step_workspace_bytes(B, *widths) if (self.fused_head and nfc == 3) else 0
-        if head_ws:
-            # the whole head -- three FC layers, cross-entropy, their backward pass, the optimiser clock -- in ONE launch
-            logits = torch.empty((B, widths[3]), dtype=torch.float32, device=x.device)
-            d = torch.empty((B, widths[0]), dtype=torch.float32, device=x.device)
-            ws = torch.empty(head_ws, dtype=torch.uint8, device=x.device)
-            g = lambda t: vp(self.gview[id(t)])
-            W1, W2, W3 = m.fc_weights
-            b1, b2, b3 = m.fc_bias
-            rc = lib.gcnb_head_step_f32(vp(h0), vp(labels), vp(W1), vp(b1), vp(W2), vp(b2), vp(W3), vp(b3), vp(logits),
-                                        vp(self._loss), g(W1), g(b1), g(W2), g(b2), g(W3), g(b3), vp(d), B, *widths,
-                                        self.keep, self.dropout_seed, self.dropout_seed + 1, vp(self.state), self.lr, self.b1, self.b2, 1,
-                                        vp(ws), ws.numel(), stream)
-            self._lib.check(rc, "gcnb_head_step_f32")
-        else:
-            logits, d = self._head_by_layers(h0, labels, gemm, gemm_epi, fc_fwd, lib, vp, stream)
+        logits, d = self._head(h0, labels, lib, vp, stream)
         # ---- backward: conv stack (d is the gradient of the mean over filters of the last layer) ----
         dy, dy_is_mean = d, True
         if not cheb:
@@ -468,6 +422,66 @@ class FusedTrainer:
         self._lib.check(rc, "gcnb_adam_tf_f32")
         return self._loss, logits
 
+    def _head(self, h0, labels, lib, vp, stream):
+        """The classifier head of the step on ``h0`` (the mean over the last conv layer's filters): forward, loss and
+        backward, the FC gradients written into the flat gradient buffer, the optimiser clock advanced.  Returns
+        ``(logits, d)`` with ``d`` the gradient w.r.t. ``h0``."""
+        m = self.model
+        nfc = len(m.M)
+
+        def gemm(A, Bm, out, bias, M_, N_, K_, ta, tb):
+            rc = lib.gcnb_gemm_f32(vp(A), vp(Bm), vp(out), None if bias is None else vp(bias), M_, N_, K_, A.shape[1],
+                                   Bm.shape[1], out.shape[1], ta, tb, stream)
+            self._lib.check(rc, "gcnb_gemm_f32")
+            return out
+
+        # The FC GEMMs are plain library GEMMs (cuBLAS fp32): at B=512 they are a few microseconds each and launch
+        # bound; the in-house 3xTF32 kernel (`gemm`, used by the spectral layer) pays off only for large operands.
+        use_own_gemm = self.own_gemm
+
+        def gemm_epi(A, Bm, out, bias, M_, N_, K_, ta, tb, epi, aux, seed):
+            rc = lib.gcnb_gemm_epilogue_f32(vp(A), vp(Bm), vp(out), None if bias is None else vp(bias), M_, N_, K_,
+                                            A.shape[1], Bm.shape[1], out.shape[1], ta, tb, epi,
+                                            None if aux is None else vp(aux), 0 if aux is None else aux.shape[1],
+                                            self.keep, seed, vp(self.state), stream)
+            self._lib.check(rc, "gcnb_gemm_epilogue_f32")
+            return out
+
+        def fc_fwd(i, a_in, hidden):
+            """FC layer i; hidden layers apply ReLU + dropout (fused into the GEMM store on the in-house path)."""
+            W = m.fc_weights[i]
+            if not use_own_gemm:
+                a = torch.addmm(m.fc_bias[i], a_in, W)
+                if hidden:
+                    rc = lib.gcnb_relu_dropout_fwd_f32(vp(a), a.shape[0], a.shape[1], a.shape[1], self.keep, self.dropout_seed + i,
+                                                       vp(self.state), stream)
+                    self._lib.check(rc, "gcnb_relu_dropout_fwd_f32")
+                return a
+            out = torch.empty((a_in.shape[0], W.shape[1]), dtype=torch.float32, device=h0.device)
+            if hidden:
+                return gemm_epi(a_in, W, out, m.fc_bias[i], a_in.shape[0], W.shape[1], W.shape[0], 0, 0,
+                                self._lib.EPI_RELU_DROPOUT, None, self.dropout_seed + i)
+            return gemm(a_in, W, out, m.fc_bias[i], a_in.shape[0], W.shape[1], W.shape[0], 0, 0)
+
+        B = h0.shape[0]
+        widths = [h0.shape[1]] + [w.shape[1] for w in m.fc_weights]
+        head_ws = lib.gcnb_head_step_workspace_bytes(B, *widths) if (self.fused_head and nfc == 3) else 0
+        if head_ws:
+            # the whole head -- three FC layers, cross-entropy, their backward pass, the optimiser clock -- in ONE launch
+            logits = torch.empty((B, widths[3]), dtype=torch.float32, device=h0.device)
+            d = torch.empty((B, widths[0]), dtype=torch.float32, device=h0.device)
+            ws = torch.empty(head_ws, dtype=torch.uint8, device=h0.device)
+            g = lambda t: vp(self.gview[id(t)])
+            W1, W2, W3 = m.fc_weights
+            b1, b2, b3 = m.fc_bias
+            rc = lib.gcnb_head_step_f32(vp(h0), vp(labels), vp(W1), vp(b1), vp(W2), vp(b2), vp(W3), vp(b3), vp(logits),
+                                        vp(self._loss), g(W1), g(b1), g(W2), g(b2), g(W3), g(b3), vp(d), B, *widths,
+                                        self.keep, self.dropout_seed, self.dropout_seed + 1, vp(self.state), self.lr, self.b1, self.b2, 1,
+                                        vp(ws), ws.numel(), stream)
+            self._lib.check(rc, "gcnb_head_step_f32")
+        else:
+            logits, d = self._head_by_layers(h0, labels, gemm, gemm_epi, fc_fwd, lib, vp, stream)
+        return logits, d
 
     def _head_by_layers(self, h0, labels, gemm, gemm_epi, fc_fwd, lib, vp, stream):
         """The head launch by launch (any number of FC layers): GEMM + fused ReLU/dropout per layer, cross-entropy,
@@ -592,6 +606,39 @@ class FusedTrainer:
             dist.barrier()
         self.flat_g, self.gview = keep
         return self._graphs[(par, key)]
+
+
+class HeadTrainer(FusedTrainer):
+    """Training step of a new classifier head on frozen graph convolutions (``finetune.finetuning_cgcnn``).
+
+    ``step(a0, labels)`` takes ``a0 [B, n0]``, the mean over the last conv layer's filters of each window (what
+    ``finetuning_cgcnn.trunk_features`` computes once per data set), and runs ``FusedTrainer``'s head on it -- one
+    ``gcnb_head_step_f32`` launch for a three-layer head the kernel takes, the layer-by-layer launches otherwise, with the
+    same dropout keep-probability, seeds and masks -- followed by ``gcnb_nadam_tf_f32`` (TF's ``NadamOptimizer``) over one
+    flat buffer that holds only the FC weights and biases, all regularised.  The conv parameters are never written.
+    Captured as one CUDA graph per batch shape; ``bind_inputs`` lets ``InputPipeline`` feed it."""
+
+    def __init__(self, model, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, use_cuda_graph=True):
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise NotImplementedError("HeadTrainer: data-parallel fine-tuning is not implemented")
+        super().__init__(model, lr=lr, distributed=False, use_cuda_graph=use_cuda_graph, beta1=beta1, beta2=beta2,
+                         eps=eps, gather=False)
+
+    def _trained_parameters(self, model):
+        """The head's weights and biases (updated with TF Nadam whatever ``model.momentum`` says)."""
+        return [p for W, b in zip(model.fc_weights, model.fc_bias) for p in (W, b)]
+
+    @torch.no_grad()
+    def _step_impl(self, a0, labels):
+        lib, C = self._lib.lib(), self.C
+        stream = C.c_void_p(torch.cuda.current_stream(a0.device).cuda_stream)
+        vp = lambda t: C.c_void_p(t.data_ptr())
+        logits, _ = self._head(a0, labels, lib, vp, stream)
+        rc = lib.gcnb_nadam_tf_f32(vp(self.flat_p), vp(self.flat_g), vp(self.flat_m), vp(self.flat_v), vp(self.decay),
+                                   vp(self.state), self.n, self.lr, self.b1, self.b2, self.eps,
+                                   float(self.model.regularization or 0.0), 0, stream)
+        self._lib.check(rc, "gcnb_nadam_tf_f32")
+        return self._loss, logits
 
 
 class InputPipeline:

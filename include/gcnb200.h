@@ -304,6 +304,18 @@ GCNB_API int gcnb_adam_tf_f32(float* p, const float* g, float* m, float* v, cons
                      gcnb_stream_t stream);
 
 /*
+ * tf.contrib.opt.NadamOptimizer step (TF's ApplyAdam with use_nesterov = true) over one flat buffer of n parameters --
+ * the optimiser of the fine-tuning model (models_gcn.py:685-933).  Same clock state[4], decay mask and tick rule as
+ * gcnb_adam_tf_f32, no gradient scale:
+ *   g' = g + reg * p (only where decay[i] != 0);  m = b1 m + (1-b1) g';  v = b2 v + (1-b2) g'^2
+ *   p -= lr sqrt(1-b2^t)/(1-b1^t) * (b1 m + (1-b1) g') / (sqrt(v) + eps)
+ * (not Dozat's momentum schedule of Keras' Nadam / torch.optim.NAdam).
+ */
+GCNB_API int gcnb_nadam_tf_f32(float* p, const float* g, float* m, float* v, const uint8_t* decay, float* state,
+                               long long n, float lr, float beta1, float beta2, float eps, float reg, int tick,
+                               gcnb_stream_t stream);
+
+/*
  * Data-parallel training: the gradient all-reduce FUSED into the optimiser update (one ordinary launch; replaces
  * ncclAllReduce + gcnb_adam_tf_f32 on the step's critical path).  Every rank's flat gradient buffer is peer-mapped;
  * the kernel raises one flag per peer over NVLink, waits for all peers' flags, reads all ranks' gradients straight from
