@@ -71,6 +71,8 @@ SIGNATURES = {
     "gcnb_adam_allreduce_flag_bytes": (_z, []),
     "gcnb_adam_tf_allreduce_f32": (_i, [_p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,
                                         _p, _p, _i, _i, _p]),
+    "gcnb_nadam_tf_allreduce_f32": (_i, [_p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,
+                                         _p, _p, _i, _i, _p]),
     "gcnb_adam_tf_f32": (_i, [_p, _p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,
                               C.c_float, C.c_float, _i, _p]),
     "gcnb_nadam_tf_f32": (_i, [_p, _p, _p, _p, _p, _p, C.c_longlong, C.c_float, C.c_float, C.c_float, C.c_float,

@@ -49,6 +49,9 @@ __device__ __forceinline__ float4 ld_cv4(const float* p) {
   return v;
 }
 
+// kNesterov: TF's NadamOptimizer (ApplyAdam with use_nesterov), the step takes b1 m + (1-b1) g_total in place of m --
+// the same rule as k_adam_tf<true> (head.cu).
+template <bool kNesterov>
 __device__ __forceinline__ void adam_one(const AdamArParams& P, long long i, float gsum, float gscale, float lr_t) {
   const float pi = P.p[i];
   float gi = gsum * gscale;
@@ -57,9 +60,10 @@ __device__ __forceinline__ void adam_one(const AdamArParams& P, long long i, flo
   const float vi = fmaf(1.f - P.b2, gi * gi - P.v[i], P.v[i]);
   P.m[i] = mi;
   P.v[i] = vi;
-  P.p[i] = pi - lr_t * mi / (sqrtf(vi) + P.eps);
+  P.p[i] = pi - lr_t * (kNesterov ? fmaf(P.b1, mi, (1.f - P.b1) * gi) : mi) / (sqrtf(vi) + P.eps);
 }
 
+template <bool kNesterov>
 __global__ void __launch_bounds__(256) k_adam_tf_allreduce(const AdamArParams P) {
   uint32_t* myflags = P.flags[P.rank];
   __shared__ uint32_t s_seq;
@@ -81,7 +85,7 @@ __global__ void __launch_bounds__(256) k_adam_tf_allreduce(const AdamArParams P)
   }
   __syncthreads();
   // (3) sum the ranks in rank order straight from peer memory (all peer loads of an element group in flight before the
-  // first add), then Adam
+  // first add), then Adam (Nadam)
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x, nth = (long long)gridDim.x * blockDim.x;
   const long long n4 = P.n >> 2;
   const float lr_t = P.state[2];
@@ -97,15 +101,15 @@ __global__ void __launch_bounds__(256) k_adam_tf_allreduce(const AdamArParams P)
       for (int u = 0; u < 8; ++u)
         if (q0 + u < P.world) { gs.x += v[u].x; gs.y += v[u].y; gs.z += v[u].z; gs.w += v[u].w; }
     }
-    adam_one(P, (i << 2) + 0, gs.x, gscale, lr_t);
-    adam_one(P, (i << 2) + 1, gs.y, gscale, lr_t);
-    adam_one(P, (i << 2) + 2, gs.z, gscale, lr_t);
-    adam_one(P, (i << 2) + 3, gs.w, gscale, lr_t);
+    adam_one<kNesterov>(P, (i << 2) + 0, gs.x, gscale, lr_t);
+    adam_one<kNesterov>(P, (i << 2) + 1, gs.y, gscale, lr_t);
+    adam_one<kNesterov>(P, (i << 2) + 2, gs.z, gscale, lr_t);
+    adam_one<kNesterov>(P, (i << 2) + 3, gs.w, gscale, lr_t);
   }
   for (long long i = (n4 << 2) + tid; i < P.n; i += nth) {
     float gs = 0.f;
     for (int q = 0; q < P.world; ++q) gs += __ldcv(P.grad[q] + i);
-    adam_one(P, i, gs, gscale, lr_t);
+    adam_one<kNesterov>(P, i, gs, gscale, lr_t);
   }
   // the last CTA to finish closes the exchange: only then may the next launch see the new counter
   __syncthreads();
@@ -123,23 +127,21 @@ __global__ void __launch_bounds__(256) k_adam_tf_allreduce(const AdamArParams P)
 
 using namespace gcnb;
 
-extern "C" {
+namespace {
 
-size_t gcnb_adam_allreduce_flag_bytes(void) { return 64 * sizeof(uint32_t); }
-
-int gcnb_adam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* decay, const float* state, long long n,
-                               float beta1, float beta2, float eps, float reg, const void* const* peer_grad,
-                               void* const* peer_flags, int rank, int world, gcnb_stream_t stream) {
-  GCNB_REQUIRE(p && m && v && state && n >= 1 && peer_grad && peer_flags, "gcnb_adam_tf_allreduce_f32: bad arguments");
+int launch_allreduce(bool nesterov, const char* what, float* p, float* m, float* v, const uint8_t* decay,
+                     const float* state, long long n, float beta1, float beta2, float eps, float reg,
+                     const void* const* peer_grad, void* const* peer_flags, int rank, int world, gcnb_stream_t stream) {
+  GCNB_REQUIRE(p && m && v && state && n >= 1 && peer_grad && peer_flags, "%s: bad arguments", what);
   GCNB_REQUIRE(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world,
-               "gcnb_adam_tf_allreduce_f32: rank %d / world %d out of range (at most %d ranks)", rank, world, kMaxRanks);
+               "%s: rank %d / world %d out of range (at most %d ranks)", what, rank, world, kMaxRanks);
   AdamArParams P{};
   P.p = p; P.m = m; P.v = v; P.decay = decay; P.state = state; P.n = n;
   P.b1 = beta1; P.b2 = beta2; P.eps = eps; P.reg = reg; P.rank = rank; P.world = world;
   for (int q = 0; q < world; ++q) {
-    GCNB_REQUIRE(peer_grad[q] != nullptr && peer_flags[q] != nullptr, "gcnb_adam_tf_allreduce_f32: peer pointer %d is NULL", q);
-    GCNB_REQUIRE((reinterpret_cast<uintptr_t>(peer_grad[q]) & 15) == 0,
-                 "gcnb_adam_tf_allreduce_f32: gradient buffers must be 16-byte aligned");
+    GCNB_REQUIRE(peer_grad[q] != nullptr && peer_flags[q] != nullptr, "%s: peer pointer %d is NULL", what, q);
+    GCNB_REQUIRE((reinterpret_cast<uintptr_t>(peer_grad[q]) & 15) == 0, "%s: gradient buffers must be 16-byte aligned",
+                 what);
     P.grad[q] = static_cast<const float*>(peer_grad[q]);
     P.flags[q] = static_cast<uint32_t*>(peer_flags[q]);
   }
@@ -148,9 +150,34 @@ int gcnb_adam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* deca
   if (rc) return rc;
   // at most one CTA per SM: every CTA spins on the flags, so all of them must be resident together with CTA 0
   const int grid = (int)std::max<long long>(1, std::min<long long>(ceil_div_ll(n, 256 * 4), di.sm_count));
-  k_adam_tf_allreduce<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(P);
-  GCNB_LAUNCH_CHECK("k_adam_tf_allreduce");
+  if (nesterov) {
+    k_adam_tf_allreduce<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(P);
+    GCNB_LAUNCH_CHECK("k_adam_tf_allreduce<true>");
+  } else {
+    k_adam_tf_allreduce<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(P);
+    GCNB_LAUNCH_CHECK("k_adam_tf_allreduce");
+  }
   return GCNB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t gcnb_adam_allreduce_flag_bytes(void) { return 64 * sizeof(uint32_t); }
+
+int gcnb_adam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* decay, const float* state, long long n,
+                               float beta1, float beta2, float eps, float reg, const void* const* peer_grad,
+                               void* const* peer_flags, int rank, int world, gcnb_stream_t stream) {
+  return launch_allreduce(false, "gcnb_adam_tf_allreduce_f32", p, m, v, decay, state, n, beta1, beta2, eps, reg,
+                          peer_grad, peer_flags, rank, world, stream);
+}
+
+int gcnb_nadam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* decay, const float* state, long long n,
+                                float beta1, float beta2, float eps, float reg, const void* const* peer_grad,
+                                void* const* peer_flags, int rank, int world, gcnb_stream_t stream) {
+  return launch_allreduce(true, "gcnb_nadam_tf_allreduce_f32", p, m, v, decay, state, n, beta1, beta2, eps, reg,
+                          peer_grad, peer_flags, rank, world, stream);
 }
 
 }  // extern "C"

@@ -6,7 +6,8 @@ The conv layers are frozen and have no dropout, so the head's input for a window
 filters, ``[n0]`` floats -- is a fixed function of the window.  ``fit`` therefore runs every training and validation
 window through the conv stack once (``trunk_features``, the calls ``predict`` makes) and trains the head on that table:
 each step is ``train.HeadTrainer``'s head launch(es) plus one ``gcnb_nadam_tf_f32`` launch, one CUDA graph, fed by
-``train.InputPipeline``.  ``predict``, ``evaluate``, ``saliency``, ``state_dict_tf`` and the checkpoint functions are
+``train.InputPipeline``.  Under a process group (``torchrun``) the trunk batches are dealt over the ranks, every rank
+steps on its shard of each drawn batch and ``gcnb_nadam_tf_allreduce_f32`` averages the head's gradients.  ``predict``, ``evaluate``, ``saliency``, ``state_dict_tf`` and the checkpoint functions are
 ``cgcnn``'s: a saved fine-tuned model loads into a plain ``cgcnn`` built with the same arguments.
 """
 from __future__ import annotations
@@ -72,18 +73,27 @@ class finetuning_cgcnn(cgcnn):
         """The head's input for every window of ``data``: ``mean_f_fwd(conv_stack(batch))`` over ``predict``'s batches,
         ``[n, n0]`` float32 -- bit for bit what ``predict`` and ``forward`` feed the head.  ``gather`` follows
         ``forward``.  ``padded=True`` also returns the rows of the zero windows that pad the last batch
-        (``ceil(n / batch_size) * batch_size`` rows), what ``evaluate_features`` takes."""
+        (``ceil(n / batch_size) * batch_size`` rows), what ``evaluate_features`` takes.  Under a process group each rank
+        runs its share of the batches and every rank gets the whole table, bit for bit one process's."""
         M0 = self.L[0].shape[0]
         if gather is None:
             if self.perm is not None and self.n_input_vertices == M0:
                 raise ValueError("finetuning_cgcnn.trunk_features: with perm set and n_input_vertices == M_0 say "
                                  "gather=True (raw windows) or gather=False (already permuted) -- the shapes are identical")
             gather = self.perm is not None and data.shape[1] == self.n_input_vertices != M0
-        size, bs = data.shape[0], self.batch_size
-        table = np.empty((-(-size // bs) * bs, self.fc_weights[0].shape[0]), np.float32)
-        for begin in range(0, size, bs):
-            h = self.conv_stack(self._padded_batch(data, begin), gather=gather)
-            table[begin:begin + bs] = ops.mean_f_fwd(h).cpu().numpy()
+        from . import train
+
+        size, bs, n0 = data.shape[0], self.batch_size, self.fc_weights[0].shape[0]
+        nb = -(-size // bs)
+        table = np.empty((nb * bs, n0), np.float32)
+        one = lambda j: (ops.mean_f_fwd(self.conv_stack(self._padded_batch(data, j * bs), gather=gather)),)
+        if train.data_parallel()[1] > 1 and nb > 0:
+            # under a process group: the batches dealt over the ranks, the table gathered to every rank (as predict does)
+            batches = train.deal(nb, one, (torch.empty((bs, n0), dtype=torch.float32, device=self.dev),))
+        else:
+            batches = (one(j) for j in range(nb))
+        for j, (h,) in enumerate(batches):
+            table[j * bs:(j + 1) * bs] = h.cpu().numpy()
         return table if padded else table[:size]
 
     @torch.no_grad()

@@ -335,21 +335,43 @@ class cgcnn(nn.Module):
 
     def _predict(self, size, logits_at, labels, return_logits):
         """``predict`` over ``size`` windows with ``logits_at(begin)`` giving the logits of the batch that starts at window
-        ``begin``: the batching, the cropping and the loss of the zero-padded last batch."""
+        ``begin``: the batching, the cropping and the loss of the zero-padded last batch.  Under a process group the
+        batches are dealt round-robin over the ranks (``train.deal``) and their logits and losses gathered to every
+        rank, which assembles them in batch order: the forward pass is batch-independent, so every rank returns
+        bit for bit what one process returns."""
+        from . import train
+
         preds = np.empty(size)
         all_logits = np.empty((size, self.M[-1]), np.float32) if return_logits else None
         total = 0.0
         bs = self.batch_size
-        for begin in range(0, size, bs):
-            end = min(begin + bs, size)
+        nb = -(-size // bs)
+
+        def one(j):
+            begin, end = j * bs, min(j * bs + bs, size)
             logits = logits_at(begin)
+            l = 0.0
             if labels is not None:
                 lab = torch.zeros(bs, dtype=torch.long, device=self.dev)
                 lab[: end - begin] = torch.as_tensor(np.asarray(labels[begin:end]), dtype=torch.long, device=self.dev)
                 l = float(self.loss(logits, lab))
                 if not np.isfinite(l):
                     l = 0.0
-                total += l
+            return logits, l
+
+        def one_as_tensors(j):
+            logits, l = one(j)
+            return logits, torch.tensor(l, dtype=torch.float64)
+
+        if train.data_parallel()[1] > 1 and nb > 0:
+            like = (torch.empty((bs, self.M[-1]), dtype=torch.float32, device=self.dev),
+                    torch.empty((), dtype=torch.float64, device=self.dev))
+            batches = ((lg, float(l)) for lg, l in train.deal(nb, one_as_tensors, like))
+        else:
+            batches = (one(j) for j in range(nb))
+        for j, (logits, l) in enumerate(batches):
+            begin, end = j * bs, min(j * bs + bs, size)
+            total += l
             preds[begin:end] = logits.argmax(1)[: end - begin].cpu().numpy()
             if return_logits:
                 all_logits[begin:end] = logits[: end - begin].detach().cpu().numpy()
@@ -437,34 +459,50 @@ class cgcnn(nn.Module):
                          trainer)
 
     def _fit(self, train_data, train_labels, evaluate, best_checkpoint_dir, trainer):
-        """The loop of ``fit`` on ``train_data`` with ``evaluate()`` giving ``evaluate``'s result at every evaluation."""
+        """The loop of ``fit`` on ``train_data`` with ``evaluate()`` giving ``evaluate``'s result at every evaluation.
+
+        Under a process group (``train.fit`` shards the batches) every rank evaluates its share of the validation batches
+        and gets the same figures; only rank 0 prints and keeps checkpoints, and every rank waits for it at a barrier
+        after each evaluation, so that the kept files exist wherever ``evaluate(checkpoint=...)`` runs next.  Every rank
+        returns the same ``(accuracies, losses, t_step)`` (rank 0's ``t_step``)."""
         import os
         import time
 
+        import torch.distributed as dist
+
         from . import checkpoints, train
 
+        rank, world = train.data_parallel()
+        say = print if rank == 0 else (lambda *a, **k: None)
         path = best_checkpoint_dir or os.path.join("checkpoints", self.dir_name, "model")
-        keeper = checkpoints.BestCheckpoints(path, num_to_keep=3, maximize=True)
+        keeper = checkpoints.BestCheckpoints(path, num_to_keep=3, maximize=True) if rank == 0 else None
         n = train_data.shape[0]
-        print("training with {} steps in total with batch_size={} and epochs={} for training_set={}:".format(
+        say("training with {} steps in total with batch_size={} and epochs={} for training_set={}:".format(
             int(self.num_epochs * n / self.batch_size), self.batch_size, self.num_epochs, n))
         accuracies, losses = [], []
         t_process, t_wall = time.process_time(), time.time()
 
         def on_eval(step, num_steps, loss_average):
-            print("step {} / {} (epoch {:.2f} / {}):".format(step, num_steps, step * self.batch_size / n, self.num_epochs))
-            print("  loss_average = {:.2e}".format(loss_average))
+            say("step {} / {} (epoch {:.2f} / {}):".format(step, num_steps, step * self.batch_size / n, self.num_epochs))
+            say("  loss_average = {:.2e}".format(loss_average))
             string, accuracy, f1, loss = evaluate()
             accuracies.append(accuracy)
             losses.append(loss)
-            print("  validation {}".format(string))
-            print("  time: {:.0f}s (wall {:.0f}s)".format(time.process_time() - t_process, time.time() - t_wall))
-            keeper.handle(accuracy, self, step)
+            say("  validation {}".format(string))
+            say("  time: {:.0f}s (wall {:.0f}s)".format(time.process_time() - t_process, time.time() - t_wall))
+            if keeper is not None:
+                keeper.handle(accuracy, self, step)
+            if world > 1:
+                dist.barrier()
 
         history = train.fit(self, train_data, train_labels, trainer=trainer, seed=None, verbose=False, on_eval=on_eval)
         if accuracies:
-            print("validation accuracy: peak = {:.2f}, mean = {:.2f}".format(max(accuracies), np.mean(accuracies[-10:])))
+            say("validation accuracy: peak = {:.2f}, mean = {:.2f}".format(max(accuracies), np.mean(accuracies[-10:])))
         t_step = (time.time() - t_wall) / max(len(history), 1)
+        if world > 1:
+            t_step = [t_step]
+            dist.broadcast_object_list(t_step, src=0)
+            t_step = t_step[0]
         return accuracies, losses, t_step
 
     def evaluate(self, data, labels, checkpoint=None, target_name=None):
@@ -476,8 +514,10 @@ class cgcnn(nn.Module):
 
         if checkpoint is not None:
             checkpoints.load_checkpoint(self, checkpoint)
+        from .train import data_parallel
+
         predictions, loss = self.predict(data, labels)
-        if target_name is not None:
+        if target_name is not None and data_parallel()[0] == 0:   # under a process group rank 0 prints the report
             print(checkpoints.classification_report(labels, predictions, target_name)[0])
             print("Confusion Matrix:")
             print(checkpoints.confusion_matrix(labels, predictions, len(target_name)))

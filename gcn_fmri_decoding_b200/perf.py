@@ -14,6 +14,7 @@ import sys
 import numpy as np
 
 from . import checkpoints
+from .train import data_parallel
 
 
 def _checkpoint_of_run(ckp_path):
@@ -47,15 +48,17 @@ class model_perf(object):
 
     def test(s, model, name, params, train_data, train_labels, val_data, val_labels, test_data, test_labels,
              target_name=None):
-        """Train ``model``, then evaluate it on the training and the test set (models_gcn.py:944-958)."""
+        """Train ``model``, then evaluate it on the training and the test set (models_gcn.py:944-958).  Under a process
+        group every rank trains its shards and gets the same figures; rank 0 prints."""
+        say = print if data_parallel()[0] == 0 else (lambda *a, **k: None)   # under a process group: rank 0 prints
         s.params[name] = params
         s.fit_accuracies[name], s.fit_losses[name], s.fit_time[name] = model.fit(train_data, train_labels, val_data, val_labels)
         string, s.train_accuracy[name], s.train_f1[name], s.train_loss[name] = model.evaluate(
             train_data, train_labels, target_name=target_name)
-        print("\ntrain {}\n".format(string))
+        say("\ntrain {}\n".format(string))
         string, s.test_accuracy[name], s.test_f1[name], s.test_loss[name] = model.evaluate(
             test_data, test_labels, target_name=target_name)
-        print("\ntest  {}\n".format(string))
+        say("\ntest  {}\n".format(string))
         sys.stdout.flush()
         s.names.add(name)
         return s

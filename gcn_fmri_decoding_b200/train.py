@@ -8,7 +8,10 @@
   Laplacians and weights are replicated and ONE all-reduce of a flat gradient buffer averages
   the gradients (SURVEY 8e).  The reference has no distributed code; this is the only
   collective the path needs.
-* ``fit`` -- the reference's step loop (``:112-184``) without sessions/checkpoints/summaries.
+* ``fit`` -- the reference's step loop (``:112-184``) without sessions/checkpoints/summaries; under a process group
+  every rank draws the reference's global batches and steps on its own shard of each.
+* ``data_parallel`` / ``deal`` -- this process's rank in the process group, and inference batches dealt round-robin
+  over the ranks with the results gathered to every rank (``cgcnn.predict``, ``finetuning_cgcnn.trunk_features``).
 * ``FusedTrainer`` -- the same step with an explicit schedule, one CUDA graph; ``HeadTrainer`` -- its head alone on cached
   conv features with TF's Nadam, the step of the fine-tuning model (``:685-933``).
 """
@@ -16,6 +19,7 @@ from __future__ import annotations
 
 import collections
 import time
+import zlib
 
 import numpy as np
 import torch
@@ -181,6 +185,53 @@ def shard(n, rank, world):
     return lo, lo + base + (1 if rank < rem else 0)
 
 
+def data_parallel():
+    """``(rank, world)`` of this process: its place in the initialised ``torch.distributed`` process group, ``(0, 1)``
+    without one.  ``world > 1`` is what switches ``fit``, ``cgcnn.predict`` and the trainers to data parallelism."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        return dist.get_rank(), dist.get_world_size()
+    return 0, 1
+
+
+def deal(nb, batch_out, like):
+    """Batches ``0 .. nb-1`` dealt round-robin over the ranks of the process group: rank r runs ``batch_out(j)`` for
+    j = r, r + world, ..., which returns one tensor per entry of ``like`` (of that entry's shape, dtype and device).
+    Every rank's results are gathered to every rank (one ``all_gather`` per entry of ``like``); returns the ``nb``
+    result tuples in batch order.  Collective: every rank must call it with the same ``nb`` and ``like`` shapes."""
+    rank, world = data_parallel()
+    per = -(-nb // world)
+    mine = [torch.zeros((per,) + tuple(t.shape), dtype=t.dtype, device=t.device) for t in like]
+    for k, j in enumerate(range(rank, nb, world)):
+        for buf, t in zip(mine, batch_out(j)):
+            buf[k] = t
+    parts = []
+    for buf in mine:
+        got = [torch.empty_like(buf) for _ in range(world)]
+        dist.all_gather(got, buf)
+        parts.append(got)
+    return [tuple(got[j % world][j // world] for got in parts) for j in range(nb)]
+
+
+def _check_training_data(model, train_data, train_labels, world):
+    """Refuse, on EVERY rank and before any step, a data-parallel ``fit`` whose shards would not average to the
+    global-batch gradient (``batch_size % world != 0``, see ``shard``) or whose ranks were given different training
+    sets (shapes and a checksum of a strided sample of rows plus all labels, gathered from every rank)."""
+    n = int(train_data.shape[0])
+    rows = np.unique(np.linspace(0, n - 1, min(n, 64)).astype(np.int64)) if n else np.zeros(0, np.int64)
+    sample = np.ascontiguousarray(np.asarray(train_data[rows]), dtype=np.float32)
+    labels = np.ascontiguousarray(np.asarray(train_labels), dtype=np.int64)
+    mine = (int(model.batch_size), tuple(int(d) for d in train_data.shape), tuple(labels.shape),
+            zlib.crc32(sample.tobytes()), zlib.crc32(labels.tobytes()))
+    every = [None] * world
+    dist.all_gather_object(every, mine)
+    if any(b % world for b, *_ in every):
+        raise ValueError("fit: batch_size %s is not a multiple of the %d ranks -- the averaged gradient is the "
+                         "global-batch gradient only for equal shards" % (sorted({e[0] for e in every}), world))
+    if any(e != every[0] for e in every):
+        raise ValueError("fit: the ranks were given different training data or batch sizes (batch size, data shape, "
+                         "label shape, checksums per rank: %s)" % (every,))
+
+
 def fit(model, train_data, train_labels, val_data=None, val_labels=None, trainer=None, seed=0, verbose=True,
         on_eval=None):
     """The reference's training loop (models_gcn.py:112-184): epochs of random batches from a deque of
@@ -188,24 +239,40 @@ def fit(model, train_data, train_labels, val_data=None, val_labels=None, trainer
 
     ``seed=None`` draws the permutations from NumPy's global generator, as the reference does (:140);
     ``on_eval(step, num_steps, loss)`` replaces the built-in report at every evaluation point (``cgcnn.fit`` uses it
-    for the reference's validation / best-checkpoint bookkeeping)."""
+    for the reference's validation / best-checkpoint bookkeeping).
+
+    Data parallelism (a trainer with ``world > 1``, i.e. ``torch.distributed`` initialised): every rank draws the same
+    global batches of ``model.batch_size`` -- with ``seed=None`` from rank 0's NumPy global-generator state, broadcast at
+    the start -- and gathers and steps on its own rows ``shard(batch_size, rank, world)`` of each.  The history holds
+    the global-batch mean cross-entropy of every step (the mean of the ranks' local means, one scalar all-reduce per
+    step); only rank 0 prints.  ``ValueError`` on every rank, before the first step, if ``batch_size % world != 0`` or
+    the ranks hold different training data."""
     trainer = trainer or Trainer(model)
+    world = int(getattr(trainer, "world", 1))
+    rank = dist.get_rank() if world > 1 else 0
+    if world > 1:
+        _check_training_data(model, train_data, train_labels, world)
+        if seed is None:
+            state = [np.random.get_state()]
+            dist.broadcast_object_list(state, src=0)
+            np.random.set_state(state[0])
     rng = np.random if seed is None else np.random.RandomState(seed)
     n = train_data.shape[0]
     num_steps = int(model.num_epochs * n / model.batch_size)
+    lo, hi = shard(model.batch_size, rank, world)
     indices = collections.deque()
     losses, t0 = [], time.time()
     dev = model.dev
     def draw():
         if len(indices) < model.batch_size:
             indices.extend(rng.permutation(n))
-        idx = [indices.popleft() for _ in range(model.batch_size)]
+        idx = [indices.popleft() for _ in range(model.batch_size)][lo:hi]
         return (np.ascontiguousarray(train_data[idx], dtype=np.float32), np.ascontiguousarray(train_labels[idx]).astype(np.int64))
 
     # a FusedTrainer is fed through the asynchronous input pipeline: the copy of batch i+1 overlaps step i
     pipe = None
     if isinstance(trainer, FusedTrainer) and trainer.use_cuda_graph and torch.device(dev).type == "cuda":
-        pipe = InputPipeline(trainer, (model.batch_size,) + tuple(train_data.shape[1:]))
+        pipe = InputPipeline(trainer, (hi - lo,) + tuple(train_data.shape[1:]))
         if num_steps > 0:
             pipe.feed(*draw())
     for step in range(1, num_steps + 1):
@@ -218,7 +285,12 @@ def fit(model, train_data, train_labels, val_data=None, val_labels=None, trainer
             x = torch.as_tensor(xb, dtype=torch.float32, device=dev)
             y = torch.as_tensor(yb, dtype=torch.long, device=dev)
             loss, _ = trainer.step(x, y, dropout=model.dropout if model.dropout else 1.0)
-        losses.append(float(loss))
+        if world > 1:
+            total = loss.detach().to(torch.float64).reshape(1)
+            dist.all_reduce(total, op=dist.ReduceOp.SUM)
+            losses.append(float(total) / world)
+        else:
+            losses.append(float(loss))
         if on_eval is not None:
             if step % model.eval_frequency == 0 or step == num_steps:
                 on_eval(step, num_steps, losses[-1])
@@ -227,7 +299,8 @@ def fit(model, train_data, train_labels, val_data=None, val_labels=None, trainer
             if val_data is not None:
                 pred, vloss = model.predict(val_data, val_labels)
                 msg += "  val acc %.2f%% loss %.4f" % (100.0 * float(np.mean(pred == np.asarray(val_labels))), vloss)
-            print(msg + "  (%.1fs)" % (time.time() - t0))
+            if rank == 0:
+                print(msg + "  (%.1fs)" % (time.time() - t0))
     return losses
 
 
@@ -616,13 +689,19 @@ class HeadTrainer(FusedTrainer):
     ``gcnb_head_step_f32`` launch for a three-layer head the kernel takes, the layer-by-layer launches otherwise, with the
     same dropout keep-probability, seeds and masks -- followed by ``gcnb_nadam_tf_f32`` (TF's ``NadamOptimizer``) over one
     flat buffer that holds only the FC weights and biases, all regularised.  The conv parameters are never written.
-    Captured as one CUDA graph per batch shape; ``bind_inputs`` lets ``InputPipeline`` feed it."""
+    Captured as one CUDA graph per batch shape; ``bind_inputs`` lets ``InputPipeline`` feed it.
 
-    def __init__(self, model, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, use_cuda_graph=True):
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-            raise NotImplementedError("HeadTrainer: data-parallel fine-tuning is not implemented")
-        super().__init__(model, lr=lr, distributed=False, use_cuda_graph=use_cuda_graph, beta1=beta1, beta2=beta2,
-                         eps=eps, gather=False)
+    Data parallelism as in ``FusedTrainer`` (``torch.distributed`` initialised with ``world > 1``, or
+    ``distributed=True``): each rank steps on its shard, the head's gradients live in peer-mapped symmetric memory and
+    ``gcnb_nadam_tf_allreduce_f32`` averages them and applies Nadam in one launch; without symmetric memory one NCCL
+    all-reduce, a 1/world scale and ``gcnb_nadam_tf_f32``."""
+
+    def __init__(self, model, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, use_cuda_graph=True, distributed=None,
+                 peer_allreduce=True):
+        super().__init__(model, lr=lr, distributed=distributed, use_cuda_graph=use_cuda_graph, beta1=beta1, beta2=beta2,
+                         eps=eps, gather=False, peer_allreduce=peer_allreduce)
+        if self._peer is not None:
+            self.allreduce_kind = "peer-memory (fused into the Nadam kernel)"
 
     def _trained_parameters(self, model):
         """The head's weights and biases (updated with TF Nadam whatever ``model.momentum`` says)."""
@@ -634,9 +713,19 @@ class HeadTrainer(FusedTrainer):
         stream = C.c_void_p(torch.cuda.current_stream(a0.device).cuda_stream)
         vp = lambda t: C.c_void_p(t.data_ptr())
         logits, _ = self._head(a0, labels, lib, vp, stream)
+        reg = float(self.model.regularization or 0.0)
+        if self._peer is not None:
+            rc = lib.gcnb_nadam_tf_allreduce_f32(vp(self.flat_p), vp(self.flat_m), vp(self.flat_v), vp(self.decay),
+                                                 vp(self.state), self.n, self.b1, self.b2, self.eps, reg,
+                                                 self._peer["grads"][self._cur_par], self._peer["flags"],
+                                                 self._peer["rank"], self.world, stream)
+            self._lib.check(rc, "gcnb_nadam_tf_allreduce_f32")
+            return self._loss, logits
+        if self.world > 1:
+            dist.all_reduce(self.flat_g, op=dist.ReduceOp.SUM)
+            self.flat_g.mul_(1.0 / self.world)
         rc = lib.gcnb_nadam_tf_f32(vp(self.flat_p), vp(self.flat_g), vp(self.flat_m), vp(self.flat_v), vp(self.decay),
-                                   vp(self.state), self.n, self.lr, self.b1, self.b2, self.eps,
-                                   float(self.model.regularization or 0.0), 0, stream)
+                                   vp(self.state), self.n, self.lr, self.b1, self.b2, self.eps, reg, 0, stream)
         self._lib.check(rc, "gcnb_nadam_tf_f32")
         return self._loss, logits
 

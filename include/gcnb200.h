@@ -332,6 +332,17 @@ GCNB_API int gcnb_adam_tf_allreduce_f32(float* p, float* m, float* v, const uint
                                         const void* const* peer_grad, void* const* peer_flags, int rank, int world,
                                         gcnb_stream_t stream);
 
+/*
+ * The same fused exchange for the fine-tuning optimiser: gcnb_nadam_tf_f32's update (TF's NadamOptimizer) on the
+ * rank-order sum of every rank's gradient scaled by gscale = 1 / world.  Arguments, flag arrays, the alternating
+ * gradient buffers, the L2 fold and the decay mask are those of gcnb_adam_tf_allreduce_f32; both calls may share one
+ * flag array only if they never run at the same time.
+ */
+GCNB_API int gcnb_nadam_tf_allreduce_f32(float* p, float* m, float* v, const uint8_t* decay, const float* state,
+                                         long long n, float beta1, float beta2, float eps, float reg,
+                                         const void* const* peer_grad, void* const* peer_flags, int rank, int world,
+                                         gcnb_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
