@@ -48,6 +48,9 @@ SIGNATURES = {
     "gcnb_cheb_bwd_f32": (_i, [_p, _p, _i, _p, _p, _p, _i, _p, _CSRP, _CSRP, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),
     "gcnb_cheb_dx_describe": (_i, [_i] * 8 + [C.c_char_p, _z, C.POINTER(_z)]),
     "gcnb_cheb_dx_f32": (_i, [_p, _p, _i, _p, _p, _p, _i, _CSRP, _CSRP, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),
+    "gcnb_cheb_dL_describe": (_i, [_i] * 7 + [C.c_char_p, _z, C.POINTER(_z)]),
+    "gcnb_cheb_dL_f32": (_i, [_p, _p, _i, _p, _p, _p, _i, _CSRP, _CSRP, _p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, _p,
+                              _z, _p]),
     "gcnb_spectral_workspace_bytes": (_z, [_i] * 6),
     "gcnb_spectral_fwd_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),
     "gcnb_spectral_bwd_f32": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),
@@ -116,6 +119,13 @@ def describe_dx(B, M, nnz, Fin, Fout, K, p, algo=ALGO_AUTO):
     """The route of the input-gradient-only call ``gcnb_cheb_dx_f32``, as ``("<route>: <its kernels>", workspace bytes)``."""
     buf, nbytes = C.create_string_buffer(512), _z()
     check(lib().gcnb_cheb_dx_describe(B, M, nnz, Fin, Fout, K, p, algo, buf, 512, C.byref(nbytes)), "gcnb_cheb_dx_describe")
+    return buf.value.decode(), nbytes.value
+
+
+def describe_dL(B, M, nnz, Fin, Fout, K, p):
+    """The kernels of the operator-gradient call ``gcnb_cheb_dL_f32`` and the workspace it takes, as a pair."""
+    buf, nbytes = C.create_string_buffer(512), _z()
+    check(lib().gcnb_cheb_dL_describe(B, M, nnz, Fin, Fout, K, p, buf, 512, C.byref(nbytes)), "gcnb_cheb_dL_describe")
     return buf.value.decode(), nbytes.value
 
 

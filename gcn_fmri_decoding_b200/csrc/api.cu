@@ -336,7 +336,7 @@ using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 104; }
+int gcnb_version(void) { return 105; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 
@@ -568,6 +568,66 @@ int gcnb_cheb_dx_f32(const float* x, const int32_t* perm, int M_in, const float*
                           st);
   }
   if (rc || !perm) return rc;
+  k_perm_scatter<<<grid_for((long long)B * s.M * Fin), 256, 0, st>>>(dxp, perm, dx, B, s.M, M_in, Fin);
+  GCNB_LAUNCH_CHECK("k_perm_scatter");
+  return GCNB_OK;
+}
+
+// workspace of gcnb_cheb_dL_f32: the general path's stacks, the expanded dy (dy_is_mean), the permuted dx (perm)
+static void dL_regions(const LayerShape& s, size_t region[3]) {
+  region[0] = general_cheb_dL_workspace(s);
+  region[1] = align_up((size_t)s.B * ceil_div(s.M, s.p) * s.Fout * sizeof(float), 256) + 256;
+  region[2] = align_up((size_t)s.B * s.M * s.Fin * sizeof(float), 256) + 256;
+}
+
+int gcnb_cheb_dL_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, char* out, size_t n,
+                          size_t* workspace_bytes) {
+  if (!out || n == 0) return GCNB_ERR_INVALID;
+  LayerShape s{B, M, nnz, Fin, Fout, K, p};
+  snprintf(out, n, "general path: HBM-resident state (k_spmm_tma, k_dz_wt), %s",
+           K > 1 ? "k_sddmm_tma on L~'s pattern and diagonal" : "K = 1: zero operator gradient");
+  size_t r[3];
+  dL_regions(s, r);
+  if (workspace_bytes) *workspace_bytes = r[0] + r[1] + r[2];
+  return GCNB_OK;
+}
+
+int gcnb_cheb_dL_f32(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax,
+                     const float* dy, int dy_is_mean, const gcnb_csr* L, const gcnb_csr* Lt, const float* W, float* dval,
+                     float* ddiag, int accumulate, float* dx, int B, int Fin, int Fout, int K, int p, int relu,
+                     void* workspace, size_t workspace_bytes, gcnb_stream_t stream) {
+  int rc = check_layer("gcnb_cheb_dL_f32", L, B, Fin, Fout, K, p, GCNB_BIAS_NONE, nullptr);
+  if (rc) return rc;
+  GCNB_REQUIRE(x && y && dy && W && ddiag && (dval || L->nnz == 0),
+               "gcnb_cheb_dL_f32: x, y, dy, W, dval and ddiag must not be NULL");
+  GCNB_REQUIRE(p == 1 || argmax != nullptr, "gcnb_cheb_dL_f32: argmax is required when p > 1");
+  GCNB_REQUIRE(M_in >= 1 && (perm != nullptr || M_in == L->M),
+               "gcnb_cheb_dL_f32: without perm, M_in (%d) must equal M (%d)", M_in, L->M);
+  GCNB_REQUIRE(K == 1 || (Lt && Lt->M == L->M && Lt->nnz == L->nnz),
+               "gcnb_cheb_dL_f32: needs the transposed operator Lt with the same M and nnz");
+  LayerShape s{B, L->M, L->nnz, Fin, Fout, K, p};
+  size_t r[3];
+  dL_regions(s, r);
+  const size_t need = r[0] + r[1] + r[2];
+  GCNB_REQUIRE(workspace != nullptr && workspace_bytes >= need,
+               "gcnb_cheb_dL_f32: workspace too small (%zu bytes, need %zu from gcnb_cheb_dL_describe)", workspace_bytes,
+               need);
+  char* base = static_cast<char*>(workspace);
+  Workspace ws(base, r[0]), ws1(base + r[0], r[1]), ws2(base + r[0] + r[1], r[2]);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* dxp = (dx && perm) ? ws2.take<float>((size_t)B * s.M * Fin) : dx;  // gradient w.r.t. the permuted input
+  if (dy_is_mean) {
+    float* full = ws1.take<float>((size_t)B * ceil_div(s.M, p) * Fout);
+    if (!full) {
+      set_error("gcnb_cheb_dL_f32: workspace too small");
+      return GCNB_ERR_WORKSPACE;
+    }
+    rc = launch_mean_f_bwd(dy, full, (long long)B * ceil_div(s.M, p), Fout, st);
+    if (rc) return rc;
+    dy = full;
+  }
+  rc = general_cheb_dL(x, perm, M_in, y, argmax, dy, *L, Lt, W, dval, ddiag, accumulate, dxp, s, relu, ws, st);
+  if (rc || !dx || !perm) return rc;
   k_perm_scatter<<<grid_for((long long)B * s.M * Fin), 256, 0, st>>>(dxp, perm, dx, B, s.M, M_in, Fin);
   GCNB_LAUNCH_CHECK("k_perm_scatter");
   return GCNB_OK;

@@ -109,6 +109,16 @@ bool spmm_tma_supported(const gcnb_csr& L, long long C, const float* src, const 
 int spmm_tma(const gcnb_csr& L, const float* src, const float* add, const float* add2, float* out, long long C,
              float alpha, float beta, float beta2, cudaStream_t st);
 
+// ---- gradient w.r.t. the operator L~ (edge saliency), sddmm_tma.cu + general.cu ---------------------------------
+// dval[b][e] (L~'s CSR order) and ddiag[b][i] from the basis stack X and the Clenshaw stack Bk (both [K][M][B*Fin],
+// with 16 bytes of readable slack behind each); K >= 2
+int sddmm_tma(const gcnb_csr& L, const float* X, const float* Bk, float* dval, float* ddiag, int accumulate,
+              const LayerShape& s, cudaStream_t st);
+size_t general_cheb_dL_workspace(const LayerShape& s);
+int general_cheb_dL(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax, const float* dy,
+                    const gcnb_csr& L, const gcnb_csr* Lt, const float* W, float* dval, float* ddiag, int accumulate,
+                    float* dx, const LayerShape& s, int relu, Workspace& ws, cudaStream_t st);
+
 // ---- tcgen05 / TMEM forward for shared-memory resident graphs, cheb_fwd_umma.cu -------------------------
 bool umma_fwd_supported(const LayerShape& s);
 int umma_fwd_describe(const LayerShape& s, char* out, size_t n);  // 0 when the shape is not supported

@@ -579,6 +579,36 @@ int general_cheb_fwd(const float* x, const int32_t* perm, int M_in, const gcnb_c
   return launch_epilogue(Zn, bias, y, argmax, s.B, s.M, s.Fout, s.p, bias_mode, relu, st);
 }
 
+// seeds G_k = dZ W_k^T for every k, then the Clenshaw form of the adjoint recursion, in place on the seeds:
+//   b_k = G_k + 2 L~^T b_{k+1} - b_{k+2}  (k = K-2 .. 1, b_{K-1} = G_{K-1}),   dx = G_0 + L~^T b_1 - b_2
+// Gs ends with dx (vertex-major) in slab 0 and b_1 .. b_{K-1} in slabs 1 .. K-1.  Lt may be NULL when K = 1.
+static int adjoint_states(const float* dZn, int ldz, const float* W, const gcnb_csr* Lt, float* Gs, bool mma_g,
+                          const LayerShape& s, cudaStream_t st) {
+  const long long C = (long long)s.B * s.Fin;
+  const long long slab = (long long)s.M * C;
+  int rc;
+  if (mma_g) {
+    rc = node_dz_wt(dZn, W, Gs, slab, s, st);
+    if (rc) return rc;
+  } else {
+    RowGemm g;
+    g.A = dZn; g.a_q = 0; g.lda = ldz;
+    g.Bm = W; g.b_z = s.Fout; g.b_q = 0; g.sbk = 1; g.sbn = (long long)s.K * s.Fout;
+    g.C = Gs; g.c_z = slab; g.ldc = s.Fin;
+    g.R = (long long)s.M * s.B; g.N = s.Fin; g.Kd = s.Fout; g.nq = 1;
+    rc = launch_rowgemm(g, s.K, st);
+    if (rc) return rc;
+  }
+  for (int k = s.K - 2; k >= 0; --k) {
+    float* bk = Gs + (long long)k * slab;
+    const float* bk1 = Gs + (long long)(k + 1) * slab;
+    const float* bk2 = k + 2 <= s.K - 1 ? Gs + (long long)(k + 2) * slab : nullptr;
+    rc = launch_spmm_step(*Lt, bk1, bk, bk2, bk, C, k == 0 ? 1.f : 2.f, 1.f, -1.f, st);
+    if (rc) return rc;
+  }
+  return GCNB_OK;
+}
+
 int general_cheb_bwd(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax, const float* dy, const gcnb_csr& L,
                      const gcnb_csr* Lt, const float* W, float* dx, float* dW, float* db, const float* xstack,
                      const LayerShape& s, int bias_mode, int relu, Workspace& ws, cudaStream_t st) {
@@ -629,28 +659,61 @@ int general_cheb_bwd(const float* x, const int32_t* perm, int M_in, const float*
     set_error("dx requested but the transposed operator Lt is NULL");
     return GCNB_ERR_INVALID;
   }
-  // seeds G_k = dZ W_k^T for every k, then the Clenshaw form of the adjoint recursion, in place on the seeds:
-  //   b_k = G_k + 2 L~^T b_{k+1} - b_{k+2}  (k = K-2 .. 1, b_{K-1} = G_{K-1}),   dx = G_0 + L~^T b_1 - b_2
-  if (mma_g) {
-    rc = node_dz_wt(dZn, W, Gs, slab, s, st);
-    if (rc) return rc;
-  } else {
-    RowGemm g;
-    g.A = dZn; g.a_q = 0; g.lda = ldz;
-    g.Bm = W; g.b_z = s.Fout; g.b_q = 0; g.sbk = 1; g.sbn = (long long)s.K * s.Fout;
-    g.C = Gs; g.c_z = slab; g.ldc = s.Fin;
-    g.R = R; g.N = s.Fin; g.Kd = s.Fout; g.nq = 1;
-    rc = launch_rowgemm(g, s.K, st);
-    if (rc) return rc;
-  }
-  for (int k = s.K - 2; k >= 0; --k) {
-    float* bk = Gs + (long long)k * slab;
-    const float* bk1 = Gs + (long long)(k + 1) * slab;
-    const float* bk2 = k + 2 <= s.K - 1 ? Gs + (long long)(k + 2) * slab : nullptr;
-    rc = launch_spmm_step(*Lt, bk1, bk, bk2, bk, C, k == 0 ? 1.f : 2.f, 1.f, -1.f, st);
-    if (rc) return rc;
-  }
+  rc = adjoint_states(dZn, ldz, W, Lt, Gs, mma_g, s, st);
+  if (rc) return rc;
   return launch_from_node_major(Gs, dx, s.B, s.M, s.Fin, st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// gradient w.r.t. the operator (edge saliency): the basis X_k and the Clenshaw states b_k of general_cheb_bwd, then
+// dL~ = sum_k c_k b_k X_{k-1}^T sampled on L~'s pattern and diagonal (k_sddmm_tma, sddmm_tma.cu).  No dW, no db.
+// ------------------------------------------------------------------------------------------------
+size_t general_cheb_dL_workspace(const LayerShape& s) {
+  const size_t slab = (size_t)s.M * s.B * s.Fin;
+  size_t n = 0;
+  auto add = [&](size_t floats) { n = align_up(n, 256) + floats * sizeof(float); };
+  add(slab * s.K + 4);                          // X stack (+16 bytes read past the end by the gathers)
+  add((size_t)s.M * s.B * node_mma_ldz(s.Fout));  // dZn
+  add(slab * s.K + 4);                          // G stack -> Clenshaw states
+  return align_up(n, 256) + 256;
+}
+
+int general_cheb_dL(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax, const float* dy,
+                    const gcnb_csr& L, const gcnb_csr* Lt, const float* W, float* dval, float* ddiag, int accumulate,
+                    float* dx, const LayerShape& s, int relu, Workspace& ws, cudaStream_t st) {
+  const long long C = (long long)s.B * s.Fin;
+  const long long slab = (long long)s.M * C;
+  const long long R = (long long)s.M * s.B;
+  // the same kernels, layouts and summation orders as general_cheb_bwd with dx, so that dx agrees bit for bit
+  const bool mma_g = node_dz_wt_supported(s);
+  const int ldz = (node_dw_supported(s) || mma_g) ? node_mma_ldz(s.Fout) : s.Fout;
+  float* Xs = ws.take<float>((size_t)slab * s.K + 4);
+  float* dZn = ws.take<float>((size_t)R * node_mma_ldz(s.Fout));
+  float* Gs = ws.take<float>((size_t)slab * s.K + 4);
+  if (!Xs || !dZn || !Gs) {
+    set_error("workspace too small for the operator gradient");
+    return GCNB_ERR_WORKSPACE;
+  }
+  if (Lt == nullptr && s.K > 1) {
+    set_error("the operator gradient needs the transposed operator Lt");
+    return GCNB_ERR_INVALID;
+  }
+  int rc = launch_dz(dy, y, argmax, dZn, ldz, s.B, s.M, s.Fout, s.p, relu, st);
+  if (rc) return rc;
+  rc = launch_to_node_major(x, perm, Xs, s.B, s.M, M_in, s.Fin, st);
+  if (rc) return rc;
+  rc = build_stack(Xs, L, slab, C, s.K, st);
+  if (rc) return rc;
+  rc = adjoint_states(dZn, ldz, W, Lt, Gs, mma_g, s, st);
+  if (rc) return rc;
+  if (s.K > 1) {
+    rc = sddmm_tma(L, Xs, Gs, dval, ddiag, accumulate, s, st);
+    if (rc) return rc;
+  } else if (!accumulate) {  // a K = 1 layer applies no operator: its gradient is zero
+    GCNB_CUDA(cudaMemsetAsync(dval, 0, (size_t)s.B * L.nnz * sizeof(float), st));
+    GCNB_CUDA(cudaMemsetAsync(ddiag, 0, (size_t)s.B * s.M * sizeof(float), st));
+  }
+  return dx ? launch_from_node_major(Gs, dx, s.B, s.M, s.Fin, st) : GCNB_OK;
 }
 
 }  // namespace gcnb

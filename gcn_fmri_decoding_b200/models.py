@@ -62,11 +62,13 @@ class cgcnn(nn.Module):
 
         # ---- keep the useful Laplacians only (models_gcn.py:462-469) ------------------------------
         M_0 = L[0].shape[0]
-        j, used = 0, []
+        j, used, levels = 0, [], []
         for pp in p:
             used.append(L[j])
+            levels.append(j)
             j += int(np.log2(pp)) if pp > 1 else 0
         self.L, self.F, self.K, self.p, self.M = used, list(F), list(K), list(p), list(M)
+        self._graph_levels = levels  # layer i uses L[levels[i]] of the constructor's list (graph_saliency's keys)
         self.num_epochs, self.learning_rate = num_epochs, learning_rate
         self.decay_rate, self.decay_steps, self.momentum = decay_rate, decay_steps, momentum
         self.regularization, self.dropout = regularization, dropout
@@ -422,6 +424,67 @@ class cgcnn(nn.Module):
             grads[begin:end] = g[: end - begin].cpu().numpy()
             targets[begin:end] = tg[: end - begin].cpu().numpy()
         return grads, targets
+
+    def graph_saliency(self, data, target=None, gather=None, absolute=False):
+        """Edge saliency maps: which connections of the brain graph the decision relies on.  Returns ``{level:
+        scipy.sparse.csr_matrix (float64)}`` for every level of the constructor's ``L`` list the network uses, each with
+        the sparsity pattern of that ``L`` (its stored entries and the whole diagonal), holding
+        ``sum_w d logit_{target_w}(x_w) / d L[i, j]`` over the windows ``w`` of ``data`` -- with ``absolute`` the sum of
+        ``|d logit / d L[i, j]|`` per window instead, each window's gradient summing every layer that uses the level
+        before the absolute value is taken.
+
+        This is the gradient w.r.t. the entries of the Laplacian (the kernels' ``L~ = L - I``), not the adjacency: the
+        chain rule through the degree normalisation is not applied.  The matrices are not symmetric; ``G + G.T`` scores
+        an undirected edge.  ``target`` and ``gather`` mean what they mean in ``saliency``; with raw windows (``gather``)
+        the level-0 matrix is in input-ROI order, ``[n_input_vertices, n_input_vertices]``, without the entries of
+        fake vertices; coarser levels stay in the model's vertex order.  Batched like ``predict`` (the padding windows of
+        the last batch contribute nothing); the per-batch sums are added on the host in float64 in batch order.  Runs on
+        the GPU through ``saliency.GraphGradient`` (one CUDA graph per batch shape).  The ``fourier`` filter is refused:
+        its operator is the eigenbasis of ``L``, not ``L``."""
+        from .saliency import GraphGradient, edge_matrix, to_input_order
+
+        if self.filter_name == "fourier":
+            raise ValueError("cgcnn.graph_saliency: the fourier filter's operator is the eigenbasis U, not the Laplacian L")
+        M0 = self.L[0].shape[0]
+        if gather is None:
+            if self.perm is not None and self.n_input_vertices == M0:
+                raise ValueError("cgcnn.graph_saliency: with perm set and n_input_vertices == M_0 say gather=True (raw "
+                                 "windows) or gather=False (already permuted) -- the shapes are identical")
+            gather = self.perm is not None and data.shape[1] == self.n_input_vertices != M0
+        gather = bool(gather) and self.perm is not None
+        perm = None
+        if gather:
+            perm = self.perm.cpu().numpy()
+            if not np.array_equal(np.sort(perm), np.arange(M0)):
+                raise ValueError("cgcnn.graph_saliency: perm is not a permutation of [0, M_0 = %d)" % M0)
+        params = tuple(p.data_ptr() for p in self.parameters())
+        cached = self.__dict__.get("_graph_saliency")
+        if cached is None or cached[0] != params:
+            cached = self.__dict__["_graph_saliency"] = (params, GraphGradient(self))
+        gg = cached[1]
+        size, bs = data.shape[0], self.batch_size
+        sums = {}
+        for begin in range(0, size, bs):
+            end = min(begin + bs, size)
+            batch = self._padded_batch(data, begin)
+            t = None
+            if target is not None:
+                t = torch.zeros(bs, dtype=torch.long, device=self.dev)
+                t[: end - begin] = torch.as_tensor(np.asarray(target[begin:end]), dtype=torch.long, device=self.dev)
+            out, _, _ = gg(batch, t, gather=gather, valid=end - begin, absolute=absolute)
+            for lvl, g in out.items():
+                v = g.cpu().numpy().astype(np.float64)
+                sums[lvl] = sums[lvl] + v if lvl in sums else v
+        result = {}
+        for i, lvl in enumerate(self._graph_levels):
+            if lvl in result:
+                continue
+            pl = self._plan(self.L[i])
+            G = edge_matrix(pl, sums[lvl] if lvl in sums else np.zeros(pl.nnz + pl.M))
+            if lvl == 0 and gather:
+                G = to_input_order(G, perm, self.n_input_vertices)
+            result[lvl] = G
+        return result
 
     # ------------------------------------------------------------------ base_model's small public methods
     def inference(self, data, dropout=1.0):

@@ -15,6 +15,8 @@ Op                       replaces (``/root/reference/lib_new/models_gcn.py``)
 ``mean_f_fwd / _bwd``     tf.reduce_mean(x, -1) of ``_inference`` ``:673``
 ``cheb_dx``               input gradient of a ChebyNet layer alone (saliency maps, ``saliency.py``; no reference
                           counterpart)
+``cheb_dL``               gradient of a ChebyNet layer w.r.t. its operator's entries (edge saliency maps,
+                          ``saliency.GraphGradient``; no reference counterpart)
 """
 from __future__ import annotations
 
@@ -293,6 +295,48 @@ def cheb_dx(x: Optional[Tensor], perm: Optional[Tensor], M_in: int, y: Tensor, a
 @cheb_dx.register_fake
 def _(x, perm, M_in, y, argmax, dy, dy_is_mean, rowptr, col, val, rowptr_t, col_t, val_t, W, K, p, relu, algo):
     return y.new_empty((y.shape[0], M_in, W.shape[0] // K))
+
+
+@torch.library.custom_op("gcn_b200::cheb_dL", mutates_args=("dval", "ddiag"), device_types="cuda")
+def cheb_dL(x: Tensor, perm: Optional[Tensor], M_in: int, y: Tensor, argmax: Tensor, dy: Tensor, dy_is_mean: bool,
+            rowptr: Tensor, col: Tensor, val: Tensor, rowptr_t: Tensor, col_t: Tensor, val_t: Tensor, W: Tensor,
+            dval: Tensor, ddiag: Tensor, accumulate: bool, K: int, p: int, relu: bool, need_dx: bool) -> Tensor:
+    """Gradient of a ChebyNet layer w.r.t. the entries of its operator (``gcnb_cheb_dL_f32``), per window: into
+    ``dval [B, nnz]`` (L~'s CSR entries) and ``ddiag [B, M]`` (the diagonal ``(i, i)``), both contiguous float32;
+    ``accumulate`` adds onto them (layers that share an operator).  Returns the layer's input gradient with ``need_dx``
+    (bit for bit ``cheb_dx`` on the general path, un-permuted through ``perm``), else an empty tensor."""
+    dy = dy.contiguous()
+    x = x.contiguous()
+    B, M = y.shape[0], rowptr.numel() - 1
+    Fout = W.shape[1]
+    Fin = W.shape[0] // K
+    nnz = val.numel()
+    if perm is None and M_in != M:
+        raise ValueError("without perm the layer input has M = %d vertices (got M_in = %d)" % (M, M_in))
+    if perm is not None and (perm.dtype != torch.int32 or perm.numel() != M):
+        raise ValueError("perm must be int32 with one entry per (padded) vertex")
+    if tuple(x.shape) != (B, M_in, Fin):
+        raise ValueError("x must be [B, M_in, Fin] = %s, got %s" % ((B, M_in, Fin), tuple(x.shape)))
+    for name, t, shape in (("dval", dval, (B, nnz)), ("ddiag", ddiag, (B, M))):
+        if tuple(t.shape) != shape or t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError("%s must be a contiguous float32 %s tensor" % (name, shape))
+    dx = torch.empty((B, M_in, Fin) if need_dx else (0,), dtype=torch.float32, device=y.device)
+    L = _lib.lib()
+    _, nbytes = _lib.describe_dL(B, M, nnz, Fin, Fout, K, p)
+    ws = _workspace(nbytes, y.device)
+    csr = csr_struct(rowptr, col, val)
+    csr_t = csr_struct(rowptr_t, col_t, val_t)
+    rc = L.gcnb_cheb_dL_f32(_ptr(x), _ptr(perm), M_in, _ptr(y), _ptr(argmax), _ptr(dy), int(dy_is_mean), C.byref(csr),
+                            C.byref(csr_t), _ptr(W.contiguous()), _ptr(dval), _ptr(ddiag), int(accumulate), _ptr(dx), B,
+                            Fin, Fout, K, p, int(relu), _ptr(ws), ws.numel(), _stream(y))
+    _lib.check(rc, "gcnb_cheb_dL_f32")
+    return dx
+
+
+@cheb_dL.register_fake
+def _(x, perm, M_in, y, argmax, dy, dy_is_mean, rowptr, col, val, rowptr_t, col_t, val_t, W, dval, ddiag, accumulate, K,
+      p, relu, need_dx):
+    return y.new_empty((y.shape[0], M_in, W.shape[0] // K) if need_dx else (0,))
 
 
 def unpermute(dx: Tensor, perm: Tensor, M_in: int) -> Tensor:

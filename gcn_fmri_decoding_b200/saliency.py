@@ -14,6 +14,10 @@ backward: ``EPI_MASK`` GEMMs down to the gradient of the mean -> ``ops.cheb_dx``
 
 The whole schedule is captured as one CUDA graph per batch shape.
 
+``GraphGradient`` (``cgcnn.graph_saliency``) differentiates the same logit w.r.t. the entries of the graph Laplacians
+instead: the same forward, seed and head backward, then ``ops.cheb_dL`` per conv layer (the operator gradient of
+``k_sddmm_tma`` on the general path's stacks, and the input gradient that feeds the layer below).
+
 The ``fourier`` filter has no input-gradient-only kernel: its layers go through ``spectral_bwd(need_dx=True)``, which also
 computes the weight and bias gradients that are then dropped, and the first layer is un-permuted by ``ops.unpermute``.
 That path is correct but not optimised.
@@ -22,6 +26,8 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
+import scipy.sparse as sp
 import torch
 
 from . import _lib, ops
@@ -49,7 +55,10 @@ class InputGradient:
 
     # -- one run, eagerly --------------------------------------------------------------------------------------------
     @torch.no_grad()
-    def _impl(self, x, target, gather):
+    def _forward(self, x, target, gather, mask=None):
+        """The forward pass, the seed and the head backward: ``(saved, d, logits, target)`` with ``saved[i] = (layer
+        input, perm, y, argmax, plan)`` and ``d`` the gradient of the mean over the last conv layer's filters.  ``mask``
+        (float32 [B] of 0 / 1, optional) zeroes the seed of the rows marked 0."""
         m = self.model
         lib = _lib.lib()
         stream = C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
@@ -105,6 +114,8 @@ class InputGradient:
         # ---- seed and head backward: d = one-hot(target); d <- (d W^T) masked by the activation it came from ----
         d = torch.zeros_like(logits)
         d.scatter_(1, target.view(-1, 1), 1.0)
+        if mask is not None:
+            d.mul_(mask.view(-1, 1))
         for i in range(nfc - 1, -1, -1):
             W = m.fc_weights[i]
             dn = torch.empty((B, W.shape[0]), dtype=torch.float32, device=x.device)
@@ -112,6 +123,16 @@ class InputGradient:
                 d = gemm(d, W, dn, None, 0, 1, B, W.shape[0], W.shape[1], _lib.EPI_MASK, acts[i])
             else:
                 d = gemm(d, W, dn, None, 0, 1, B, W.shape[0], W.shape[1])
+        return saved, d, logits, target
+
+    @torch.no_grad()
+    def _impl(self, x, target, gather):
+        m = self.model
+        mode = m._bias_mode()
+        cheb = m.filter_name != "fourier"
+        nconv = len(m.p)
+        saved, d, logits, target = self._forward(x, target, gather)
+        h = saved[-1][2]
         # ---- conv backward: input gradients only (d is the gradient of the mean over the last layer's filters) ----
         if cheb:
             dy, dy_is_mean = d, True
@@ -163,3 +184,130 @@ class InputGradient:
             st.copy_(target, non_blocking=True)
         graph.replay()
         return out
+
+
+class GraphGradient(InputGradient):
+    """``grads, logits, target = GraphGradient(model)(x, target=None, gather=False, valid=None, absolute=False)``: the
+    gradient of ``logits[b, target[b]]`` w.r.t. every entry of every graph Laplacian the network uses -- which
+    connections of the graph the decision relies on -- summed over the windows ``b`` of the batch.
+
+    ``grads[level]`` (float32 ``[nnz + M]``, ``level`` an index into the model's constructor ``L`` list) holds the
+    entries of the rescaled operator's CSR pattern (``GraphPlan``'s order) followed by the diagonal ``(i, i)``.  The
+    gradient w.r.t. ``L~ = L - I`` is the gradient w.r.t. ``L``.  ``valid``: the first ``valid`` rows are windows, the
+    rest padding, whose seed is zero.  ``absolute``: ``sum_b |dL_b|`` instead of ``sum_b dL_b``, the absolute value taken
+    per window after the contributions of every layer that uses the Laplacian are added up.
+
+    Schedule: ``InputGradient``'s forward, seed and head backward, then from the top conv layer down one
+    ``ops.cheb_dL`` per layer, accumulating into one ``[B, nnz + M]`` buffer per distinct Laplacian (its ``dx`` feeds the
+    layer below), and a fixed-order sum over the windows per buffer (``gcnb_colsum_multi_f32``).  One CUDA graph per
+    batch shape.  The ``fourier`` filter is refused: its operator is the eigenbasis, not ``L``.
+    """
+
+    def __init__(self, model, use_cuda_graph=True):
+        if model.filter_name == "fourier":
+            raise ValueError("GraphGradient: the fourier filter's operator is the eigenbasis U, not the Laplacian L")
+        super().__init__(model, use_cuda_graph)
+
+    @torch.no_grad()
+    def _impl(self, x, target, gather, mask=None, absolute=False):
+        m = self.model
+        lib = _lib.lib()
+        stream = C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
+        nconv = len(m.p)
+        saved, dy, logits, target = self._forward(x, target, gather, mask)
+        B = x.shape[0]
+        bufs = {}  # level -> (dL [B, nnz + M] as its dval [B, nnz] and ddiag [B, M] blocks)
+        dy_is_mean = True
+        for i in range(nconv - 1, -1, -1):
+            hin, perm, y, am, pl = saved[i]
+            lvl = m._graph_levels[i]
+            accumulate = lvl in bufs
+            if not accumulate:
+                buf = torch.empty(B * (pl.nnz + pl.M), dtype=torch.float32, device=x.device)
+                bufs[lvl] = (buf, buf[: B * pl.nnz].view(B, pl.nnz), buf[B * pl.nnz:].view(B, pl.M))
+            _, dval, ddiag = bufs[lvl]
+            M_in = x.shape[1] if i == 0 else hin.shape[1]
+            dy = ops.cheb_dL(hin, perm, M_in, y, am, dy, dy_is_mean, *pl.tensors(), m.conv_weights[i], dval, ddiag,
+                             accumulate, m.K[i], m.p[i], True, i > 0)
+            dy_is_mean = False
+        # ---- sum over the windows, fixed order: the dval and ddiag blocks of every buffer as column sums ----
+        out, mats = {}, []
+        for lvl, (buf, dval, ddiag) in sorted(bufs.items()):
+            if absolute:
+                buf.abs_()
+            o = torch.empty(dval.shape[1] + ddiag.shape[1], dtype=torch.float32, device=x.device)
+            out[lvl] = o
+            if dval.shape[1]:
+                mats.append((dval, o[: dval.shape[1]]))
+            mats.append((ddiag, o[dval.shape[1]:]))
+        for c in range(0, len(mats), 4):
+            part = mats[c:c + 4]
+            n = len(part)
+            rc = lib.gcnb_colsum_multi_f32((C.c_void_p * n)(*[a.data_ptr() for a, _ in part]),
+                                           (C.c_void_p * n)(*[o.data_ptr() for _, o in part]),
+                                           (C.c_int * n)(*[a.shape[0] for a, _ in part]),
+                                           (C.c_int * n)(*[a.shape[1] for a, _ in part]), n, stream)
+            _lib.check(rc, "gcnb_colsum_multi_f32")
+        return out, logits, target
+
+    def __call__(self, x, target=None, gather=False, valid=None, absolute=False):
+        """``({level: float32 [nnz + M]}, logits [B, C], target [B] int64)`` for the batch ``x`` (float32, on the model's
+        device); ``target`` (int64 [B] or None) is the class whose logit is differentiated, ``valid`` the number of
+        leading rows that are windows (None: all)."""
+        gather = bool(gather) and self.model.perm is not None
+        B = x.shape[0]
+        valid = B if valid is None else int(valid)
+        mask = (torch.arange(B, device=x.device) < valid).to(torch.float32)
+        if target is not None:
+            target = torch.as_tensor(target, dtype=torch.long, device=x.device)
+        if not self.use_cuda_graph:
+            return self._impl(x, target, gather, mask, bool(absolute))
+        key = (tuple(x.shape), gather, target is not None, bool(absolute))
+        if key not in self._graphs:
+            sx, sm = torch.empty_like(x), torch.empty_like(mask)
+            st = torch.zeros(B, dtype=torch.long, device=x.device) if target is not None else None
+            sx.copy_(x)
+            sm.copy_(mask)
+            if st is not None:
+                st.copy_(target)
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                for _ in range(2):  # warm up: allocator, lazy library set-up, operator images
+                    self._impl(sx, st, gather, sm, bool(absolute))
+            torch.cuda.current_stream().wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                out = self._impl(sx, st, gather, sm, bool(absolute))
+            self._graphs[key] = (sx, st, sm, out, graph)
+        sx, st, sm, out, graph = self._graphs[key]
+        sx.copy_(x, non_blocking=True)
+        sm.copy_(mask, non_blocking=True)
+        if st is not None:
+            st.copy_(target, non_blocking=True)
+        graph.replay()
+        return out
+
+
+def edge_matrix(plan, g):
+    """``[M, M]`` float64 CSR from a ``GraphGradient`` vector ``g [nnz + M]`` of ``plan``'s operator: the off-diagonal
+    entries of its CSR pattern and the whole diagonal (the pattern of ``L``).  A diagonal entry the operator stores
+    itself holds the same quantity as ``g[nnz + i]`` and is taken from there once."""
+    rp, ci, _ = plan._host[False]
+    M, nnz = plan.M, plan.nnz
+    g = np.asarray(g, np.float64)
+    rows = np.repeat(np.arange(M), np.diff(rp))
+    off = rows != ci
+    r = np.concatenate([rows[off], np.arange(M)])
+    c = np.concatenate([ci[off], np.arange(M)])
+    v = np.concatenate([g[:nnz][off], g[nnz:]])
+    return sp.csr_matrix((v, (r, c)), shape=(M, M))
+
+
+def to_input_order(G, perm, M_in):
+    """A level-0 edge matrix in the model's vertex order -> input-ROI order ``[M_in, M_in]``: entry ``(i, j)`` goes to
+    ``(perm[i], perm[j])``; entries that touch a fake vertex (``perm >= M_in``) are dropped."""
+    perm = np.asarray(perm)
+    G = sp.coo_matrix(G)
+    keep = (perm[G.row] < M_in) & (perm[G.col] < M_in)
+    return sp.csr_matrix((G.data[keep], (perm[G.row[keep]], perm[G.col[keep]])), shape=(M_in, M_in))

@@ -197,6 +197,29 @@ GCNB_API int gcnb_cheb_dx_f32(const float* x, const int32_t* perm, int M_in, con
                               size_t workspace_bytes, gcnb_stream_t stream);
 
 /*
+ * Gradient of a ChebyNet layer w.r.t. the entries of its operator L~ (edge saliency maps), per window.  With dz rebuilt
+ * from dy / y / argmax as in gcnb_cheb_bwd_f32, G_k = dz W_k^T and the Clenshaw states of the adjoint
+ *   b_{K-1} = G_{K-1},  b_k = G_k + 2 L~^T b_{k+1} - b_{k+2}  (k = K-2 .. 1),
+ * the gradient of <dy, layer(x)> is
+ *   dL~[b][i][j] = sum_f b_1[i][b][f] X_0[j][b][f] + sum_{k=2}^{K-1} 2 sum_f b_k[i][b][f] X_{k-1}[j][b][f]
+ * (X_k the Chebyshev basis of the permuted input), on L~'s pattern and on the diagonal:
+ *   dval  [B][nnz]  entry e of L~'s CSR order (may be NULL when nnz = 0)
+ *   ddiag [B][M]    entry (i, i), whether or not L~ stores it
+ * L~ = L - I (lmax = 2), so these are also the gradients w.r.t. the entries of the Laplacian L.  K = 1 gives zeros.
+ * accumulate != 0 adds onto dval / ddiag instead of overwriting them (layers that share an operator).  dx (nullable) is
+ * the layer's input gradient, as gcnb_cheb_dx_f32 computes it on the general path (bit for bit), un-permuted through
+ * perm to [B][M_in][Fin] when perm is given.  No dW, no db.  Lt is required when K > 1.  No allocation and no
+ * synchronisation: the call can be captured in a CUDA graph.  Runs on the general path (HBM-resident stacks) and
+ * k_sddmm_tma; the workspace is gcnb_cheb_dL_describe's (256-byte aligned pointer).
+ */
+GCNB_API int gcnb_cheb_dL_describe(int B, int M, int nnz, int Fin, int Fout, int K, int p, char* out, size_t n,
+                                   size_t* workspace_bytes);
+GCNB_API int gcnb_cheb_dL_f32(const float* x, const int32_t* perm, int M_in, const float* y, const uint8_t* argmax,
+                              const float* dy, int dy_is_mean, const gcnb_csr* L, const gcnb_csr* Lt, const float* W,
+                              float* dval, float* ddiag, int accumulate, float* dx, int B, int Fin, int Fout, int K,
+                              int p, int relu, void* workspace, size_t workspace_bytes, gcnb_stream_t stream);
+
+/*
  * Spectral layer (cgcnn.fourier + filter_in_fourier, models_gcn.py:512-539) with the same fused
  * bias/ReLU/pool epilogue.  Ut[M][M] is the transposed eigenvector matrix (row i = i-th
  * eigenvector), exactly the constant the reference builds at :536.  W[M][Fout][Fin].
