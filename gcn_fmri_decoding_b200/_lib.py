@@ -26,8 +26,17 @@ class GcnbCsr(C.Structure):
                 ("image", C.c_void_p), ("image_bytes", C.c_size_t)]
 
 
+class GcnbAdjLevel(C.Structure):
+    """``struct gcnb_adj_level`` -- one coarsening level of ``gcnb_adjacency_grad_f32`` (device pointers)."""
+
+    _fields_ = [("dval", C.c_void_p), ("rowptr", C.c_void_p), ("val", C.c_void_p), ("rowptr_t", C.c_void_p),
+                ("tpos", C.c_void_p), ("ss", C.c_void_p), ("hinv", C.c_void_p), ("parent", C.c_void_p),
+                ("M", C.c_int32), ("nnz", C.c_int32)]
+
+
 _i, _p, _z = C.c_int, C.c_void_p, C.c_size_t
 _CSRP = C.POINTER(GcnbCsr)
+_ADJP = C.POINTER(GcnbAdjLevel)
 
 # name -> (restype, argtypes); must list every symbol include/gcnb200.h declares
 SIGNATURES = {
@@ -51,6 +60,8 @@ SIGNATURES = {
     "gcnb_cheb_dL_describe": (_i, [_i] * 7 + [C.c_char_p, _z, C.POINTER(_z)]),
     "gcnb_cheb_dL_f32": (_i, [_p, _p, _i, _p, _p, _p, _i, _CSRP, _CSRP, _p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, _p,
                               _z, _p]),
+    "gcnb_adjacency_grad_workspace_bytes": (_z, [_ADJP, _i, _i]),
+    "gcnb_adjacency_grad_f32": (_i, [_ADJP, _i, _p, _i, _p, _i, _i, _p, _z, _p]),
     "gcnb_spectral_workspace_bytes": (_z, [_i] * 6),
     "gcnb_spectral_fwd_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),
     "gcnb_spectral_bwd_f32": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _z, _p]),

@@ -336,7 +336,7 @@ using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 105; }
+int gcnb_version(void) { return 106; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 
@@ -631,6 +631,35 @@ int gcnb_cheb_dL_f32(const float* x, const int32_t* perm, int M_in, const float*
   k_perm_scatter<<<grid_for((long long)B * s.M * Fin), 256, 0, st>>>(dxp, perm, dx, B, s.M, M_in, Fin);
   GCNB_LAUNCH_CHECK("k_perm_scatter");
   return GCNB_OK;
+}
+
+size_t gcnb_adjacency_grad_workspace_bytes(const gcnb_adj_level* levels, int nlevels, int B) {
+  if (!levels || nlevels < 1 || nlevels > GCNB_ADJ_MAX_LEVELS || B < 1) return 0;
+  return adjacency_grad_workspace(levels, nlevels, B);
+}
+
+int gcnb_adjacency_grad_f32(const gcnb_adj_level* levels, int nlevels, const int32_t* edges, int E, float* out, int B,
+                            int absolute, void* workspace, size_t workspace_bytes, gcnb_stream_t stream) {
+  GCNB_REQUIRE(levels && nlevels >= 1 && nlevels <= GCNB_ADJ_MAX_LEVELS,
+               "gcnb_adjacency_grad_f32: 1..%d levels (got %d)", GCNB_ADJ_MAX_LEVELS, nlevels);
+  GCNB_REQUIRE(B >= 1 && E >= 0, "gcnb_adjacency_grad_f32: bad B (%d) or E (%d)", B, E);
+  GCNB_REQUIRE(E == 0 || (edges && out && levels[0].nnz > 0),
+               "gcnb_adjacency_grad_f32: edges and out must not be NULL, and level 0 must have entries, when E > 0");
+  for (int l = 0; l < nlevels; ++l) {
+    const gcnb_adj_level& lv = levels[l];
+    const bool last = l == nlevels - 1;
+    GCNB_REQUIRE(lv.M >= 1 && lv.nnz >= 0, "gcnb_adjacency_grad_f32: level %d: bad M (%d) or nnz (%d)", l, lv.M, lv.nnz);
+    GCNB_REQUIRE(lv.nnz == 0 || (lv.dval && lv.rowptr && lv.val && lv.rowptr_t && lv.tpos && lv.ss && lv.hinv),
+                 "gcnb_adjacency_grad_f32: level %d: dval, rowptr, val, rowptr_t, tpos, ss and hinv must not be NULL", l);
+    GCNB_REQUIRE(last == (lv.parent == nullptr) || lv.nnz == 0,
+                 "gcnb_adjacency_grad_f32: level %d: parent must be %s", l, last ? "NULL on the last level" : "given");
+  }
+  const size_t need = adjacency_grad_workspace(levels, nlevels, B);
+  GCNB_REQUIRE(workspace != nullptr && workspace_bytes >= need,
+               "gcnb_adjacency_grad_f32: workspace too small (%zu bytes, need %zu from "
+               "gcnb_adjacency_grad_workspace_bytes)", workspace_bytes, need);
+  Workspace ws(workspace, workspace_bytes);
+  return adjacency_grad(levels, nlevels, edges, E, out, B, absolute, ws, static_cast<cudaStream_t>(stream));
 }
 
 int gcnb_brelu_fwd_f32(const float* x, const float* bias, float* y, int B, int M, int F, int bias_mode,

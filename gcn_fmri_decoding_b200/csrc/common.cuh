@@ -119,6 +119,11 @@ int general_cheb_dL(const float* x, const int32_t* perm, int M_in, const float* 
                     const gcnb_csr& L, const gcnb_csr* Lt, const float* W, float* dval, float* ddiag, int accumulate,
                     float* dx, const LayerShape& s, int relu, Workspace& ws, cudaStream_t st);
 
+// ---- gradient w.r.t. the adjacency (the chain through the normalisation and the coarsening), adjacency_grad.cu ----
+size_t adjacency_grad_workspace(const gcnb_adj_level* levels, int nlevels, int B);
+int adjacency_grad(const gcnb_adj_level* levels, int nlevels, const int32_t* edges, int E, float* out, int B,
+                   int absolute, Workspace& ws, cudaStream_t st);
+
 // ---- tcgen05 / TMEM forward for shared-memory resident graphs, cheb_fwd_umma.cu -------------------------
 bool umma_fwd_supported(const LayerShape& s);
 int umma_fwd_describe(const LayerShape& s, char* out, size_t n);  // 0 when the shape is not supported

@@ -69,6 +69,7 @@ class cgcnn(nn.Module):
             j += int(np.log2(pp)) if pp > 1 else 0
         self.L, self.F, self.K, self.p, self.M = used, list(F), list(K), list(p), list(M)
         self._graph_levels = levels  # layer i uses L[levels[i]] of the constructor's list (graph_saliency's keys)
+        self._n_laplacians = len(L)  # A's coarsening has len(L) - 1 levels (adjacency_saliency)
         self.num_epochs, self.learning_rate = num_epochs, learning_rate
         self.decay_rate, self.decay_steps, self.momentum = decay_rate, decay_steps, momentum
         self.regularization, self.dropout = regularization, dropout
@@ -485,6 +486,59 @@ class cgcnn(nn.Module):
                 G = to_input_order(G, perm, self.n_input_vertices)
             result[lvl] = G
         return result
+
+    def adjacency_saliency(self, data, A, target=None, gather=None, absolute=False):
+        """Edge saliency maps in the coordinates the graph was built in: which functional connections drive the decision.
+        ``A`` is the symmetric, zero-diagonal adjacency ``[n_roi, n_roi]`` (scipy sparse or dense) that the
+        constructor's ``L`` list was built from (``graclus.coarsen(A, len(L) - 1)`` then ``graphs.laplacian`` per level,
+        as the reference's ``model.py`` does).  Returns a symmetric ``scipy.sparse.csr_matrix`` (float64) on the pattern
+        of ``A``, in ROI order, whose entry ``(i, j) = (j, i)`` is ``sum_w d logit_{target_w}(x_w) / d w_ij``: the
+        gradient w.r.t. the weight of the undirected edge ``{i, j}``, collecting every path through which it reaches the
+        network (the level-0 Laplacian's entries and degrees, and every coarser Laplacian built from the Graclus-summed
+        graphs with its own degrees).  With ``absolute`` the sum over windows of ``|d logit / d w_ij|``, taken per
+        window after all those paths are added up.
+
+        The Graclus matching is held fixed: its discrete pairing is not differentiable, and a perturbed ``A`` may pair
+        vertices differently.  ``target``, ``gather`` and the batching mean what they mean in ``graph_saliency`` (the
+        per-batch sums are added on the host in float64 in batch order); the result is in ROI order either way.  Raises
+        ``ValueError`` when ``A`` is not square, not symmetric or has a nonzero diagonal, when its coarsening's vertex
+        order is not ``perm``, when a Laplacian the network uses, rebuilt from ``A``, rescaled and cast to fp32, is not
+        exactly the model's, and for the ``fourier`` filter.  Runs on the GPU through ``saliency.AdjacencyGradient``
+        (one CUDA graph per batch shape); the maps from ``A`` are built once per model and ``A``."""
+        from scipy import sparse
+
+        from .saliency import AdjacencyGradient, AdjacencyMaps
+
+        if self.filter_name == "fourier":
+            raise ValueError("cgcnn.adjacency_saliency: the fourier filter's operator is the eigenbasis U, not the "
+                             "Laplacian L")
+        M0 = self.L[0].shape[0]
+        if gather is None:
+            if self.perm is not None and self.n_input_vertices == M0:
+                raise ValueError("cgcnn.adjacency_saliency: with perm set and n_input_vertices == M_0 say gather=True "
+                                 "(raw windows) or gather=False (already permuted) -- the shapes are identical")
+            gather = self.perm is not None and data.shape[1] == self.n_input_vertices != M0
+        gather = bool(gather) and self.perm is not None
+        A = sparse.csr_matrix(A)
+        params = tuple(p.data_ptr() for p in self.parameters())
+        cached = self.__dict__.get("_adjacency_saliency")
+        if (cached is None or cached[0] != params or cached[1].shape != A.shape or cached[1].dtype != A.dtype
+                or (cached[1] != A).nnz):
+            maps = AdjacencyMaps(self, A)  # also checks that perm is a permutation of [0, M_0)
+            cached = self.__dict__["_adjacency_saliency"] = (params, A.copy(), AdjacencyGradient(self, maps))
+        ag = cached[2]
+        size, bs = data.shape[0], self.batch_size
+        total = np.zeros(len(ag.maps.rows))
+        for begin in range(0, size, bs):
+            end = min(begin + bs, size)
+            batch = self._padded_batch(data, begin)
+            t = None
+            if target is not None:
+                t = torch.zeros(bs, dtype=torch.long, device=self.dev)
+                t[: end - begin] = torch.as_tensor(np.asarray(target[begin:end]), dtype=torch.long, device=self.dev)
+            g, _, _ = ag(batch, t, gather=gather, valid=end - begin, absolute=absolute)
+            total += g.cpu().numpy().astype(np.float64)
+        return ag.maps.matrix(total)
 
     # ------------------------------------------------------------------ base_model's small public methods
     def inference(self, data, dropout=1.0):

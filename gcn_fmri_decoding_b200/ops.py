@@ -17,6 +17,8 @@ Op                       replaces (``/root/reference/lib_new/models_gcn.py``)
                           counterpart)
 ``cheb_dL``               gradient of a ChebyNet layer w.r.t. its operator's entries (edge saliency maps,
                           ``saliency.GraphGradient``; no reference counterpart)
+``adjacency_grad``        chain rule from the operator gradients to the edge weights of the adjacency (edge saliency
+                          maps in ROI coordinates, ``saliency.AdjacencyGradient``; no reference counterpart)
 """
 from __future__ import annotations
 
@@ -337,6 +339,42 @@ def cheb_dL(x: Tensor, perm: Optional[Tensor], M_in: int, y: Tensor, argmax: Ten
 def _(x, perm, M_in, y, argmax, dy, dy_is_mean, rowptr, col, val, rowptr_t, col_t, val_t, W, dval, ddiag, accumulate, K,
       p, relu, need_dx):
     return y.new_empty((y.shape[0], M_in, W.shape[0] // K) if need_dx else (0,))
+
+
+def adjacency_grad(levels, edges: Tensor, absolute: bool) -> Tensor:
+    """Gradient w.r.t. the undirected edge weights of the adjacency, per window (``gcnb_adjacency_grad_f32``): float32
+    ``[B, E]``.  ``levels``, finest first: one ``(dval [B, nnz], rowptr, val, rowptr_t, tpos, ss, hinv, parent)`` per
+    level, ``dval`` the level's operator gradient (``cheb_dL``'s, contiguous float32), ``rowptr / val / rowptr_t`` its
+    plan's CSR arrays, ``tpos`` (int32 [nnz]) the position in ``val`` of each entry of the transpose's CSR order,
+    ``ss`` (float32 [nnz]) ``s_a s_b``, ``hinv`` (float32 [M]) ``1 / (2 d)``, ``parent`` (int32 [nnz]) the entry of the next
+    level in the list or -1, None for the last.  ``edges`` (int32 [E, 2]): the level-0 entries ``(a, b)`` and ``(b, a)`` of
+    each edge.  ``absolute``: ``|.|`` per window.  No host synchronisation (CUDA-graph capturable)."""
+    dev = edges.device
+    B = levels[0][0].shape[0]
+    structs = (_lib.GcnbAdjLevel * len(levels))()
+    for l, (dval, rowptr, val, rowptr_t, tpos, ss, hinv, parent) in enumerate(levels):
+        M, nnz = rowptr.numel() - 1, val.numel()
+        if tuple(dval.shape) != (B, nnz) or dval.dtype != torch.float32 or not dval.is_contiguous():
+            raise ValueError("level %d: dval must be a contiguous float32 %s tensor" % (l, (B, nnz)))
+        for name, t, n, dt in (("rowptr_t", rowptr_t, M + 1, torch.int32), ("tpos", tpos, nnz, torch.int32),
+                               ("ss", ss, nnz, torch.float32), ("hinv", hinv, M, torch.float32)):
+            if t.numel() != n or t.dtype != dt or t.device != dev:
+                raise ValueError("level %d: %s must be %s with %d entries on %s" % (l, name, dt, n, dev))
+        if (parent is None) != (l == len(levels) - 1) or (parent is not None and parent.numel() != nnz):
+            raise ValueError("level %d: parent must be int32 [nnz] on every level but the last, None there" % l)
+        addr = lambda t: None if t is None or t.numel() == 0 else t.data_ptr()
+        structs[l] = _lib.GcnbAdjLevel(addr(dval), addr(rowptr), addr(val), addr(rowptr_t), addr(tpos), addr(ss),
+                                       addr(hinv), addr(parent), M, nnz)
+    if edges.dim() != 2 or edges.shape[1] != 2 or edges.dtype != torch.int32:
+        raise ValueError("edges must be int32 [E, 2]")
+    E = edges.shape[0]
+    out = torch.empty((B, E), dtype=torch.float32, device=dev)
+    L = _lib.lib()
+    ws = _workspace(L.gcnb_adjacency_grad_workspace_bytes(structs, len(levels), B), dev)
+    rc = L.gcnb_adjacency_grad_f32(structs, len(levels), _ptr(edges), E, _ptr(out), B, int(absolute), _ptr(ws),
+                                   ws.numel(), _stream(out))
+    _lib.check(rc, "gcnb_adjacency_grad_f32")
+    return out
 
 
 def unpermute(dx: Tensor, perm: Tensor, M_in: int) -> Tensor:

@@ -17,6 +17,8 @@ The whole schedule is captured as one CUDA graph per batch shape.
 ``GraphGradient`` (``cgcnn.graph_saliency``) differentiates the same logit w.r.t. the entries of the graph Laplacians
 instead: the same forward, seed and head backward, then ``ops.cheb_dL`` per conv layer (the operator gradient of
 ``k_sddmm_tma`` on the general path's stacks, and the input gradient that feeds the layer below).
+``AdjacencyGradient`` (``cgcnn.adjacency_saliency``) carries those per-level gradients on to the edge weights of the
+adjacency the Laplacians were built from (``ops.adjacency_grad``, with the host maps of ``AdjacencyMaps``).
 
 The ``fourier`` filter has no input-gradient-only kernel: its layers go through ``spectral_bwd(need_dx=True)``, which also
 computes the weight and bias gradients that are then dropped, and the first layer is un-permuted by ``ops.unpermute``.
@@ -209,10 +211,10 @@ class GraphGradient(InputGradient):
         super().__init__(model, use_cuda_graph)
 
     @torch.no_grad()
-    def _impl(self, x, target, gather, mask=None, absolute=False):
+    def _level_grads(self, x, target, gather, mask):
+        """The forward pass, the seed and the ``cheb_dL`` loop: ``(bufs, logits, target)`` with ``bufs[level] = (buf,
+        dval [B, nnz], ddiag [B, M])``, the per-window gradient w.r.t. that level's operator."""
         m = self.model
-        lib = _lib.lib()
-        stream = C.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
         nconv = len(m.p)
         saved, dy, logits, target = self._forward(x, target, gather, mask)
         B = x.shape[0]
@@ -230,6 +232,11 @@ class GraphGradient(InputGradient):
             dy = ops.cheb_dL(hin, perm, M_in, y, am, dy, dy_is_mean, *pl.tensors(), m.conv_weights[i], dval, ddiag,
                              accumulate, m.K[i], m.p[i], True, i > 0)
             dy_is_mean = False
+        return bufs, logits, target
+
+    @torch.no_grad()
+    def _impl(self, x, target, gather, mask=None, absolute=False):
+        bufs, logits, target = self._level_grads(x, target, gather, mask)
         # ---- sum over the windows, fixed order: the dval and ddiag blocks of every buffer as column sums ----
         out, mats = {}, []
         for lvl, (buf, dval, ddiag) in sorted(bufs.items()):
@@ -240,14 +247,7 @@ class GraphGradient(InputGradient):
             if dval.shape[1]:
                 mats.append((dval, o[: dval.shape[1]]))
             mats.append((ddiag, o[dval.shape[1]:]))
-        for c in range(0, len(mats), 4):
-            part = mats[c:c + 4]
-            n = len(part)
-            rc = lib.gcnb_colsum_multi_f32((C.c_void_p * n)(*[a.data_ptr() for a, _ in part]),
-                                           (C.c_void_p * n)(*[o.data_ptr() for _, o in part]),
-                                           (C.c_int * n)(*[a.shape[0] for a, _ in part]),
-                                           (C.c_int * n)(*[a.shape[1] for a, _ in part]), n, stream)
-            _lib.check(rc, "gcnb_colsum_multi_f32")
+        _colsums(mats, x.device)
         return out, logits, target
 
     def __call__(self, x, target=None, gather=False, valid=None, absolute=False):
@@ -287,6 +287,167 @@ class GraphGradient(InputGradient):
             st.copy_(target, non_blocking=True)
         graph.replay()
         return out
+
+
+def _colsums(mats, device):
+    """``out = a.sum(0)`` in a fixed order for every ``(a [R, C], out [C])`` of ``mats`` (``gcnb_colsum_multi_f32``, up
+    to four matrices per launch)."""
+    lib = _lib.lib()
+    stream = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    for c in range(0, len(mats), 4):
+        part = mats[c:c + 4]
+        n = len(part)
+        rc = lib.gcnb_colsum_multi_f32((C.c_void_p * n)(*[a.data_ptr() for a, _ in part]),
+                                       (C.c_void_p * n)(*[o.data_ptr() for _, o in part]),
+                                       (C.c_int * n)(*[a.shape[0] for a, _ in part]),
+                                       (C.c_int * n)(*[a.shape[1] for a, _ in part]), n, stream)
+        _lib.check(rc, "gcnb_colsum_multi_f32")
+
+
+class AdjacencyMaps:
+    """The host maps of the chain rule from the per-level operator gradients of ``GraphGradient`` to the undirected edge
+    weights of the adjacency ``A`` the model's Laplacians were built from (``A -> graclus.coarsen -> graphs.laplacian``
+    per level), built once per model and ``A``.
+
+    The coarsening is recomputed from ``A`` with ``len(L) - 1`` levels of the constructor's ``L`` list; its vertex order
+    must be ``model.perm`` and every Laplacian the network uses must come out, rescaled and cast to fp32, exactly as
+    the model's operator.  Per used level (finest first): ``tpos`` (the position in the operator's CSR of each entry of
+    the transpose's CSR order), ``ss = s_a s_b`` per entry and ``hinv = 1 / (2 d)`` per vertex (fp64, then fp32; 0 for
+    an isolated vertex), and ``parent``, the entry of the next used level that entry ``(a, b)`` is summed into through
+    the coarsening (``(a >> q, b >> q)``, q the levels in between; -1 for a pair inside one cluster).  ``edges [E, 2]``:
+    the level-0 entries ``(a, b)``, ``(b, a)`` of every edge ``(rows[k], cols[k])``, ``rows < cols``, of ``A`` (the
+    upper triangle in CSR order)."""
+
+    def __init__(self, model, A):
+        from . import graclus, graphs
+
+        if model.filter_name == "fourier":
+            raise ValueError("adjacency saliency: the fourier filter's operator is the eigenbasis U, not the Laplacian L")
+        A = sp.csr_matrix(A, copy=True)
+        if A.shape[0] != A.shape[1]:
+            raise ValueError("adjacency saliency: A must be square (got %s)" % (A.shape,))
+        if not np.issubdtype(A.dtype, np.floating):
+            raise ValueError("adjacency saliency: A must hold floating-point weights (got %s)" % A.dtype)
+        A.sum_duplicates()
+        A.eliminate_zeros()
+        if (A != A.T).nnz:
+            raise ValueError("adjacency saliency: A must be symmetric")
+        if A.diagonal().any():
+            raise ValueError("adjacency saliency: A must have a zero diagonal")
+        state = np.random.get_state()  # graclus.metis seeds the global generator, as the reference does
+        try:
+            gs, perm = graclus.coarsen(A, model._n_laplacians - 1)
+        finally:
+            np.random.set_state(state)
+        mperm = None if model.perm is None else model.perm.cpu().numpy()
+        if (perm is None) != (mperm is None) or (perm is not None and not np.array_equal(perm, mperm)):
+            raise ValueError("adjacency saliency: the vertex order of A's coarsening differs from model.perm")
+        used = sorted(set(model._graph_levels))
+        self.n, self.levels, host = A.shape[0], used, []
+        for lvl in range(used[-1] + 1):
+            rp, ci, v = graphs.csr_arrays(graphs.rescale_L(graphs.laplacian(gs[lvl])))
+            M = len(rp) - 1
+            rows = np.repeat(np.arange(M), np.diff(rp)).astype(np.int64)
+            if lvl in used:
+                pl = model._plan(model.L[model._graph_levels.index(lvl)])
+                if not all(np.array_equal(a, b) for a, b in zip((rp, ci, v), pl._host[False])):
+                    raise ValueError("adjacency saliency: the Laplacian of level %d built from A (rescaled, fp32) is not "
+                                     "the model's" % lvl)
+            G = sp.csr_matrix(gs[lvl], dtype=np.float64)
+            G.sum_duplicates()
+            G.sort_indices()
+            if not (np.array_equal(G.indptr, rp) and np.array_equal(G.indices, ci)):
+                raise ValueError("adjacency saliency: level %d: the operator's pattern is not the adjacency's" % lvl)
+            d = np.asarray(G.sum(axis=0)).ravel()
+            s = np.where(d > 0, 1 / np.sqrt(np.where(d > 0, d, 1)), 0)
+            host.append(dict(M=M, rows=rows, cols=ci.astype(np.int64), tpos=np.lexsort((rows, ci)),
+                             ss=(s[rows] * s[ci]).astype(np.float32),
+                             hinv=np.where(d > 0, 0.5 / np.where(d > 0, d, 1), 0).astype(np.float32)))
+        # entry (a, b) of level l -> entry (a >> 1, b >> 1) of level l + 1, then composed across the unused levels
+        for lvl in range(used[-1]):
+            h, up = host[lvl], host[lvl + 1]
+            pa, pb = h["rows"] >> 1, h["cols"] >> 1
+            cross = pa != pb
+            h["up"] = np.full(len(pa), -1, np.int64)
+            h["up"][cross] = _entry_index(up, pa[cross], pb[cross])
+        self.parent = {}
+        for i, lvl in enumerate(used):
+            if i + 1 == len(used):
+                self.parent[lvl] = None
+                continue
+            par = host[lvl]["up"]
+            for mid in range(lvl + 1, used[i + 1]):
+                par = np.where(par >= 0, host[mid]["up"][np.maximum(par, 0)], -1)
+            self.parent[lvl] = par.astype(np.int32)
+        # the edges of A in ROI order -> their two level-0 entries in the model's vertex order
+        U = sp.triu(A, 1).tocsr()
+        self.rows = np.repeat(np.arange(self.n), np.diff(U.indptr))
+        self.cols = U.indices.astype(np.int64)
+        inv = np.arange(host[0]["M"])
+        if perm is not None:
+            inv[np.asarray(perm)] = np.arange(len(perm))
+        a, b = inv[self.rows], inv[self.cols]
+        self.edges = np.stack([_entry_index(host[0], a, b), _entry_index(host[0], b, a)], 1).astype(np.int32)
+        self.tpos = {lvl: host[lvl]["tpos"].astype(np.int32) for lvl in used}
+        self.ss = {lvl: host[lvl]["ss"] for lvl in used}
+        self.hinv = {lvl: host[lvl]["hinv"] for lvl in used}
+        self._dev = {}
+
+    def device(self, device):
+        """The maps as device tensors: ``({level: (tpos, ss, hinv, parent or None)}, edges)``."""
+        device = torch.device(device)
+        if device not in self._dev:
+            t = lambda a: None if a is None else torch.from_numpy(np.ascontiguousarray(a)).to(device)
+            self._dev[device] = ({lvl: (t(self.tpos[lvl]), t(self.ss[lvl]), t(self.hinv[lvl]), t(self.parent[lvl]))
+                                  for lvl in self.levels}, t(self.edges))
+        return self._dev[device]
+
+    def matrix(self, g):
+        """Symmetric ``[n, n]`` float64 CSR on the pattern of ``A`` from an edge vector ``g [E]``."""
+        g = np.asarray(g, np.float64)
+        return sp.csr_matrix((np.concatenate([g, g]), (np.concatenate([self.rows, self.cols]),
+                                                       np.concatenate([self.cols, self.rows]))), shape=(self.n, self.n))
+
+
+def _entry_index(h, r, c):
+    """Positions of the entries ``(r[k], c[k])`` in a level's CSR order (sorted rows); every entry must be stored."""
+    key = h["rows"] * h["M"] + h["cols"]
+    q = np.asarray(r, np.int64) * h["M"] + np.asarray(c, np.int64)
+    pos = np.minimum(np.searchsorted(key, q), max(len(key) - 1, 0))
+    if len(q) and (len(key) == 0 or (key[pos] != q).any()):
+        raise ValueError("adjacency saliency: the coarsening maps an entry onto one its coarser level does not store")
+    return pos
+
+
+class AdjacencyGradient(GraphGradient):
+    """``g, logits, target = AdjacencyGradient(model, maps)(x, target=None, gather=False, valid=None, absolute=False)``:
+    the gradient of ``logits[b, target[b]]`` w.r.t. every undirected edge weight of the adjacency ``A`` behind the
+    model's Laplacians (``maps = AdjacencyMaps(model, A)``), summed over the windows ``b`` of the batch: float32
+    ``[E]`` in the order of ``maps.rows / maps.cols``.  ``absolute``: ``sum_b |dA_b|``, the absolute value taken per
+    window after every path through which the weight reaches the network is added up.
+
+    Schedule: ``GraphGradient``'s forward, seed and ``cheb_dL`` loop, then ``ops.adjacency_grad`` on the per-level
+    buffers (the chain through each level's degree normalisation and the coarsening, into ``[B, E]``) and a
+    fixed-order sum over the windows (``gcnb_colsum_multi_f32``).  One CUDA graph per batch shape."""
+
+    def __init__(self, model, maps, use_cuda_graph=True):
+        super().__init__(model, use_cuda_graph)
+        self.maps = maps
+
+    @torch.no_grad()
+    def _impl(self, x, target, gather, mask=None, absolute=False):
+        m = self.model
+        bufs, logits, target = self._level_grads(x, target, gather, mask)
+        per_level, edges = self.maps.device(x.device)
+        levels = []
+        for lvl in self.maps.levels:
+            pl = m._plan(m.L[m._graph_levels.index(lvl)])
+            levels.append((bufs[lvl][1], pl.rowptr, pl.val, pl.rowptr_t) + per_level[lvl])
+        S = ops.adjacency_grad(levels, edges, absolute)
+        out = torch.empty(S.shape[1], dtype=torch.float32, device=x.device)
+        if S.shape[1]:
+            _colsums([(S, out)], x.device)
+        return out, logits, target
 
 
 def edge_matrix(plan, g):

@@ -220,6 +220,38 @@ GCNB_API int gcnb_cheb_dL_f32(const float* x, const int32_t* perm, int M_in, con
                               int p, int relu, void* workspace, size_t workspace_bytes, gcnb_stream_t stream);
 
 /*
+ * Gradient w.r.t. the edge weights of the adjacency A the Laplacians were built from (edge saliency maps in ROI
+ * coordinates), per window, from the per-level operator gradients G_l of gcnb_cheb_dL_f32.  Per level l, with A_l the
+ * level's adjacency (zero diagonal), d_b = sum_a A_l[a][b], s = d^-1/2 and L~_l = -s_a A_ab s_b off the diagonal:
+ *   r_b = sum_j G_bj L~_bj,  c_b = sum_i G_ib L~_ib  (stored entries)
+ *   T_l[(a, b)] = -G_ab s_a s_b - (r_b + c_b) / (2 d_b) + T_next[parent[(a, b)]]
+ * where T_next is the next entry of `levels` (a coarser level: the Graclus coarsening sums the entries of merged vertex
+ * pairs, so its gradient flows back by a gather) and parent is -1 for a pair inside one cluster.  Then for every
+ * undirected edge k of A:  out[b][k] = T_0[b][edges[2k]] + T_0[b][edges[2k + 1]]  (|.| with absolute != 0), the two
+ * entries being (a, b) and (b, a) of level 0.  levels[0] is the finest level, levels[nlevels - 1] the coarsest; a
+ * level no layer uses (G = 0) is skipped by composing the parent maps across it.  The diagonal of L is constant, so
+ * gcnb_cheb_dL_f32's ddiag does not enter.  Every output is written by one thread in a fixed order: bit-reproducible.
+ * No allocation and no synchronisation (capturable); the workspace holds T_l, [B][nnz_l] per level.
+ */
+#define GCNB_ADJ_MAX_LEVELS 16
+typedef struct gcnb_adj_level {
+  const float* dval;        /* [B][nnz] G_l in L~_l's CSR order (may be NULL when nnz = 0) */
+  const int32_t* rowptr;    /* [M+1] L~_l's CSR (rows sorted by column, as gcnb_csr) */
+  const float* val;         /* [nnz] L~_l's values */
+  const int32_t* rowptr_t;  /* [M+1] CSR of L~_l^T */
+  const int32_t* tpos;      /* [nnz] entry t of L~_l^T's CSR order is entry tpos[t] of L~_l's */
+  const float* ss;          /* [nnz] s_a s_b of entry (a, b) */
+  const float* hinv;        /* [M] 1 / (2 d_b), 0 for an isolated vertex */
+  const int32_t* parent;    /* [nnz] entry of levels[l + 1], or -1; NULL for the last level */
+  int32_t M;
+  int32_t nnz;
+} gcnb_adj_level;
+GCNB_API size_t gcnb_adjacency_grad_workspace_bytes(const gcnb_adj_level* levels, int nlevels, int B);
+GCNB_API int gcnb_adjacency_grad_f32(const gcnb_adj_level* levels, int nlevels, const int32_t* edges, int E, float* out,
+                                     int B, int absolute, void* workspace, size_t workspace_bytes,
+                                     gcnb_stream_t stream);
+
+/*
  * Spectral layer (cgcnn.fourier + filter_in_fourier, models_gcn.py:512-539) with the same fused
  * bias/ReLU/pool epilogue.  Ut[M][M] is the transposed eigenvector matrix (row i = i-th
  * eigenvector), exactly the constant the reference builds at :536.  W[M][Fout][Fin].
