@@ -79,6 +79,7 @@ SIGNATURES = {
     "gcnb_relu_dropout_fwd_f32": (_i, [_p, C.c_longlong, _i, _i, C.c_float, C.c_uint, _p, _p]),
     "gcnb_relu_dropout_bwd_f32": (_i, [_p, _p, C.c_longlong, _i, _i, _i, C.c_float, _p]),
     "gcnb_colsum_multi_f32": (_i, [_p, _p, _p, _p, _i, _p]),
+    "gcnb_group_colsum_f32": (_i, [_p, _i, _i, _p, _i, _i, _p, _p]),
     "gcnb_gemm_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "gcnb_gemm_epilogue_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _i, C.c_float, C.c_uint, _p,
                                     _p]),

@@ -336,7 +336,7 @@ using namespace gcnb;
 
 extern "C" {
 
-int gcnb_version(void) { return 106; }
+int gcnb_version(void) { return 107; }
 
 const char* gcnb_last_error_string(void) { return g_err; }
 

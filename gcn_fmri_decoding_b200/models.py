@@ -383,14 +383,22 @@ class cgcnn(nn.Module):
             out += (all_logits,)
         return out if len(out) > 1 else out[0]
 
-    def saliency(self, data, target=None, gather=None):
+    def saliency(self, data, target=None, gather=None, groups=None, absolute=False):
         """Gradient saliency maps: ``(grad [n, n_input_vertices, channel] float32, target [n] int64)``, the gradient of
         the logit of class ``target[i]`` w.r.t. window ``i`` of ``data`` -- which ROIs and which TRs drive the decision.
         ``target=None`` takes the predicted class (the arg-max of the logits, as ``prediction()``).  Batched like
         ``predict``: batches of ``batch_size``, the last one zero-padded.  ``gather`` follows ``forward``: raw windows
         are permuted in the first layer's load and their gradient un-permuted in its store (with ``gather=False`` the
         data and the gradient are in the first layer's vertex order, ``[n, M_0, channel]``).  Runs on the GPU through
-        ``saliency.InputGradient`` (one CUDA graph per batch shape)."""
+        ``saliency.InputGradient`` (one CUDA graph per batch shape).
+
+        Group maps: with ``groups`` -- an integer array ``[n]`` of non-negative ids (class labels, subjects, runs), or
+        ``"target"`` to group by the class whose logit is differentiated -- returns ``(sums [G, n_input_vertices,
+        channel] float64, counts [G] int64, target [n] int64)``: ``sums[g]`` is the sum of the gradients of the windows
+        of group ``g`` (with ``absolute`` the sum of their absolute values), ``counts[g]`` how many windows it has
+        (divide for the group mean).  ``G = groups.max() + 1``, or the number of classes for ``"target"``.  The sums
+        are formed on the GPU per batch and added on the host in float64 in batch order; only ``[groups in the batch,
+        ...]`` leaves the device.  ``absolute`` needs ``groups``."""
         from .saliency import InputGradient
 
         M0 = self.L[0].shape[0]
@@ -405,11 +413,21 @@ class cgcnn(nn.Module):
             perm = self.perm.cpu().numpy()
             if not np.array_equal(np.sort(perm), np.arange(M0)):
                 raise ValueError("cgcnn.saliency: perm is not a permutation of [0, M_0 = %d)" % M0)
+        if groups is None and absolute:
+            raise ValueError("cgcnn.saliency: absolute needs groups (the per-window maps are returned signed)")
         params = tuple(p.data_ptr() for p in self.parameters())
         cached = self.__dict__.get("_saliency")
         if cached is None or cached[0] != params:
             cached = self.__dict__["_saliency"] = (params, InputGradient(self))
         ig = cached[1]
+        if groups is not None:
+            ids, G = self._saliency_groups("cgcnn.saliency", groups, data.shape[0])
+            sums, targets = self._grouped_saliency(
+                data, target, ids, G, (G,) + tuple(data.shape[1:]),
+                lambda batch, t, group, n_groups, valid: ig(batch, t, gather=gather, group=group, n_groups=n_groups,
+                                                            absolute=absolute, valid=valid),
+                lambda out, k: out[:k].cpu().numpy())
+            return sums, self._group_counts(ids, targets, G), targets
         size, bs = data.shape[0], self.batch_size
         grads = np.empty((size,) + tuple(data.shape[1:]), np.float32)
         targets = np.empty(size, np.int64)
@@ -426,7 +444,59 @@ class cgcnn(nn.Module):
             targets[begin:end] = tg[: end - begin].cpu().numpy()
         return grads, targets
 
-    def graph_saliency(self, data, target=None, gather=None, absolute=False):
+    @staticmethod
+    def _saliency_groups(name, groups, size):
+        """``(ids int64 [n] or None for "target", G)`` of a grouped saliency call's ``groups`` (``G = None`` for
+        "target": the number of classes); ``ValueError`` for a malformed one."""
+        if isinstance(groups, str):
+            if groups != "target":
+                raise ValueError("%s: groups must be an integer array of ids or 'target' (got %r)" % (name, groups))
+            return None, None
+        ids = np.asarray(groups)
+        if ids.ndim != 1 or ids.shape[0] != size:
+            raise ValueError("%s: groups must have one id per window, shape [%d] (got %s)" % (name, size, ids.shape))
+        if not np.issubdtype(ids.dtype, np.integer):
+            raise ValueError("%s: groups must hold integer ids (got dtype %s)" % (name, ids.dtype))
+        if size and ids.min() < 0:
+            raise ValueError("%s: groups must hold non-negative ids (got %d)" % (name, ids.min()))
+        ids = ids.astype(np.int64)
+        return ids, int(ids.max()) + 1 if size else 0
+
+    def _grouped_saliency(self, data, target, ids, G, shape, call, fetch):
+        """The batches of a grouped saliency call: ``call(batch, target, group, n_groups, valid)`` on every zero-padded
+        batch, with ``group`` the batch's ids mapped to ``0..k-1`` in ascending order (-1 on the padding rows, capacity
+        ``n_groups = batch_size``), or ``"target"``; ``fetch(out, k)`` copies the first ``k`` group rows of the result
+        to the host.  Returns ``(sums float64 [*shape] (shape[0] = G, or the number of classes for "target"), targets
+        [n] int64)``, the per-batch rows added in batch order."""
+        size, bs = data.shape[0], self.batch_size
+        if ids is None:
+            shape = (self.M[-1],) + tuple(shape[1:])
+        sums = np.zeros(shape)
+        targets = np.empty(size, np.int64)
+        for begin in range(0, size, bs):
+            end = min(begin + bs, size)
+            batch = self._padded_batch(data, begin)
+            t = None
+            if target is not None:
+                t = torch.zeros(bs, dtype=torch.long, device=self.dev)
+                t[: end - begin] = torch.as_tensor(np.asarray(target[begin:end]), dtype=torch.long, device=self.dev)
+            if ids is None:
+                out, _, tg = call(batch, t, "target", None, end - begin)
+                sums += fetch(out, shape[0])
+            else:
+                uniq, dense = np.unique(ids[begin:end], return_inverse=True)
+                group = torch.full((bs,), -1, dtype=torch.int32, device=self.dev)
+                group[: end - begin] = torch.as_tensor(dense.reshape(-1), dtype=torch.int32, device=self.dev)
+                out, _, tg = call(batch, t, group, bs, end - begin)
+                sums[uniq] += fetch(out, len(uniq))
+            targets[begin:end] = tg[: end - begin].cpu().numpy()
+        return sums, targets
+
+    def _group_counts(self, ids, targets, G):
+        """Windows per group: of the ids, or (``ids`` None) of the targets over the classes."""
+        return np.bincount(targets if ids is None else ids, minlength=self.M[-1] if ids is None else G).astype(np.int64)
+
+    def graph_saliency(self, data, target=None, gather=None, absolute=False, groups=None):
         """Edge saliency maps: which connections of the brain graph the decision relies on.  Returns ``{level:
         scipy.sparse.csr_matrix (float64)}`` for every level of the constructor's ``L`` list the network uses, each with
         the sparsity pattern of that ``L`` (its stored entries and the whole diagonal), holding
@@ -441,7 +511,10 @@ class cgcnn(nn.Module):
         fake vertices; coarser levels stay in the model's vertex order.  Batched like ``predict`` (the padding windows of
         the last batch contribute nothing); the per-batch sums are added on the host in float64 in batch order.  Runs on
         the GPU through ``saliency.GraphGradient`` (one CUDA graph per batch shape).  The ``fourier`` filter is refused:
-        its operator is the eigenbasis of ``L``, not ``L``."""
+        its operator is the eigenbasis of ``L``, not ``L``.
+
+        Group maps: ``groups`` as in ``saliency`` (ids ``[n]`` or ``"target"``) returns ``({level: [G csr_matrix]},
+        counts [G] int64)``, one matrix per group, each the map above over that group's windows only."""
         from .saliency import GraphGradient, edge_matrix, to_input_order
 
         if self.filter_name == "fourier":
@@ -463,6 +536,26 @@ class cgcnn(nn.Module):
         if cached is None or cached[0] != params:
             cached = self.__dict__["_graph_saliency"] = (params, GraphGradient(self))
         gg = cached[1]
+        levels = {}
+        for i, lvl in enumerate(self._graph_levels):
+            levels.setdefault(lvl, self._plan(self.L[i]))
+
+        def as_matrix(lvl, v):
+            G = edge_matrix(levels[lvl], v)
+            return to_input_order(G, perm, self.n_input_vertices) if lvl == 0 and gather else G
+
+        if groups is not None:
+            ids, G = self._saliency_groups("cgcnn.graph_saliency", groups, data.shape[0])
+            widths = np.cumsum([0] + [pl.nnz + pl.M for _, pl in sorted(levels.items())])
+            sums, targets = self._grouped_saliency(
+                data, target, ids, G, (G, widths[-1]),
+                lambda batch, t, group, n_groups, valid: gg(batch, t, gather=gather, valid=valid, absolute=absolute,
+                                                            group=group, n_groups=n_groups),
+                lambda out, k: np.concatenate([a[:k].cpu().numpy() for _, pair in sorted(out.items()) for a in pair],
+                                              axis=1))
+            result = {lvl: [as_matrix(lvl, sums[g, widths[j]:widths[j + 1]]) for g in range(sums.shape[0])]
+                      for j, lvl in enumerate(sorted(levels))}
+            return result, self._group_counts(ids, targets, G)
         size, bs = data.shape[0], self.batch_size
         sums = {}
         for begin in range(0, size, bs):
@@ -476,18 +569,10 @@ class cgcnn(nn.Module):
             for lvl, g in out.items():
                 v = g.cpu().numpy().astype(np.float64)
                 sums[lvl] = sums[lvl] + v if lvl in sums else v
-        result = {}
-        for i, lvl in enumerate(self._graph_levels):
-            if lvl in result:
-                continue
-            pl = self._plan(self.L[i])
-            G = edge_matrix(pl, sums[lvl] if lvl in sums else np.zeros(pl.nnz + pl.M))
-            if lvl == 0 and gather:
-                G = to_input_order(G, perm, self.n_input_vertices)
-            result[lvl] = G
-        return result
+        return {lvl: as_matrix(lvl, sums[lvl] if lvl in sums else np.zeros(pl.nnz + pl.M))
+                for lvl, pl in levels.items()}
 
-    def adjacency_saliency(self, data, A, target=None, gather=None, absolute=False):
+    def adjacency_saliency(self, data, A, target=None, gather=None, absolute=False, groups=None):
         """Edge saliency maps in the coordinates the graph was built in: which functional connections drive the decision.
         ``A`` is the symmetric, zero-diagonal adjacency ``[n_roi, n_roi]`` (scipy sparse or dense) that the
         constructor's ``L`` list was built from (``graclus.coarsen(A, len(L) - 1)`` then ``graphs.laplacian`` per level,
@@ -504,7 +589,10 @@ class cgcnn(nn.Module):
         ``ValueError`` when ``A`` is not square, not symmetric or has a nonzero diagonal, when its coarsening's vertex
         order is not ``perm``, when a Laplacian the network uses, rebuilt from ``A``, rescaled and cast to fp32, is not
         exactly the model's, and for the ``fourier`` filter.  Runs on the GPU through ``saliency.AdjacencyGradient``
-        (one CUDA graph per batch shape); the maps from ``A`` are built once per model and ``A``."""
+        (one CUDA graph per batch shape); the maps from ``A`` are built once per model and ``A``.
+
+        Group maps: ``groups`` as in ``saliency`` (ids ``[n]`` or ``"target"``) returns ``([G symmetric csr_matrix],
+        counts [G] int64)``, one matrix per group, each the map above over that group's windows only."""
         from scipy import sparse
 
         from .saliency import AdjacencyGradient, AdjacencyMaps
@@ -527,6 +615,14 @@ class cgcnn(nn.Module):
             maps = AdjacencyMaps(self, A)  # also checks that perm is a permutation of [0, M_0)
             cached = self.__dict__["_adjacency_saliency"] = (params, A.copy(), AdjacencyGradient(self, maps))
         ag = cached[2]
+        if groups is not None:
+            ids, G = self._saliency_groups("cgcnn.adjacency_saliency", groups, data.shape[0])
+            sums, targets = self._grouped_saliency(
+                data, target, ids, G, (G, len(ag.maps.rows)),
+                lambda batch, t, group, n_groups, valid: ag(batch, t, gather=gather, valid=valid, absolute=absolute,
+                                                            group=group, n_groups=n_groups),
+                lambda out, k: out[:k].cpu().numpy())
+            return [ag.maps.matrix(v) for v in sums], self._group_counts(ids, targets, G)
         size, bs = data.shape[0], self.batch_size
         total = np.zeros(len(ag.maps.rows))
         for begin in range(0, size, bs):

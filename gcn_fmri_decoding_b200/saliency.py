@@ -20,6 +20,10 @@ instead: the same forward, seed and head backward, then ``ops.cheb_dL`` per conv
 ``AdjacencyGradient`` (``cgcnn.adjacency_saliency``) carries those per-level gradients on to the edge weights of the
 adjacency the Laplacians were built from (``ops.adjacency_grad``, with the host maps of ``AdjacencyMaps``).
 
+Every class also has a grouped mode (``group=...``): instead of per-window values it returns, per group of windows (a
+class, a subject, a run), the sum of the windows' gradients (or of their absolute values) -- the fixed-order grouped
+column sum ``gcnb_group_colsum_f32`` inside the same CUDA graph, so only ``[n_groups, ...]`` leaves the device.
+
 The ``fourier`` filter has no input-gradient-only kernel: its layers go through ``spectral_bwd(need_dx=True)``, which also
 computes the weight and bias gradients that are then dropped, and the first layer is un-permuted by ``ops.unpermute``.
 That path is correct but not optimised.
@@ -42,6 +46,13 @@ class InputGradient:
     layer permutes (``model.perm`` must then be a permutation of ``[0, M_0)``, which ``cgcnn.saliency`` checks); else
     ``x`` is already in the first layer's vertex order ``[B, M_0, channel]``.
 
+    Grouped mode, ``group`` (int32 ``[B]`` on the device, or ``"target"``): ``(sums [n_groups, *x.shape[1:]], logits,
+    target)`` with ``sums[g]`` the sum of the gradients of the windows ``b`` with ``group[b] == g`` (``absolute``: of
+    their absolute values).  Rows with a group outside ``[0, n_groups)`` (-1 on padding rows) count nowhere, and rows of
+    ``sums`` whose group occurs in no row are not written.  ``n_groups`` defaults to ``B``; the cost does not depend on
+    it.  ``group="target"`` groups by the differentiated class: ``n_groups`` is the number of classes, the first
+    ``valid`` rows (None: all) are windows, and ``sums`` is zeroed first.
+
     With ``use_cuda_graph`` the returned tensors belong to the captured graph of that batch shape and are overwritten by
     the next call with the same shape.  A graph reads the model's parameters where they are when it is captured: build a
     new ``InputGradient`` after the parameters are replaced (not merely updated in place).
@@ -52,7 +63,7 @@ class InputGradient:
             raise ValueError("InputGradient: unsupported filter %r" % model.filter_name)
         self.model = model
         self.use_cuda_graph = use_cuda_graph
-        self._graphs = {}  # (x shape, gather, target given) -> (static x, static target, outputs, graph)
+        self._graphs = {}  # (x shape, gather, target given, ..., grouping) -> (static inputs, outputs, graph)
         self._step = None  # device counter of the dropout generator: keep = 1 never reads a mask, but the call takes one
 
     # -- one run, eagerly --------------------------------------------------------------------------------------------
@@ -128,7 +139,7 @@ class InputGradient:
         return saved, d, logits, target
 
     @torch.no_grad()
-    def _impl(self, x, target, gather):
+    def _impl(self, x, target, gather, group=None, mask=None, grouping=None):
         m = self.model
         mode = m._bias_mode()
         cheb = m.filter_name != "fourier"
@@ -153,39 +164,72 @@ class InputGradient:
                 if perm is not None:
                     dy = ops.unpermute(dy, perm, M_in)
             dy_is_mean = False
-        return dy, logits, target
+        if grouping is None:
+            return dy, logits, target
+        n_groups, absolute, _ = grouping
+        B = x.shape[0]
+        out = _grouped_out((n_groups,) + tuple(x.shape[1:]), grouping, x.device)
+        _group_sums([(dy.reshape(B, -1), out.view(n_groups, -1))], _group_vector(group, target, mask), n_groups,
+                    absolute)
+        return out, logits, target
 
-    def __call__(self, x, target=None, gather=False):
-        """``(grad [B, *x.shape[1:]], logits [B, C], target [B] int64)`` for the batch ``x`` (float32, on the model's
-        device); ``target`` (int64 [B] or None) is the class whose logit is differentiated."""
-        gather = bool(gather) and self.model.perm is not None
-        if target is not None:
-            target = torch.as_tensor(target, dtype=torch.long, device=x.device)
+    def _grouping(self, x, group, n_groups, absolute, valid):
+        """The grouped call's ``(group int32 [B] or None, mask or None, (n_groups, absolute, by target))`` (None:
+        ungrouped)."""
+        B = x.shape[0]
+        if group is None:
+            return None, None, None
+        if isinstance(group, str):
+            if group != "target":
+                raise ValueError("%s: group must be an int32 tensor or 'target' (got %r)" % (type(self).__name__, group))
+            valid = B if valid is None else int(valid)
+            mask = (torch.arange(B, device=x.device) < valid).to(torch.float32)
+            return None, mask, (int(self.model.M[-1]), bool(absolute), True)
+        n_groups = B if n_groups is None else int(n_groups)
+        if not 1 <= n_groups <= B:
+            raise ValueError("%s: n_groups = %d outside [1, B = %d]" % (type(self).__name__, n_groups, B))
+        group = torch.as_tensor(group, dtype=torch.int32, device=x.device)
+        if tuple(group.shape) != (B,):
+            raise ValueError("%s: group must have shape [%d] (got %s)" % (type(self).__name__, B, tuple(group.shape)))
+        return group, None, (n_groups, bool(absolute), False)
+
+    def _run(self, key, fn, *inputs):
+        """``fn(*inputs)``; with ``use_cuda_graph`` replayed from the CUDA graph of ``key``, captured on static copies of
+        the tensor ``inputs`` (a None input stays None) and fed by copies into them."""
         if not self.use_cuda_graph:
-            return self._impl(x, target, gather)
-        key = (tuple(x.shape), gather, target is not None)
+            return fn(*inputs)
         if key not in self._graphs:
-            sx = torch.empty_like(x)
-            st = torch.zeros(x.shape[0], dtype=torch.long, device=x.device) if target is not None else None
-            sx.copy_(x)
-            if st is not None:
-                st.copy_(target)
+            static = tuple(None if t is None else t.clone() for t in inputs)
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(side):
                 for _ in range(2):  # warm up: allocator, lazy library set-up, operator images
-                    self._impl(sx, st, gather)
+                    fn(*static)
             torch.cuda.current_stream().wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                out = self._impl(sx, st, gather)
-            self._graphs[key] = (sx, st, out, graph)
-        sx, st, out, graph = self._graphs[key]
-        sx.copy_(x, non_blocking=True)
-        if st is not None:
-            st.copy_(target, non_blocking=True)
+                out = fn(*static)
+            self._graphs[key] = (static, out, graph)
+        static, out, graph = self._graphs[key]
+        for s_, t in zip(static, inputs):
+            if s_ is not None:
+                s_.copy_(t, non_blocking=True)
         graph.replay()
         return out
+
+    def __call__(self, x, target=None, gather=False, group=None, n_groups=None, absolute=False, valid=None):
+        """``(grad [B, *x.shape[1:]], logits [B, C], target [B] int64)`` for the batch ``x`` (float32, on the model's
+        device); ``target`` (int64 [B] or None) is the class whose logit is differentiated.  With ``group``: ``(sums
+        [n_groups, *x.shape[1:]], logits, target)`` (see the class)."""
+        gather = bool(gather) and self.model.perm is not None
+        if target is not None:
+            target = torch.as_tensor(target, dtype=torch.long, device=x.device)
+        group, mask, grouping = self._grouping(x, group, n_groups, absolute, valid)
+        if grouping is None and absolute:
+            raise ValueError("InputGradient: absolute needs group (the per-window gradient is returned signed)")
+        key = (tuple(x.shape), gather, target is not None, grouping)
+        return self._run(key, lambda sx, st, sg, sm: self._impl(sx, st, gather, sg, sm, grouping), x, target, group,
+                         mask)
 
 
 class GraphGradient(InputGradient):
@@ -203,6 +247,10 @@ class GraphGradient(InputGradient):
     ``ops.cheb_dL`` per layer, accumulating into one ``[B, nnz + M]`` buffer per distinct Laplacian (its ``dx`` feeds the
     layer below), and a fixed-order sum over the windows per buffer (``gcnb_colsum_multi_f32``).  One CUDA graph per
     batch shape.  The ``fourier`` filter is refused: its operator is the eigenbasis, not ``L``.
+
+    Grouped mode (``group``, ``n_groups`` as in ``InputGradient``): ``grads[level] = (sums [n_groups, nnz], sums
+    [n_groups, M])``, the CSR-entry and diagonal blocks summed per group by ``gcnb_group_colsum_f32`` (with
+    ``absolute`` the absolute value fused into that sum, still per window after all layers are added up).
     """
 
     def __init__(self, model, use_cuda_graph=True):
@@ -235,8 +283,16 @@ class GraphGradient(InputGradient):
         return bufs, logits, target
 
     @torch.no_grad()
-    def _impl(self, x, target, gather, mask=None, absolute=False):
+    def _impl(self, x, target, gather, mask=None, absolute=False, group=None, grouping=None):
         bufs, logits, target = self._level_grads(x, target, gather, mask)
+        if grouping is not None:
+            n_groups, absolute, _ = grouping
+            out, mats = {}, []
+            for lvl, (buf, dval, ddiag) in sorted(bufs.items()):
+                out[lvl] = tuple(_grouped_out((n_groups, a.shape[1]), grouping, x.device) for a in (dval, ddiag))
+                mats += [(a, o) for a, o in zip((dval, ddiag), out[lvl]) if a.shape[1]]
+            _group_sums(mats, _group_vector(group, target, mask), n_groups, absolute)
+            return out, logits, target
         # ---- sum over the windows, fixed order: the dval and ddiag blocks of every buffer as column sums ----
         out, mats = {}, []
         for lvl, (buf, dval, ddiag) in sorted(bufs.items()):
@@ -250,43 +306,22 @@ class GraphGradient(InputGradient):
         _colsums(mats, x.device)
         return out, logits, target
 
-    def __call__(self, x, target=None, gather=False, valid=None, absolute=False):
+    def __call__(self, x, target=None, gather=False, valid=None, absolute=False, group=None, n_groups=None):
         """``({level: float32 [nnz + M]}, logits [B, C], target [B] int64)`` for the batch ``x`` (float32, on the model's
         device); ``target`` (int64 [B] or None) is the class whose logit is differentiated, ``valid`` the number of
-        leading rows that are windows (None: all)."""
+        leading rows that are windows (None: all).  With ``group``: ``({level: (sums [n_groups, nnz], sums [n_groups,
+        M])}, logits, target)`` (see the class)."""
         gather = bool(gather) and self.model.perm is not None
         B = x.shape[0]
         valid = B if valid is None else int(valid)
         mask = (torch.arange(B, device=x.device) < valid).to(torch.float32)
         if target is not None:
             target = torch.as_tensor(target, dtype=torch.long, device=x.device)
-        if not self.use_cuda_graph:
-            return self._impl(x, target, gather, mask, bool(absolute))
-        key = (tuple(x.shape), gather, target is not None, bool(absolute))
-        if key not in self._graphs:
-            sx, sm = torch.empty_like(x), torch.empty_like(mask)
-            st = torch.zeros(B, dtype=torch.long, device=x.device) if target is not None else None
-            sx.copy_(x)
-            sm.copy_(mask)
-            if st is not None:
-                st.copy_(target)
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                for _ in range(2):  # warm up: allocator, lazy library set-up, operator images
-                    self._impl(sx, st, gather, sm, bool(absolute))
-            torch.cuda.current_stream().wait_stream(side)
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                out = self._impl(sx, st, gather, sm, bool(absolute))
-            self._graphs[key] = (sx, st, sm, out, graph)
-        sx, st, sm, out, graph = self._graphs[key]
-        sx.copy_(x, non_blocking=True)
-        sm.copy_(mask, non_blocking=True)
-        if st is not None:
-            st.copy_(target, non_blocking=True)
-        graph.replay()
-        return out
+        group, _, grouping = self._grouping(x, group, n_groups, absolute, valid)
+        absolute = bool(absolute)
+        key = (tuple(x.shape), gather, target is not None, absolute, grouping)
+        return self._run(key, lambda sx, st, sm, sg: self._impl(sx, st, gather, sm, absolute, sg, grouping), x, target,
+                         mask, group)
 
 
 def _colsums(mats, device):
@@ -302,6 +337,32 @@ def _colsums(mats, device):
                                        (C.c_int * n)(*[a.shape[0] for a, _ in part]),
                                        (C.c_int * n)(*[a.shape[1] for a, _ in part]), n, stream)
         _lib.check(rc, "gcnb_colsum_multi_f32")
+
+
+def _group_sums(mats, group, n_groups, absolute):
+    """``out[g] = sum of the rows r of a with group[r] == g`` (``|a|`` with ``absolute``) in a fixed order for every
+    ``(a [R, C], out [n_groups, C])`` of ``mats`` (``gcnb_group_colsum_f32``, one launch each); ``group`` int32 [R] on
+    the device.  Rows of ``out`` whose group occurs in no row are not written."""
+    lib = _lib.lib()
+    stream = C.c_void_p(torch.cuda.current_stream(group.device).cuda_stream)
+    for a, out in mats:
+        a = a.contiguous()  # the kernel takes dense rows; ops.unpermute's gradient (fourier) is a strided view
+        rc = lib.gcnb_group_colsum_f32(C.c_void_p(a.data_ptr()), a.shape[0], a.shape[1], C.c_void_p(group.data_ptr()),
+                                       n_groups, int(absolute), C.c_void_p(out.data_ptr()), stream)
+        _lib.check(rc, "gcnb_group_colsum_f32")
+
+
+def _group_vector(group, target, mask):
+    """The group of every row of a grouped call: ``group`` as given, or (``group`` None: by target) the target class,
+    -1 on the padding rows (``mask`` 0)."""
+    if group is not None:
+        return group
+    return torch.where(mask > 0, target, torch.full_like(target, -1)).to(torch.int32)
+
+
+def _grouped_out(shape, grouping, device):
+    """The float32 output of a grouped sum: zeroed when grouped by target (rows of absent classes are not written)."""
+    return (torch.zeros if grouping[2] else torch.empty)(shape, dtype=torch.float32, device=device)
 
 
 class AdjacencyMaps:
@@ -428,14 +489,17 @@ class AdjacencyGradient(GraphGradient):
 
     Schedule: ``GraphGradient``'s forward, seed and ``cheb_dL`` loop, then ``ops.adjacency_grad`` on the per-level
     buffers (the chain through each level's degree normalisation and the coarsening, into ``[B, E]``) and a
-    fixed-order sum over the windows (``gcnb_colsum_multi_f32``).  One CUDA graph per batch shape."""
+    fixed-order sum over the windows (``gcnb_colsum_multi_f32``).  One CUDA graph per batch shape.
+
+    Grouped mode (``group``, ``n_groups`` as in ``InputGradient``): ``g [n_groups, E]``, the per-window edge gradients
+    summed per group by ``gcnb_group_colsum_f32``."""
 
     def __init__(self, model, maps, use_cuda_graph=True):
         super().__init__(model, use_cuda_graph)
         self.maps = maps
 
     @torch.no_grad()
-    def _impl(self, x, target, gather, mask=None, absolute=False):
+    def _impl(self, x, target, gather, mask=None, absolute=False, group=None, grouping=None):
         m = self.model
         bufs, logits, target = self._level_grads(x, target, gather, mask)
         per_level, edges = self.maps.device(x.device)
@@ -443,6 +507,13 @@ class AdjacencyGradient(GraphGradient):
         for lvl in self.maps.levels:
             pl = m._plan(m.L[m._graph_levels.index(lvl)])
             levels.append((bufs[lvl][1], pl.rowptr, pl.val, pl.rowptr_t) + per_level[lvl])
+        if grouping is not None:
+            n_groups, absolute, _ = grouping
+            S = ops.adjacency_grad(levels, edges, False)
+            out = _grouped_out((n_groups, S.shape[1]), grouping, x.device)
+            if S.shape[1]:
+                _group_sums([(S, out)], _group_vector(group, target, mask), n_groups, absolute)
+            return out, logits, target
         S = ops.adjacency_grad(levels, edges, absolute)
         out = torch.empty(S.shape[1], dtype=torch.float32, device=x.device)
         if S.shape[1]:

@@ -345,6 +345,14 @@ GCNB_API int gcnb_relu_dropout_bwd_f32(float* d, const float* act, long long row
  * the `+ b` of cgcnn.fc (models_gcn.py:653-654, :298-303). */
 GCNB_API int gcnb_colsum_multi_f32(const float* const* mats, float* const* outs, const int* rows, const int* cols,
                           int count, gcnb_stream_t stream);
+/* out[g][c] = sum over the rows r with group[r] == g of X[r][c] (|X[r][c]| with absolute != 0), X row-major
+ * [rows][cols], out [n_groups][cols]: per-group sums of per-window saliency maps (one row per window).  Rows whose group
+ * is < 0 or >= n_groups contribute nothing; rows of out whose group occurs in no row are NOT written.  1 <= rows <= 8192,
+ * cols >= 1, 1 <= n_groups <= rows.  Fixed summation order that depends only on (rows, group): bit-reproducible, no
+ * float atomics, no allocation, no synchronisation, CUDA-graph capturable.  The work grows with rows x cols and not with
+ * n_groups, so a caller may pass a capacity. */
+GCNB_API int gcnb_group_colsum_f32(const float* X, int rows, int cols, const int32_t* group, int n_groups,
+                                   int absolute, float* out, gcnb_stream_t stream);
 
 /*
  * tf.train.AdamOptimizer step (models_gcn.py:294, TF-1.x "epsilon hat" form) over one flat buffer of n parameters:
